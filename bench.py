@@ -19,6 +19,9 @@ data-path collective); timing is max over ranks, value the aggregate.
 drop-in calls (numpy in / numpy out, one pair per call), the k-means / cosine sweep of configs[4], and --
 on every N -- the one collective of the path: whole Lloyd fits over row-sharded vectors with the NCCL
 all-reduce (`dist_kmeans`), plus the host-link ceiling with all ranks uploading at once.
+
+`--dump-outputs DIR` writes what the last timed step computed (rank 0) as DIR/<name>.npy.  The clip is
+generated from a fixed seed, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -61,7 +64,14 @@ def parse():
     ap.add_argument("--k", type=int, default=1, help="the reference's -c: clusters per grid cell (every documented command uses 1)")
     ap.add_argument("--no-extras", action="store_true", help="only the headline workload")
     ap.add_argument("--lanes", type=int, default=3, help="chunks in flight on separate streams (LanedPipeline); 1 = one chain of kernels")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computed as DIR/<name>.npy (float32 / "
+                         "float64; flow and visualisation as a fixed, seeded sample of pixels) to compare two builds")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     global H, W, LEVELS, ALGO_BYTES_PER_PAIR, SIZE_NAME, METRIC
     H, W, LEVELS, ALGO_BYTES_PER_PAIR = SIZES[args.size]
     SIZE_NAME = args.size
@@ -176,8 +186,6 @@ def run_reference(args):
         v, wall = cpu_reference_throughput(frames, workers, ppw, args.k)
         if i >= args.warmup:
             times.append((v, wall))
-        if sum(w for _, w in times) > 150:
-            break
     value = sum(workers * ppw for _ in times) / sum(w for _, w in times)
     ms = 1e3 * sum(w for _, w in times) / len(times)
     sample = f"{workers} processes x {ppw} consecutive {SIZE_NAME} pairs per step, cv2.setNumThreads(1), k={args.k}"
@@ -585,6 +593,39 @@ def h2d_concurrent_leg(dev, world):
     return {"per_rank_min_gb_s": float(lo.item()), "all_ranks_gb_s": float(tot.item()), "ranks": world}
 
 
+DUMP_SAMPLE_PX = 1 << 20           # --dump-outputs: (pair, pixel) positions kept of the per-pixel outputs
+DUMP_SAMPLE_SEED = 0
+
+
+def dump_sample_index(n_px):
+    """the positions (flat index over pairs x rows x columns, ascending) at which --dump-outputs keeps the per-pixel
+    outputs: every position when there are at most DUMP_SAMPLE_PX, else DUMP_SAMPLE_PX drawn from a fixed seed"""
+    import torch
+    if n_px <= DUMP_SAMPLE_PX:
+        return torch.arange(n_px)
+    g = torch.Generator().manual_seed(DUMP_SAMPLE_SEED)
+    return torch.randint(n_px, (DUMP_SAMPLE_PX,), generator=g).sort().values
+
+
+def dump_outputs(out_dir, pipe, P):
+    """--dump-outputs: what the last timed step computed, i.e. what a caller of LanedPipeline.submit reads from the lane
+    that ran it, as out_dir/<name>.npy.  Per-cell rows and magnitudes are written whole; the flow and the visualisation
+    (0.7 GB at 1080p) at the positions of dump_sample_index.  Integer outputs are widened to float32 (exact), the mean
+    magnitude stays float64 (the host division of ClipPipeline.process_clip).  At most about 20 MB at any size."""
+    import numpy as np
+    idx = dump_sample_index(P * pipe.H * pipe.W).to(pipe.device)
+    out = {"avg_hue": pipe.avg_hue[:P], "km_hue": pipe.km_hue[:P], "km_centre": pipe.km_centre[:P], "avg_bgr": pipe.avg_bgr[:P],
+           "mean_magnitude": pipe.mag_sum[:P].cpu() / float(pipe.H * pipe.W),
+           "flow_sample": pipe.flow[:P].reshape(-1, 2)[idx], "viz_sample": pipe.viz[:P].reshape(-1, 3)[idx]}
+    if pipe.km_n_iter is not None:
+        out["km_n_iter"] = pipe.km_n_iter[:P]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in out.items():
+        a = t.cpu().numpy()
+        np.save(os.path.join(out_dir, name + ".npy"), a if a.dtype in (np.float32, np.float64) else a.astype(np.float32))
+    return sorted(out)
+
+
 _JSON_OUT = None
 
 
@@ -656,7 +697,7 @@ def main():
     torch.cuda.cudart().cudaProfilerStart()
     e0.record()
     for i in range(args.warmup, args.warmup + args.steps):
-        lp.submit(clip[starts[i]:starts[i] + F])            # each lane's stream waits for e0 through the current stream
+        last_lane, _ = lp.submit(clip[starts[i]:starts[i] + F])   # each lane's stream waits for e0 through the current stream
     for l in range(n_lanes):
         main_stream.wait_event(lp.done_event(l))
     e1.record()
@@ -664,6 +705,10 @@ def main():
     sampler.sample_now()        # after the last enqueue: the GPU is still working, and a slow NVML call cannot stall the timed steps
     barrier()
     clocks = sampler.stop()
+    dumped = None
+    if args.dump_outputs and rank == 0:          # before the e2e loop below reuses the lanes
+        dumped = {"dir": os.path.abspath(args.dump_outputs), "arrays": dump_outputs(args.dump_outputs, lp.lane(last_lane), P),
+                  "step": args.warmup + args.steps - 1, "frames": [starts[-1], starts[-1] + F]}
     ms_total = e0.elapsed_time(e1)
     t = torch.tensor([ms_total], dtype=torch.float64, device=dev)
     if world > 1:
@@ -852,6 +897,7 @@ def main():
                              f"({pipe.plan.workspace_bytes / 1e6:.0f} MB workspace) are rewritten every step"},
             "clocks": clocks, "e2e": e2e, "gpu_launches": launches_per_step * args.steps,
             "roofline": roofline, "cpu_baseline": cpu_baseline, "kernels": kernels, "extras": extras,
+            **({"dump_outputs": dumped} if dumped else {}),
         }), file=_claim_stdout(), flush=True)
     if world > 1:
         dist.destroy_process_group()

@@ -29,6 +29,16 @@ def golden_dir():
     return GOLDEN
 
 
+def run_without_gpu(code):
+    """Run ``code`` in a child Python started in the repository root that sees no CUDA device (``CUDA_VISIBLE_DEVICES``
+    empty), so that the no-GPU behaviour is checked on machines with a GPU too; returns the child's stdout."""
+    import subprocess
+    r = subprocess.run([sys.executable, "-c", code], cwd=ROOT, env=dict(os.environ, CUDA_VISIBLE_DEVICES=""),
+                       capture_output=True, text=True)
+    assert r.returncode == 0, r.stderr[-3000:]
+    return r.stdout
+
+
 def have_cv2():
     try:
         import cv2  # noqa: F401

@@ -5,7 +5,7 @@ import re
 
 import pytest
 
-from tests.conftest import ROOT
+from tests.conftest import ROOT, run_without_gpu
 
 
 @pytest.fixture(scope="module")
@@ -47,14 +47,18 @@ def test_sass_is_sm100a(so_path):
 
 def test_no_gpu_means_loud_failure():
     """No CPU fallback: without a CUDA device the operators raise."""
-    import numpy as np
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip("GPU present")
-    from opticalflowclustering_b200 import _lib, flow
-    with pytest.raises(_lib.OfcError):
-        flow.calc_optical_flow_farneback(np.zeros((64, 64), np.uint8), np.zeros((64, 64), np.uint8), None,
-                                         0.5, 3, 15, 3, 5, 1.2, 0)
+    out = run_without_gpu("""
+import numpy as np
+import torch
+assert not torch.cuda.is_available()
+from opticalflowclustering_b200 import _lib, flow
+try:
+    flow.calc_optical_flow_farneback(np.zeros((64, 64), np.uint8), np.zeros((64, 64), np.uint8), None,
+                                     0.5, 3, 15, 3, 5, 1.2, 0)
+except _lib.OfcError:
+    print("raised")
+""")
+    assert out.split() == ["raised"]
 
 
 def test_product_never_imports_oracle():

@@ -4,9 +4,8 @@ import csv
 import os
 
 import numpy as np
-import pytest
 
-from tests.conftest import GOLDEN
+from tests.conftest import GOLDEN, run_without_gpu
 
 
 def test_hue_row_text_matches_reference_layout():
@@ -68,11 +67,16 @@ def test_grid_lines_host_match_oracle_rectangles():
 
 
 def test_dropins_fail_loudly_without_gpu():
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip("GPU present")
-    from opticalflowclustering_b200 import _lib, cosine, kmeans
-    with pytest.raises(_lib.OfcError):
-        kmeans.kmeans_fit(np.zeros((8, 4), np.uint8), np.zeros((2, 4)))
-    with pytest.raises(_lib.OfcError):
-        cosine.sliding_cosine([1, 2], [1, 2, 3])
+    out = run_without_gpu("""
+import numpy as np
+import torch
+assert not torch.cuda.is_available()
+from opticalflowclustering_b200 import _lib, cosine, kmeans
+for call in (lambda: kmeans.kmeans_fit(np.zeros((8, 4), np.uint8), np.zeros((2, 4))),
+             lambda: cosine.sliding_cosine([1, 2], [1, 2, 3])):
+    try:
+        call()
+    except _lib.OfcError:
+        print("raised")
+""")
+    assert out.split() == ["raised", "raised"]
