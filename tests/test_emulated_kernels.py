@@ -228,3 +228,26 @@ def test_emu_streaming_form_equals_pairs():
         assert (pl.stream_next(g[t]) == want[t - 1]).all(), t
     with pytest.raises(RuntimeError, match="stream_begin"):
         E.Plan(W, H, max_frames=2).stream_next(g[1])
+
+
+@pytest.mark.parametrize("levels", [0, 1])
+def test_emu_pair_flow_independent_of_pair_count(levels):
+    """DESIGN 5a: a pair's flow bits do not depend on how many pairs share the call.  The iteration kernel of a level is
+    chosen from its geometry alone: a 240-px-wide level (a whole 240-column strip) must not switch from the square-tile
+    kernel to the strip walk once n_pairs * rows passes a multiple of the SM count (the emulation reports 3 SMs, so 5
+    pairs of 72 rows are past any such line and 2 pairs are short of it)."""
+    from opticalflowclustering_b200.synthetic import synthetic_clip
+    H, W = 72, 240
+    g = E.bgr2gray(synthetic_clip(6, H, W, seed=3).numpy())
+    two = E.Plan(W, H, max_frames=3, levels=levels).sequence(g[:3])
+    five = E.Plan(W, H, max_frames=6, levels=levels).sequence(g)
+    pl = E.Plan(W, H, max_frames=2, levels=levels)
+    pl.stream_begin(g[0])
+    streamed = pl.stream_next(g[1])
+    for name, got in (("5-pair sequence", five[0]), ("stream form", streamed)):
+        d = np.abs(got - two[0])
+        assert (got == two[0]).all(), (name, int((d.max(-1) > 0).sum()), float(d.max()))
+    assert (five[1] == two[1]).all()
+    ref = FB.calc_optical_flow_farneback(g[0], g[1], levels=levels)
+    e = np.linalg.norm(two[0] - ref, axis=-1)
+    assert e.mean() < 2e-6 and e.max() < 1e-4, (e.mean(), e.max())
