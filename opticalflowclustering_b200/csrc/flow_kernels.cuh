@@ -40,14 +40,13 @@ struct IterParams {
     int upsample;                // flow_in is the coarser level: bilinear resize * flow_mul
     int wc, hc;
     double usx, usy, flow_mul;
-    int ups_fast;                // w == 2 wc, h == 2 hc and flow_mul a power of two: integer resize coordinates, float scaling
+    float solve_c_hi, solve_c_lo; // 1e-3 / blur_scale^2 as two floats (solve2x2)
     float2* flow_out;
     int64_t flow_out_stride;
     int w, h;
     unsigned* minmax;            // [n_pairs][2] float bits (min, max) of |flow|, or null
     float border[5];
     double blur_scale;           // 1 / winsize^2
-    float solve_c_hi, solve_c_lo; // 1e-3 / blur_scale^2 as two floats (solve2x2)
 };
 
 // OPTFLOW_FARNEBACK_GAUSSIAN window: k[0] centre tap, k[i] the tap at distance i (2r+1 taps)
@@ -60,8 +59,7 @@ struct GaussWindow {
 int launch_prefilter(const PrefilterParams& p, int n_frames, size_t smem, void* stream);
 // all down-sampled levels whose size is an exact power-of-two fraction of the frame in ONE launch
 // (prefilter_pyr_kernel); done[i] is set for the levels it covered, the others go through launch_prefilter
-int launch_prefilter_pyramid(const PrefilterParams* levels, const size_t* smem_fallback, int n_levels, int n_frames,
-                             bool* done, void* stream);
+int launch_prefilter_pyramid(const PrefilterParams* levels, int n_levels, int n_frames, bool* done, void* stream);
 // gray != null: full-resolution level with the fixed 3-tap pre-filter; I is produced from the 8-bit
 // frame inside the expansion kernel (and written to I_out as a by-product)
 int launch_polyexp(const PolyParams& p, int poly_n, int n_frames, const unsigned char* gray, int64_t gray_stride,

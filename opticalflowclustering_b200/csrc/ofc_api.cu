@@ -220,7 +220,6 @@ static int run_farneback(const ofc_flow_plan* pl, const uint8_t* gray, int64_t g
     } side_join{fork ? pl->side : nullptr, (cudaStream_t)stream, fork ? pl->ev_fork : cudaEvent_t(), fork};
     // the pre-filter of every level that is an exact power-of-two fraction of the frame: one launch
     std::vector<PrefilterParams> pfs(nl);
-    std::vector<size_t> pf_smem(nl);
     std::vector<char> pf_done(nl, 0);
     for (int l = 0; l < nl; ++l) {
         const Level& L = pl->lv[l];
@@ -232,10 +231,9 @@ static int run_farneback(const ofc_flow_plan* pl, const uint8_t* gray, int64_t g
         pf.taps = pl->d_taps + L.taps_off;
         pf.identity3 = (L.sigma <= 0 && L.ksz == 3 && L.w == pl->W && L.h == pl->H) ? 1 : 0;
         pf.tx = L.tx; pf.ty = L.ty; pf.in_rows = L.in_rows; pf.in_pitch = L.in_pitch; pf.taps_pad = L.taps_pad;
-        pf_smem[l] = L.prefilter_smem;
     }
     {
-        int rc = stage1_frames > 0 ? launch_prefilter_pyramid(pfs.data(), pf_smem.data(), nl, stage1_frames,
+        int rc = stage1_frames > 0 ? launch_prefilter_pyramid(pfs.data(), nl, stage1_frames,
                                                              reinterpret_cast<bool*>(pf_done.data()), stream1)
                                    : OFC_OK;
         if (rc != OFC_OK) return rc;
@@ -292,7 +290,7 @@ static int run_farneback(const ofc_flow_plan* pl, const uint8_t* gray, int64_t g
                 ip.solve_c_hi = (float)c;
                 ip.solve_c_lo = (float)(c - (double)ip.solve_c_hi);
             }
-            ip.upsample = 0; ip.wc = ip.hc = 0; ip.usx = ip.usy = 1.0; ip.flow_mul = 1.0; ip.ups_fast = 0;
+            ip.upsample = 0; ip.wc = ip.hc = 0; ip.usx = ip.usy = 1.0; ip.flow_mul = 1.0;
             if (it == 0 && l == 0 && init_flow) {
                 // cv2 flag 4: resize(flow0, INTER_AREA) * scale seeds the coarsest level (other ping-pong buffer)
                 double scale = 1.0;
@@ -311,9 +309,6 @@ static int run_farneback(const ofc_flow_plan* pl, const uint8_t* gray, int64_t g
                     ip.usx = 1.0 / ((double)L.w / prev_w);
                     ip.usy = 1.0 / ((double)L.h / prev_h);
                     ip.flow_mul = 1.0 / pl->pyr_scale;
-                    int e2 = 0;
-                    const bool pow2 = frexp(ip.flow_mul, &e2) == 0.5 && ip.flow_mul >= 1.0 && ip.flow_mul <= 16.0;
-                    ip.ups_fast = (pow2 && L.w == 2 * prev_w && L.h == 2 * prev_h) ? 1 : 0;
                 }
             } else {
                 ip.flow_in = (const float2*)(ws + L.off_flow[(it - 1) & 1]);
@@ -480,18 +475,14 @@ int ofc_flow_plan_create(ofc_flow_plan** out, int width, int height, int max_fra
     pl->d_taps = (float*)d;
     rc = check_cuda(cudaMemcpy(pl->d_taps, all_taps.data(), all_taps.size() * sizeof(float), cudaMemcpyHostToDevice), "cudaMemcpy(taps)");
     if (rc != OFC_OK) { cudaFree(d); delete pl; return rc; }
-    {
-        const char* e = getenv("OFC_OVERLAP");
-        if (!(e && atoi(e) == 0)) {
-            if (cudaStreamCreateWithFlags(&pl->side, cudaStreamNonBlocking) != cudaSuccess) pl->side = nullptr;
-            if (pl->side) {
-                bool ok = cudaEventCreateWithFlags(&pl->ev_fork, cudaEventDisableTiming) == cudaSuccess;
-                pl->ev_level.resize(pl->lv.size());
-                for (size_t i = 0; ok && i < pl->lv.size(); ++i)
-                    ok = cudaEventCreateWithFlags(&pl->ev_level[i], cudaEventDisableTiming) == cudaSuccess;
-                if (!ok) { cudaStreamDestroy(pl->side); pl->side = nullptr; }
-            }
-        }
+    // the side stream of stage 1 (run_farneback); without it everything runs on the caller's stream
+    if (cudaStreamCreateWithFlags(&pl->side, cudaStreamNonBlocking) != cudaSuccess) pl->side = nullptr;
+    if (pl->side) {
+        bool ok = cudaEventCreateWithFlags(&pl->ev_fork, cudaEventDisableTiming) == cudaSuccess;
+        pl->ev_level.resize(pl->lv.size());
+        for (size_t i = 0; ok && i < pl->lv.size(); ++i)
+            ok = cudaEventCreateWithFlags(&pl->ev_level[i], cudaEventDisableTiming) == cudaSuccess;
+        if (!ok) { cudaStreamDestroy(pl->side); pl->side = nullptr; }
     }
     *out = pl;
     return OFC_OK;

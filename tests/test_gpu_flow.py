@@ -362,15 +362,14 @@ def _flow_with_env(monkeypatch, env, W, H, gray, levels=3):
 
 
 @pytest.mark.parametrize("size,levels", [((1080, 1920), 3), ((720, 1280), 3), ((2160, 3840), 5)])
-def test_pyramid_prefilter_and_fused_upsample_bit_identical(ofc, size, levels, monkeypatch):
-    """one-launch pyramid pre-filter == per-level tile kernels (I of every level, bit for bit), and the coarse flow
-    up-sampled inside the TMEM walk == the separate up-sample launch (final flow, bit for bit)"""
+def test_pyramid_prefilter_bit_identical(ofc, size, levels, monkeypatch):
+    """one-launch pyramid pre-filter == per-level tile kernels: I of every level and the final flow, bit for bit"""
     from opticalflowclustering_b200.flow import bgr2gray
     from opticalflowclustering_b200.synthetic import synthetic_clip
     H, W = size
     gray = bgr2gray(synthetic_clip(2, H, W, seed=31, device="cuda"))
-    new, inew = _flow_with_env(monkeypatch, {"OFC_PREFILTER_PYR": "1", "OFC_FUSE_UPSAMPLE": "1"}, W, H, gray, levels)
-    old, iold = _flow_with_env(monkeypatch, {"OFC_PREFILTER_PYR": "0", "OFC_FUSE_UPSAMPLE": "0"}, W, H, gray, levels)
+    new, inew = _flow_with_env(monkeypatch, {"OFC_PREFILTER_PYR": "1"}, W, H, gray, levels)
+    old, iold = _flow_with_env(monkeypatch, {"OFC_PREFILTER_PYR": "0"}, W, H, gray, levels)
     for a, b in zip(inew, iold):
         assert torch.equal(a, b)
     assert torch.equal(new, old)

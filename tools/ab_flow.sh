@@ -1,6 +1,6 @@
 #!/bin/bash
 # A/B of kernel switches on one B200: each line "NAME VAR=VAL ..." runs the short bench in a fresh process and prints
-# pairs/s plus the per-kernel times.  Usage: bash tools/ab_flow.sh <tag> "base" "f64 OFC_SOLVE_F64=1" ...
+# pairs/s plus the per-kernel times.  Usage: bash tools/ab_flow.sh <tag> "base" "noshare OFC_TMEM_SHARE=0" ...
 TAG=$1; shift
 export PYTHONPATH=.
 mkdir -p gpurun_out
