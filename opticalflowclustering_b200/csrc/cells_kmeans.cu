@@ -88,11 +88,13 @@ template <int SEL> __device__ __forceinline__ unsigned spread2(unsigned w) {
 
 }  // namespace
 
-#ifndef OFC_CELLS_MINB
-#define OFC_CELLS_MINB 3         // CTAs per SM the compiler must allow for (80 registers at 3; 64 at 4 spills 316 bytes)
-#endif
-template <int KP, int RU, bool PACK>
-__global__ void __launch_bounds__(256, ((KP <= 4 || RU == 2) ? OFC_CELLS_MINB : 2)) kmeans_cells_fast_kernel(KmCellsFastParams p) {
+// KP = 8 steps two rows per thread with the plain label chain, so it fits 80 registers = 3 CTAs per SM (64 registers
+// at 4 CTAs spill 316 bytes).  Measured on 1080p visualisation cells, k = 8 (r02f / r02g): 0.241 ms per frame, against
+// 0.264 with four rows per step and 0.285 with the index packed into the mantissa (one more ALU-pipe op per distance).
+template <int KP>
+__global__ void __launch_bounds__(256, KP <= 8 ? 3 : 2) kmeans_cells_fast_kernel(KmCellsFastParams p) {
+    constexpr int RU = KP == 8 ? 2 : 4;                   // rows per thread step of the E-step
+    constexpr bool PACK = KP != 8;                        // E-step arg-min index packed into the distances' low bits
     constexpr int D = 4;
     OFC_DYN_SMEM(unsigned char, smraw);
     const int n = p.n, k = p.k, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -292,9 +294,9 @@ __global__ void __launch_bounds__(256, ((KP <= 4 || RU == 2) ? OFC_CELLS_MINB : 
     // factor 2 on the dot product the total is < 3.7e6 u = 0.22 < E = 0.25.  ||x - c'||^2 and the centred float64
     // chain differ by a per-row constant (||x||^2 - ||x - mean||^2 terms cancel between clusters), and the float64
     // chain's own rounding (< 1e-9) is far inside the margin, so a filtered gap > MARGIN (below) fixes the arg-min.
-    // Four rows per thread step and no serial best/second chain: the distances of a row are independent, the
+    // RU rows per thread step and no serial best/second chain: the distances of a row are independent, the
     // minimum is a tree, the label the lowest index that attains it, and "near tie" = more than one distance within
-    // 1.0 of the minimum -- so a thread always has four rows' worth of independent arithmetic in flight.
+    // 1.0 of the minimum -- so a thread always has RU rows' worth of independent arithmetic in flight.
     auto e_step = [&](auto&& on_label) {
         float fx[KP], fy[KP], fz[KP], fw[KP], fq[KP];
 #pragma unroll
@@ -377,14 +379,15 @@ __global__ void __launch_bounds__(256, ((KP <= 4 || RU == 2) ? OFC_CELLS_MINB : 
     for (int j = tid; j < KP; j += 256) s_cnt[j] = 0;
     int iters = 0;
     bool strict = false;
-    int prev_changed = n;                                  // the first E-step labels every row
     for (int it = 0; it < p.max_iter; ++it) {
         prepare_centres();
         if (tid == 0) { s_changed = 0; s_nmoves = 0; }
-        // M-step mode of this iteration (same decision in every thread): while many labels still move, the sums are
-        // rebuilt from scratch in registers (16-bit fields, warp reductions -- no contended atomics); once few rows
-        // move, only those rows touch the sums.  Both are exact integer arithmetic, so the mode cannot change a bit.
-        const bool full = p.mstep_mode == 1 || (p.mstep_mode == 0 && (long long)prev_changed * 8 > n) || it == 0;
+        // M-step of this iteration: the first E-step labels every row, so its sums are built from scratch in registers
+        // (16-bit fields, warp reductions -- no contended atomics); every later iteration updates them from the rows
+        // whose label moved.  Both are exact integer arithmetic, so the choice cannot change a bit.  Measured on
+        // 350 x 5852 random rows (r02c): k = 3 / 8 / 16 -> 0.47 / 1.11 / 1.67 ms, against 0.53 / 1.49 / 2.32 ms
+        // rebuilding every iteration.
+        const bool full = it == 0;
         if (full) {
             for (int e = tid; e < KP * D; e += 256) s_sum[e] = 0u;
             for (int j = tid; j < KP; j += 256) s_cnt[j] = 0;
@@ -444,7 +447,6 @@ __global__ void __launch_bounds__(256, ((KP <= 4 || RU == 2) ? OFC_CELLS_MINB : 
         }
         if (changed) atomicAdd(&s_changed, changed);
         __syncthreads();
-        prev_changed = s_changed;
         // empty clusters take the farthest points (squared distance to the old centre of their label); the labels
         // stay as they are (_k_means_common.pyx:167-211), so the moves are undone on the running sums below.
         // The member counts are final behind the barrier above: every thread tests them itself (no flag, no barrier)
@@ -784,9 +786,7 @@ __global__ void __launch_bounds__(256, 2) kmeans_step_u8d4_kernel(KmAssignParams
 bool kmeans_step_u8d4_usable(const KmAssignParams& p, int batch) {
     if (p.dtype != DT_U8 || p.d != 4 || p.k < 1 || p.k > 8) return false;
     if (((uintptr_t)p.X & 15) || ((uintptr_t)p.labels & 15) || (p.prev_labels && ((uintptr_t)p.prev_labels & 15))) return false;
-    if (batch > 1 && (p.n & 3)) return false;                      // the next problem's rows would be misaligned
-    const char* e = getenv("OFC_KMEANS_STEP_FAST");
-    return !(e && atoi(e) == 0);
+    return batch <= 1 || (p.n & 3) == 0;                           // else the next problem's rows would be misaligned
 }
 
 int launch_kmeans_step_u8d4(const KmAssignParams& p, int batch, int grid, double* partial, long long* cnt_partial, void* stream) {
@@ -797,11 +797,6 @@ int launch_kmeans_step_u8d4(const KmAssignParams& p, int batch, int grid, double
     }
     OFC_CHECK_LAUNCH("kmeans_step_u8d4");
     return OFC_OK;
-}
-
-static int env_int_cells(const char* name, int dflt) {
-    const char* e = getenv(name);
-    return e ? atoi(e) : dflt;
 }
 
 // shared memory of one CTA; *closest_in_smem says whether the k-means++ scratch fits as well
@@ -833,32 +828,19 @@ int launch_kmeans_cells_fast(KmCellsFastParams p, int batch, void* stream) {
     int in_smem = 0;
     const size_t smem = cells_fast_smem(p.n, kp, p.init == nullptr, &in_smem);
     p.closest_in_smem = in_smem;
-    // 2 (default): the first iteration rebuilds the sums in registers, every later one updates them from the rows whose
-    // label moved; 1: always rebuild; 0: rebuild while more than 1/8 of the rows move.  Measured on 350 x 5852 random
-    // rows (r02c): k = 3 / 8 / 16 -> 0.47 / 1.11 / 1.67 ms incremental, 0.53 / 1.49 / 2.32 ms always rebuilding
-    p.mstep_mode = env_int_cells("OFC_CELLS_MSTEP", 2);
     if (p.init == nullptr && !in_smem && p.closest_ws == nullptr) {
         set_error("k-means++ seeding of %d-row cells needs %zu bytes of workspace", p.n, (size_t)batch * p.n * 4);
         return OFC_ERR_WORKSPACE;
     }
     ProfScope prof(PK_KMEANS, stream);
-#define OFC_CELLS_FAST(KPV, RUV, PK)                                                                        \
-    {                                                                                                       \
-        OFC_SMEM_OPTIN((kmeans_cells_fast_kernel<KPV, RUV, PK>), smem);                                     \
-        OFC_LAUNCH((kmeans_cells_fast_kernel<KPV, RUV, PK>), dim3(batch), dim3(256), smem, stream, p);      \
+#define OFC_CELLS_FAST(KPV)                                                                     \
+    {                                                                                           \
+        OFC_SMEM_OPTIN((kmeans_cells_fast_kernel<KPV>), smem);                                  \
+        OFC_LAUNCH((kmeans_cells_fast_kernel<KPV>), dim3(batch), dim3(256), smem, stream, p);   \
     }
-    // tuning switches for the k <= 8 form (rows per thread step, index-in-mantissa arg-min)
-    // measured on 1080p visualisation cells, k = 8 (r02f / r02g): 0.264 ms per frame with 4 rows per step and the plain
-    // label chain, 0.285 with the index packed into the mantissa (one more ALU-pipe op per distance); 2 rows per step
-    // fit 80 registers = 3 CTAs per SM: 0.241 ms (default)
-    const int ru = env_int_cells("OFC_CELLS_RU", 2), pack = env_int_cells("OFC_CELLS_PACK", 0);
-    if (kp == 4) OFC_CELLS_FAST(4, 4, true)
-    else if (kp == 8) {
-        if (ru == 2 && pack) OFC_CELLS_FAST(8, 2, true)
-        else if (ru == 2) OFC_CELLS_FAST(8, 2, false)
-        else if (pack) OFC_CELLS_FAST(8, 4, true)
-        else OFC_CELLS_FAST(8, 4, false)
-    } else OFC_CELLS_FAST(16, 4, true)
+    if (kp == 4) OFC_CELLS_FAST(4)
+    else if (kp == 8) OFC_CELLS_FAST(8)
+    else OFC_CELLS_FAST(16)
 #undef OFC_CELLS_FAST
     OFC_CHECK_LAUNCH("kmeans_cells_fast");
     return OFC_OK;

@@ -352,7 +352,7 @@ __global__ void __launch_bounds__(256) kmeans_sums_kernel(KmSumsParams p) {
 // fold over CTAs give the same bits as kmeans_sums_kernel in any order; X is read once per
 // iteration instead of twice and no floating-point atomic exists anywhere.
 // ---------------------------------------------------------------------------
-template <int DP, int KREG>
+template <int DP>
 __global__ void __launch_bounds__(256) kmeans_step_u8_kernel(KmAssignParams p, double* __restrict__ partial,
                                                              long long* __restrict__ cnt_partial) {
     OFC_DYN_SMEM(unsigned char, raw);
@@ -374,15 +374,6 @@ __global__ void __launch_bounds__(256) kmeans_step_u8_kernel(KmAssignParams p, d
     int32_t* labels = p.labels + (int64_t)b * p.n;
     const int32_t* prev = p.prev_labels ? p.prev_labels + (int64_t)b * p.n : nullptr;
     unsigned changed = 0;
-    double creg[KREG > 0 ? KREG : 1][DP], c2reg[KREG > 0 ? KREG : 1];
-    if (KREG > 0) {
-#pragma unroll
-        for (int j = 0; j < KREG; ++j) {
-            c2reg[j] = j < k ? sc2[j] : 0.0;
-#pragma unroll
-            for (int t = 0; t < DP; ++t) creg[j][t] = j < k ? sc[j * d + t] : 0.0;
-        }
-    }
     for (int64_t base = (int64_t)blockIdx.x * 256; base < p.n; base += (int64_t)gridDim.x * 256) {
         const int64_t i = base + tid;
         if (i < p.n) {
@@ -400,28 +391,14 @@ __global__ void __launch_bounds__(256) kmeans_step_u8_kernel(KmAssignParams p, d
             for (int t = 0; t < DP; ++t) x[t] = t < d ? (double)xr[t] - smean[t] : 0.0;
             double best = 0.0;
             int label = 0;
-            if (KREG > 0) {
-                // the reference's pixel shape (d = 4, k <= 8): centres and norms live in registers
+            for (int j = 0; j < k; ++j) {
+                const double* c = sc + j * d;
+                double dot = 0.0;
 #pragma unroll
-                for (int j = 0; j < KREG; ++j) {
-                    if (j < k) {
-                        double dot = 0.0;
-#pragma unroll
-                        for (int t = 0; t < DP; ++t) dot = fma(x[t], creg[j][t], dot);
-                        const double dist = fma(-2.0, dot, c2reg[j]);
-                        if (j == 0 || dist < best) { best = dist; label = j; }
-                    }
-                }
-            } else {
-                for (int j = 0; j < k; ++j) {
-                    const double* c = sc + j * d;
-                    double dot = 0.0;
-#pragma unroll
-                    for (int t = 0; t < DP; ++t)
-                        if (t < d) dot = fma(x[t], c[t], dot);
-                    const double dist = fma(-2.0, dot, sc2[j]);
-                    if (j == 0 || dist < best) { best = dist; label = j; }
-                }
+                for (int t = 0; t < DP; ++t)
+                    if (t < d) dot = fma(x[t], c[t], dot);
+                const double dist = fma(-2.0, dot, sc2[j]);
+                if (j == 0 || dist < best) { best = dist; label = j; }
             }
             labels[i] = label;
             if (prev && prev[i] != label) ++changed;
@@ -1466,9 +1443,9 @@ int launch_kmeans_assign(KmAssignParams p, int batch, double* c2_ws, void* strea
     const int parts = kmeans_assign_grid(p.n);
     if ((int)grid.x > parts) grid.x = parts;
     // centres fit shared memory and the row fits a warp's registers: same arithmetic, X read once
-    static const int use_medium = getenv("OFC_KMEANS_MEDIUM") ? atoi(getenv("OFC_KMEANS_MEDIUM")) : 1;
+    // (test seam: OFC_KMEANS_MEDIUM=0 runs the generic kernel, the tests' reference)
     const size_t msmem = ((size_t)p.k * p.d + p.k) * wsz;
-    if (use_medium && p.d <= 512 && msmem <= 200 * 1024) {
+    if (!seam_off("OFC_KMEANS_MEDIUM") && p.d <= 512 && msmem <= 200 * 1024) {
 #define OFC_KM_MED(TT, WW, NTV)                                                                                        \
     {                                                                                                                  \
         OFC_SMEM_OPTIN((kmeans_assign_medium_kernel<TT, WW, NTV>), msmem);                                             \
@@ -1546,23 +1523,21 @@ int launch_kmeans_step_u8(KmAssignParams p, int batch, double* partial, long lon
     if (p.d > 32 || smem > 200 * 1024) { set_error("fused k-means step: shape d=%d k=%d does not fit shared memory", p.d, p.k); return OFC_ERR_UNSUPPORTED; }
     const int grid = kmeans_step_grid(p.n, batch);
     ProfScope prof(PK_KMEANS, stream);
-#define OFC_KM_STEP(DPV, KR)                                                                                                \
-    {                                                                                                                     \
-        OFC_SMEM_OPTIN((kmeans_step_u8_kernel<DPV, KR>), smem);                                                           \
-        OFC_LAUNCH((kmeans_step_u8_kernel<DPV, KR>), dim3(grid, batch), dim3(256), smem, stream, p, partial, cnt_partial); \
+#define OFC_KM_STEP(DPV)                                                                                                \
+    {                                                                                                                 \
+        OFC_SMEM_OPTIN((kmeans_step_u8_kernel<DPV>), smem);                                                           \
+        OFC_LAUNCH((kmeans_step_u8_kernel<DPV>), dim3(grid, batch), dim3(256), smem, stream, p, partial, cnt_partial); \
     }
-    // (register-resident centres, KREG = 8, measured slower at d = 4, k = 8: 1.15 vs 0.75 ms per 64 M rows -- the
-    // 64 extra registers cost more occupancy than the shared-memory broadcasts they save)
-    static const int kreg = getenv("OFC_KMEANS_STEP_KREG") ? atoi(getenv("OFC_KMEANS_STEP_KREG")) : 0;
+    // Centres stay in shared memory at every d.  (Centres held in registers were measured slower at d = 4, k = 8: 1.15
+    // against 0.75 ms per 64 M rows -- the 64 extra registers cost more occupancy than the broadcasts they save.)
     if (kmeans_step_u8d4_usable(p, batch)) {
         // the reference's pixel shape: float32-filtered E-step + packed register M-step, same bits (cells_kmeans.cu)
         int rc = launch_kmeans_step_u8d4(p, batch, grid, partial, cnt_partial, stream);
         if (rc != OFC_OK) return rc;
-    } else if (kreg && p.d == 4 && p.k <= 8) OFC_KM_STEP(4, 8)
-    else if (p.d <= 4) OFC_KM_STEP(4, 0)
-    else if (p.d <= 8) OFC_KM_STEP(8, 0)
-    else if (p.d <= 16) OFC_KM_STEP(16, 0)
-    else OFC_KM_STEP(32, 0)
+    } else if (p.d <= 4) OFC_KM_STEP(4)
+    else if (p.d <= 8) OFC_KM_STEP(8)
+    else if (p.d <= 16) OFC_KM_STEP(16)
+    else OFC_KM_STEP(32)
 #undef OFC_KM_STEP
     OFC_CHECK_LAUNCH("kmeans_step_u8");
     const int64_t kd = (int64_t)p.k * p.d;

@@ -92,7 +92,6 @@ struct KmCellsFastParams {
     unsigned char* dom_hue;        // [batch]    BGR2HSV hue of its first three channels, or null
     unsigned* closest_ws;          // [batch][n] k-means++ scratch when it does not fit shared memory
     int closest_in_smem;           // set by the launcher
-    int mstep_mode;                // set by the launcher (OFC_CELLS_MSTEP)
 };
 bool kmeans_cells_fast_supported(int64_t n, int d, int k);
 size_t kmeans_cells_fast_workspace(int batch, int64_t n, int k, bool seeding);

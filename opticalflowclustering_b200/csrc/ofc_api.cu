@@ -882,10 +882,8 @@ int ofc_kmeans_cells(const uint8_t* X, int batch, int64_t n, int d, int k, const
         return OFC_ERR_WORKSPACE;
     }
     // the reference's own shape (4 channels, small k) runs the shared-memory / filtered form (cells_kmeans.cu):
-    // same labels, centres, n_iter, counts and inertia, bit for bit (OFC_CELLS_FAST=0 keeps the first kernel)
-    const char* fast_env = getenv("OFC_CELLS_FAST");          // read per call: tests compare both kernels in one process
-    const bool fast_on = !(fast_env && atoi(fast_env) == 0);
-    if (fast_on && kmeans_cells_fast_supported(n, d, k)) {
+    // same labels, centres, n_iter, counts and inertia, bit for bit (test seam: OFC_CELLS_FAST=0 keeps the first kernel)
+    if (!seam_off("OFC_CELLS_FAST") && kmeans_cells_fast_supported(n, d, k)) {
         KmCellsFastParams p;
         memset(&p, 0, sizeof(p));
         p.X = X; p.n = (int)n; p.k = k; p.init = init; p.seed = seed; p.problem_offset = 0; p.max_iter = max_iter; p.tol = tol;

@@ -11,6 +11,7 @@
 
 #include <stdint.h>
 #include <stddef.h>
+#include <stdlib.h>
 
 #ifndef OFC_EMULATE
 #include <cuda_runtime.h>
@@ -78,6 +79,13 @@ struct ProfScope {
     ~ProfScope();
 };
 extern int g_prof_level;         // pyramid level (0 = finest) of the flow_iter launch being issued
+
+// Test seam (DESIGN §5a.5): true when the environment variable `name` is set to 0, which selects the form a fast
+// kernel replaced and gives the same bits.  Read on every call, so one process can run and compare both forms.
+static inline bool seam_off(const char* name) {
+    const char* e = getenv(name);
+    return e && atoi(e) == 0;
+}
 
 static inline double host_dmul(double a, double b) { volatile double r = a * b; return r; }
 static inline double host_dadd(double a, double b) { volatile double r = a + b; return r; }

@@ -832,11 +832,10 @@ template <int BN>
 int launch_tc(const CUtensorMap& tmAh, const CUtensorMap& tmAl, const CUtensorMap& tmBh, const CUtensorMap& tmBl, TcParams p,
               void* stream) {
     // centre-resident form when one centre tile covers all k and the resident tiles leave room for >= 2 row stages
-    static const int want_bres = getenv("OFC_TC_BRES") ? atoi(getenv("OFC_TC_BRES")) : 1;
     const int n_ktiles = (p.d + BK - 1) / BK;
     const size_t bres_bytes = (size_t)n_ktiles * 2 * TcCfg<BN>::B_BYTES;
     const size_t budget = 200 * 1024;
-    if (want_bres && p.k <= BN && bres_bytes + 2 * (2 * TcCfg<BN>::A_BYTES) <= budget) {
+    if (p.k <= BN && bres_bytes + 2 * (2 * TcCfg<BN>::A_BYTES) <= budget) {
         int st = (int)((budget - bres_bytes) / (2 * TcCfg<BN>::A_BYTES));
         if (st > MAX_STAGES) st = MAX_STAGES;
         p.stages = st;
@@ -919,14 +918,13 @@ static int tc_assign_impl(const float* Xh, const float* Xl, const float* xnorm, 
     TcParams p;
     p.n = n; p.d = d; p.k = k; p.c2 = c2; p.xnorm = xnorm; p.cmax = cmax;
     // per distance: 2 |x| |c| (2^-19 split remainder + d 2^-23 accumulation); two distances; x1.5 margin
-    static const float tol_mul = getenv("OFC_TC_TOL_MUL") ? (float)atof(getenv("OFC_TC_TOL_MUL")) : 1.5f;
-    p.tol_scale = tol_mul * 4.f * (1.f / 524288.f + (float)d * (1.f / 8388608.f));
+    p.tol_scale = 1.5f * 4.f * (1.f / 524288.f + (float)d * (1.f / 8388608.f));
     p.tol_c2 = 0.f;
     if (X8) {
         // against the float64 distance of the bytes: also the float32 rounding of the centred row and of the centres
         // (2 x 2^-24 |x| |c| per dot product) and of the squared norms / the final fma (2^-24 (c2 + |dist|) each)
-        p.tol_scale = tol_mul * 4.f * (1.f / 524288.f + 1.f / 4194304.f + (float)d * (1.f / 8388608.f));
-        p.tol_c2 = tol_mul * 4.f * (1.f / 8388608.f);
+        p.tol_scale = 1.5f * 4.f * (1.f / 524288.f + 1.f / 4194304.f + (float)d * (1.f / 8388608.f));
+        p.tol_c2 = 1.5f * 4.f * (1.f / 8388608.f);
     }
     p.labels = labels; p.amb = (int4*)(ws + w.off_amb); p.amb_count = count; p.error_flag = err;
     if (BN == 64) rc = launch_tc<64>(tmAh, tmAl, tmBh, tmBl, p, stream);

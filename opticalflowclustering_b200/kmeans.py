@@ -204,12 +204,6 @@ class TensorCoreSteps:
     precision (float32 rows: float32; uint8 rows: float64 on the original bytes), so the labels are those
     of the CUDA-core E-step; the M-step walks a label-sorted member list (uint8: exact integer sums)."""
 
-    @staticmethod
-    def usable(st: "LloydState") -> bool:
-        return (_TEST_LIBRARY is None and st.X.is_cuda and st.dtype in (0, 1) and st.B == 1 and st.d > 32 and st.d % 4 == 0
-                and 2 <= st.k <= 4096 and st.n < 2 ** 31 and _tc_worth_it(st.dtype, st.d, st.k)
-                and os.environ.get("OFC_KMEANS_TC", "1") != "0")
-
     def __init__(self, st: "LloydState", mean: torch.Tensor):
         self.st = st
         c = st.ctx
@@ -258,9 +252,11 @@ def _tc_worth_it(dtype: int, d: int, k: int) -> bool:
 
 
 def _tc_wanted(Xb, k) -> bool:
-    return (_TEST_LIBRARY is None and Xb.is_cuda and Xb.dtype in (torch.float32, torch.uint8) and Xb.shape[0] == 1
-            and Xb.shape[2] > 32 and Xb.shape[2] % 4 == 0 and 2 <= k <= 4096
-            and _tc_worth_it(_DT[Xb.dtype], int(Xb.shape[2]), k) and os.environ.get("OFC_KMEANS_TC", "1") != "0")
+    """does the fit of ``Xb`` ([B, n, d]) with k clusters run its E/M steps on the tensor cores (TensorCoreSteps)?"""
+    B, n, d = (int(s) for s in Xb.shape)
+    return (_TEST_LIBRARY is None and Xb.is_cuda and Xb.dtype in (torch.float32, torch.uint8) and B == 1
+            and d > 32 and d % 4 == 0 and 2 <= k <= 4096 and n < 2 ** 31
+            and _tc_worth_it(_DT[Xb.dtype], d, k) and os.environ.get("OFC_KMEANS_TC", "1") != "0")
 
 
 def _relocate_across_ranks(st: "LloydState", mean, labels, centres_old, sums, counts, raw_sums: bool, group, row_offset: int):
@@ -391,7 +387,8 @@ def lloyd(X, init, max_iter: int = 300, tol: float = 1e-4, group=None, _host_rel
     k = int(init.shape[1])
     if init.shape[0] != B or init.shape[2] != d:
         raise ValueError(f"init shape {tuple(init.shape)} does not match X {tuple(Xb.shape)}")
-    st = LloydState(ctx, Xb, k, ws_k=1 if _tc_wanted(Xb, k) else None)
+    use_tc = _tc_wanted(Xb, k)
+    st = LloydState(ctx, Xb, k, ws_k=1 if use_tc else None)
     dev = Xb.device
     row_offset, n_total = 0, n
     if group is not None:
@@ -414,7 +411,7 @@ def lloyd(X, init, max_iter: int = 300, tol: float = 1e-4, group=None, _host_rel
     if is_f32:
         centres = centres.to(torch.float32).to(torch.float64).contiguous()
     # dense float32 corner (d > 32): E/M steps on the tensor-core path, same labels as the float32 kernels
-    tc = TensorCoreSteps(st, mean[0].contiguous()) if TensorCoreSteps.usable(st) else None
+    tc = TensorCoreSteps(st, mean[0].contiguous()) if use_tc else None
     fused = tc is None and is_u8 and st.step_supported()
 
     active = st.active
@@ -519,12 +516,8 @@ def lloyd(X, init, max_iter: int = 300, tol: float = 1e-4, group=None, _host_rel
     heavy = tc is not None and float(n) * k * d >= 1e9
     if heavy and lag:
         lag = 1
-    # under a process group the captured iteration contains the NCCL collectives as well (torch.distributed's NCCL ops
-    # are capturable once the communicator is warm -- the two eager iterations); OFC_KMEANS_GRAPH_NCCL=0 keeps that
-    # path eager
     use_graph = (is_cuda and _TEST_LIBRARY is None and max_iter >= 8 and not heavy and os.environ.get("OFC_KMEANS_GRAPH", "1") != "0"
-                 and (group is None or px is not None
-                      or (not _host_relocation and os.environ.get("OFC_KMEANS_GRAPH_NCCL", "0") == "1")))
+                 and (group is None or px is not None))
     it = 0
     done = False
     n_eager = min(max_iter, _EAGER_ITERATIONS) if use_graph else max_iter

@@ -52,8 +52,7 @@ class ClipPipeline:
         self.km_centre = torch.empty((P, self.cells, 4), dtype=torch.uint8, device=dev)
         self.km_hue = torch.empty((P, self.cells), dtype=torch.uint8, device=dev)
         self.keep_viz = keep_viz
-        import os
-        self.fuse_grid = os.environ.get("OFC_FUSE_GRID", "1") != "0"
+        self.fuse_grid = True            # False runs the visualisation and the grid pass as two kernels (same bytes)
         self.n_clusters = int(n_clusters)
         if self.n_clusters < 1:
             raise ValueError("n_clusters must be >= 1")

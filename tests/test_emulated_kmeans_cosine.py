@@ -185,34 +185,19 @@ def test_fused_uint8_step_equals_two_kernel_iteration(L, shape, monkeypatch):
     assert all(torch.equal(x, y) for x, y in zip(a, b))
 
 
-def test_medium_assign_kernel_equals_generic(L):
+def test_medium_assign_kernel_equals_generic(L, monkeypatch):
     """kmeans_assign_medium_kernel (centres in shared memory, row in registers) keeps the generic kernel's arithmetic
-    order: whole fits must be bit-identical.  The switch is read once per process, hence two child processes."""
-    import subprocess
-    import sys
-    code = r'''
-import os, sys, hashlib, numpy as np
-sys.path.insert(0, os.getcwd())
-from tests.emu import emu_lib as E
-from opticalflowclustering_b200 import kmeans as km
-km._use_test_library(E.lib())
-rng = np.random.default_rng(2)
-h = hashlib.sha256()
-for dt, (n, d, k, B) in [(np.uint8, (260, 350, 8, 1)), (np.float32, (300, 70, 9, 2)), (np.float64, (200, 130, 5, 1)),
-                         (np.uint8, (200, 33, 12, 1))]:
-    X = (rng.integers(0, 256, (B, n, d)) if dt == np.uint8 else rng.normal(0, 3, (B, n, d))).astype(dt)
-    for t in km.lloyd(X, X[:, :k].astype(np.float64), max_iter=4):
-        h.update(t.cpu().numpy().tobytes())
-print(h.hexdigest())
-'''
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    digests = []
-    for flag in ("0", "1"):
-        env = dict(os.environ, OFC_KMEANS_MEDIUM=flag, OFC_KMEANS_TC="0")
-        r = subprocess.run([sys.executable, "-c", code], cwd=root, env=env, capture_output=True, text=True, timeout=900)
-        assert r.returncode == 0, r.stderr[-2000:]
-        digests.append(r.stdout.strip().splitlines()[-1])
-    assert digests[0] == digests[1]
+    order: whole fits must be bit-identical"""
+    rng = np.random.default_rng(2)
+    for dt, (n, d, k, B) in [(np.uint8, (260, 350, 8, 1)), (np.float32, (300, 70, 9, 2)), (np.float64, (200, 130, 5, 1)),
+                             (np.uint8, (200, 33, 12, 1))]:
+        X = (rng.integers(0, 256, (B, n, d)) if dt == np.uint8 else rng.normal(0, 3, (B, n, d))).astype(dt)
+        init = X[:, :k].astype(np.float64)
+        monkeypatch.setenv("OFC_KMEANS_MEDIUM", "0")
+        a = km.lloyd(X, init, max_iter=4)
+        monkeypatch.setenv("OFC_KMEANS_MEDIUM", "1")
+        b = km.lloyd(X, init, max_iter=4)
+        assert all(torch.equal(x, y) for x, y in zip(a, b)), (dt, n, d, k, B)
 
 
 def test_sliding_cosine_goldens(L):
