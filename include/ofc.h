@@ -168,6 +168,14 @@ int ofc_draw_grid(uint8_t* bgr, int n_frames, int height, int width, int rows, i
 #define OFC_U8 0
 #define OFC_F32 1
 #define OFC_F64 2
+/* OR-ed into the dtype of ofc_kmeans_assign / _sums / _step / _relocate (and accepted by
+ * ofc_kmeans_step_supported): every problem of the batch reads the same X [n][d] -- several
+ * starts of one fit (KMeans n_init) without a copy of the rows per start.  Everything else
+ * (centres, labels, sums, ...) stays per problem.  A problem's results are the bits it gets
+ * when run alone (batch = 1).  Such a batch needs at most batch * ofc_kmeans_workspace_bytes(1, n, d, k)
+ * bytes of workspace.  ofc_kmeans_far_points / _far_payload (row-sharded fits) return
+ * OFC_ERR_UNSUPPORTED for it. */
+#define OFC_KMEANS_SHARED_ROWS 0x100
 
 size_t ofc_kmeans_workspace_bytes(int batch, int64_t n, int d, int k);
 /* the (small) prefix of that workspace ofc_kmeans_assign and ofc_kmeans_centres need on their own */

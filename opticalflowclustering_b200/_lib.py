@@ -12,6 +12,8 @@ PKG = os.path.dirname(os.path.abspath(__file__))
 SO = os.path.join(PKG, "libofc.so")
 
 OFC_OK, OFC_ERR_INVALID, OFC_ERR_UNSUPPORTED, OFC_ERR_CUDA, OFC_ERR_WORKSPACE = 0, -1, -2, -3, -4
+#: OR-ed into the dtype of the stepwise k-means calls: every problem of the batch reads the same rows
+OFC_KMEANS_SHARED_ROWS = 0x100
 
 _vp, _i, _i64, _sz, _d = C.c_void_p, C.c_int, C.c_int64, C.c_size_t, C.c_double
 

@@ -705,7 +705,7 @@ __global__ void __launch_bounds__(256, 2) kmeans_step_u8d4_kernel(KmAssignParams
     };
 
     const int64_t n = p.n, n4 = n >> 2;
-    const uint4* X4 = reinterpret_cast<const uint4*>(reinterpret_cast<const unsigned char*>(p.X) + (int64_t)b * n * D);
+    const uint4* X4 = reinterpret_cast<const uint4*>(reinterpret_cast<const unsigned char*>(p.X) + (int64_t)b * p.x_stride);
     int4* L4 = reinterpret_cast<int4*>(p.labels + (int64_t)b * n);
     const int4* P4 = p.prev_labels ? reinterpret_cast<const int4*>(p.prev_labels + (int64_t)b * n) : nullptr;
     unsigned a0[KP], a1[KP], ac[KP];
@@ -765,7 +765,7 @@ __global__ void __launch_bounds__(256, 2) kmeans_step_u8d4_kernel(KmAssignParams
     // the n % 4 last rows: scalar, exact chain
     if (blockIdx.x == 0 && tid < (int)(n & 3)) {
         const int64_t i = (n4 << 2) + tid;
-        const unsigned w = reinterpret_cast<const unsigned*>(reinterpret_cast<const unsigned char*>(p.X) + (int64_t)b * n * D)[i];
+        const unsigned w = reinterpret_cast<const unsigned*>(reinterpret_cast<const unsigned char*>(p.X) + (int64_t)b * p.x_stride)[i];
         const int label = exact_label(w);
         p.labels[(int64_t)b * n + i] = label;
         if (p.prev_labels && p.prev_labels[(int64_t)b * n + i] != label) ++changed;

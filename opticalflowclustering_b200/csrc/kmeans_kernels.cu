@@ -73,7 +73,7 @@ __global__ void __launch_bounds__(256) kmeans_assign_small_kernel(KmAssignParams
     for (int j = tid; j < k; j += 256) sc2[j] = centre_norm_sq(sc + j * d, d);
     __syncthreads();
 
-    const T* X = reinterpret_cast<const T*>(p.X) + (int64_t)b * p.n * d;
+    const T* X = reinterpret_cast<const T*>(p.X) + (int64_t)b * p.x_stride;
     int32_t* labels = p.labels + (int64_t)b * p.n;
     const int32_t* prev = p.prev_labels ? p.prev_labels + (int64_t)b * p.n : nullptr;
     double inert = 0.0;
@@ -141,7 +141,7 @@ __global__ void __launch_bounds__(256) kmeans_assign_generic_kernel(KmAssignPara
     const double* cen = p.centres + (int64_t)b * k * d;
     const double* c2 = p.c2 + (int64_t)b * k;
     const double* mean = p.mean ? p.mean + (int64_t)b * d : nullptr;
-    const T* X = reinterpret_cast<const T*>(p.X) + (int64_t)b * p.n * d;
+    const T* X = reinterpret_cast<const T*>(p.X) + (int64_t)b * p.x_stride;
     int32_t* labels = p.labels + (int64_t)b * p.n;
     const int32_t* prev = p.prev_labels ? p.prev_labels + (int64_t)b * p.n : nullptr;
     double inert = 0.0;
@@ -211,7 +211,7 @@ __global__ void __launch_bounds__(256) kmeans_assign_medium_kernel(KmAssignParam
     W m[NT];
 #pragma unroll
     for (int u = 0; u < NT; ++u) { const int t = lane + 32 * u; m[u] = (mean && t < d) ? (W)mean[t] : (W)0; }
-    const T* X = reinterpret_cast<const T*>(p.X) + (int64_t)b * p.n * d;
+    const T* X = reinterpret_cast<const T*>(p.X) + (int64_t)b * p.x_stride;
     int32_t* labels = p.labels + (int64_t)b * p.n;
     const int32_t* prev = p.prev_labels ? p.prev_labels + (int64_t)b * p.n : nullptr;
     double inert = 0.0;
@@ -303,7 +303,7 @@ __global__ void __launch_bounds__(256) kmeans_sums_kernel(KmSumsParams p) {
     double* my = acc + (size_t)copy * kt * dt + t;
     int* mycnt = cnt + copy * kt;
     const double m = (p.mean && dim_ok) ? p.mean[(int64_t)b * d + dim] : 0.0;
-    const T* X = reinterpret_cast<const T*>(p.X) + (int64_t)b * p.n * d;
+    const T* X = reinterpret_cast<const T*>(p.X) + (int64_t)b * p.x_stride;
     const int32_t* labels = p.labels ? p.labels + (int64_t)b * p.n : nullptr;
 
     for (int k0 = 0; k0 < k; k0 += kt) {
@@ -370,7 +370,7 @@ __global__ void __launch_bounds__(256) kmeans_step_u8_kernel(KmAssignParams p, d
     __syncthreads();
     for (int j = tid; j < k; j += 256) sc2[j] = norm_sq_numpy_f64(sc + j * d, d);
     __syncthreads();
-    const unsigned char* X = reinterpret_cast<const unsigned char*>(p.X) + (int64_t)b * p.n * d;
+    const unsigned char* X = reinterpret_cast<const unsigned char*>(p.X) + (int64_t)b * p.x_stride;
     int32_t* labels = p.labels + (int64_t)b * p.n;
     const int32_t* prev = p.prev_labels ? p.prev_labels + (int64_t)b * p.n : nullptr;
     unsigned changed = 0;
@@ -626,7 +626,7 @@ __global__ void __launch_bounds__(256) kmeans_freeze_labels_kernel(int64_t n, co
 // unconditionally (no device->host round trip to decide).
 // ---------------------------------------------------------------------------
 template <typename T>
-__global__ void __launch_bounds__(1024) kmeans_relocate_kernel(const T* Xall, int64_t n, int d, int k, const double* mean_all,
+__global__ void __launch_bounds__(1024) kmeans_relocate_kernel(const T* Xall, int64_t x_stride, int64_t n, int d, int k, const double* mean_all,
                                                                 const int32_t* labels_all, const double* centres_all,
                                                                 double* sums_all, long long* counts_all,
                                                                 int raw_sums, const unsigned char* active) {
@@ -642,7 +642,7 @@ __global__ void __launch_bounds__(1024) kmeans_relocate_kernel(const T* Xall, in
     }
     __syncthreads();
     if (!s_any) return;
-    const T* X = Xall + (int64_t)b * n * d;
+    const T* X = Xall + (int64_t)b * x_stride;
     const int32_t* labels = labels_all + (int64_t)b * n;
     const double* cen = centres_all + (int64_t)b * k * d;
     const double* mean = mean_all ? mean_all + (int64_t)b * d : nullptr;
@@ -711,7 +711,7 @@ __global__ void __launch_bounds__(1024) kmeans_relocate_kernel(const T* Xall, in
 // launch on 1 M x 128 float32 rows with a handful of empty clusters (ncu r02e) against ~1 ms this way.
 // ---------------------------------------------------------------------------
 template <typename T>
-__global__ void __launch_bounds__(256) kmeans_rowdist_kernel(const T* Xall, int64_t n, int d, int k, const double* mean_all,
+__global__ void __launch_bounds__(256) kmeans_rowdist_kernel(const T* Xall, int64_t x_stride, int64_t n, int d, int k, const double* mean_all,
                                                              const int32_t* labels_all, const double* centres_all,
                                                              const long long* counts_all, double* scratch_all, int force,
                                                              const unsigned char* active) {
@@ -728,7 +728,7 @@ __global__ void __launch_bounds__(256) kmeans_rowdist_kernel(const T* Xall, int6
         __syncthreads();
         if (!s_any) return;
     }
-    const T* X = Xall + (int64_t)b * n * d;
+    const T* X = Xall + (int64_t)b * x_stride;
     const int32_t* labels = labels_all + (int64_t)b * n;
     const double* cen = centres_all + (int64_t)b * k * d;
     const double* mean = mean_all ? mean_all + (int64_t)b * d : nullptr;
@@ -773,7 +773,7 @@ __device__ __forceinline__ void block_argmax_1024(const double* scratch, int64_t
 }
 
 template <typename T>
-__global__ void __launch_bounds__(1024) kmeans_relocate_apply_kernel(const T* Xall, int64_t n, int d, int k, const double* mean_all,
+__global__ void __launch_bounds__(1024) kmeans_relocate_apply_kernel(const T* Xall, int64_t x_stride, int64_t n, int d, int k, const double* mean_all,
                                                                       const int32_t* labels_all, double* scratch_all, double* sums_all,
                                                                       long long* counts_all, int raw_sums, const unsigned char* active) {
     const int b = blockIdx.x, tid = threadIdx.x;
@@ -791,7 +791,7 @@ __global__ void __launch_bounds__(1024) kmeans_relocate_apply_kernel(const T* Xa
     }
     __syncthreads();
     if (!s_any) return;
-    const T* X = Xall + (int64_t)b * n * d;
+    const T* X = Xall + (int64_t)b * x_stride;
     const int32_t* labels = labels_all + (int64_t)b * n;
     const double* mean = mean_all ? mean_all + (int64_t)b * d : nullptr;
     double* sums = sums_all + (int64_t)b * k * d;
@@ -1639,16 +1639,16 @@ static int rowdist_grid(int64_t n, int batch) {
 }
 
 template <typename T>
-static int launch_rowdist(const void* X, int batch, int64_t n, int d, int k, const double* mean, const int32_t* labels,
+static int launch_rowdist(const void* X, int64_t x_stride, int batch, int64_t n, int d, int k, const double* mean, const int32_t* labels,
                           const double* centres_old, const long long* counts, double* scratch, int force,
                           const unsigned char* active, void* stream) {
-    OFC_LAUNCH(kmeans_rowdist_kernel<T>, dim3(rowdist_grid(n, batch), batch), dim3(256), 0, stream, (const T*)X, n, d, k, mean, labels,
+    OFC_LAUNCH(kmeans_rowdist_kernel<T>, dim3(rowdist_grid(n, batch), batch), dim3(256), 0, stream, (const T*)X, x_stride, n, d, k, mean, labels,
                centres_old, counts, scratch, force, active);
     OFC_CHECK_LAUNCH("kmeans_rowdist");
     return OFC_OK;
 }
 
-int launch_kmeans_relocate(const void* X, int dtype, int batch, int64_t n, int d, int k, const double* mean,
+int launch_kmeans_relocate(const void* X, int64_t x_stride, int dtype, int batch, int64_t n, int d, int k, const double* mean,
                            const int32_t* labels, const double* centres_old, double* sums, long long* counts,
                            int raw_sums, const unsigned char* active, double* scratch, void* stream) {
     if (batch <= 0) return OFC_OK;
@@ -1657,18 +1657,18 @@ int launch_kmeans_relocate(const void* X, int dtype, int batch, int64_t n, int d
     if (scratch) {
         // two kernels: distances by the whole grid, then the pick loop (see kmeans_rowdist_kernel)
         int rc;
-        if (dtype == DT_U8) rc = launch_rowdist<unsigned char>(X, batch, n, d, k, mean, labels, centres_old, counts, scratch, 0, active, stream);
-        else if (dtype == DT_F32) rc = launch_rowdist<float>(X, batch, n, d, k, mean, labels, centres_old, counts, scratch, 0, active, stream);
-        else rc = launch_rowdist<double>(X, batch, n, d, k, mean, labels, centres_old, counts, scratch, 0, active, stream);
+        if (dtype == DT_U8) rc = launch_rowdist<unsigned char>(X, x_stride, batch, n, d, k, mean, labels, centres_old, counts, scratch, 0, active, stream);
+        else if (dtype == DT_F32) rc = launch_rowdist<float>(X, x_stride, batch, n, d, k, mean, labels, centres_old, counts, scratch, 0, active, stream);
+        else rc = launch_rowdist<double>(X, x_stride, batch, n, d, k, mean, labels, centres_old, counts, scratch, 0, active, stream);
         if (rc != OFC_OK) return rc;
         if (dtype == DT_U8)
-            OFC_LAUNCH(kmeans_relocate_apply_kernel<unsigned char>, dim3(batch), dim3(1024), 0, stream, (const unsigned char*)X, n, d, k, mean,
+            OFC_LAUNCH(kmeans_relocate_apply_kernel<unsigned char>, dim3(batch), dim3(1024), 0, stream, (const unsigned char*)X, x_stride, n, d, k, mean,
                        labels, scratch, sums, counts, raw_sums, active);
         else if (dtype == DT_F32)
-            OFC_LAUNCH(kmeans_relocate_apply_kernel<float>, dim3(batch), dim3(1024), 0, stream, (const float*)X, n, d, k, mean, labels,
+            OFC_LAUNCH(kmeans_relocate_apply_kernel<float>, dim3(batch), dim3(1024), 0, stream, (const float*)X, x_stride, n, d, k, mean, labels,
                        scratch, sums, counts, raw_sums, active);
         else
-            OFC_LAUNCH(kmeans_relocate_apply_kernel<double>, dim3(batch), dim3(1024), 0, stream, (const double*)X, n, d, k, mean, labels,
+            OFC_LAUNCH(kmeans_relocate_apply_kernel<double>, dim3(batch), dim3(1024), 0, stream, (const double*)X, x_stride, n, d, k, mean, labels,
                        scratch, sums, counts, raw_sums, active);
         OFC_CHECK_LAUNCH("kmeans_relocate_apply");
         return OFC_OK;
@@ -1680,13 +1680,13 @@ int launch_kmeans_relocate(const void* X, int dtype, int batch, int64_t n, int d
     OFC_SMEM_OPTIN(kmeans_relocate_kernel<float>, smem);
     OFC_SMEM_OPTIN(kmeans_relocate_kernel<double>, smem);
     if (dtype == DT_U8)
-        OFC_LAUNCH(kmeans_relocate_kernel<unsigned char>, dim3(batch), dim3(1024), smem, stream, (const unsigned char*)X, n, d, k,
+        OFC_LAUNCH(kmeans_relocate_kernel<unsigned char>, dim3(batch), dim3(1024), smem, stream, (const unsigned char*)X, x_stride, n, d, k,
                    mean, labels, centres_old, sums, counts, raw_sums, active);
     else if (dtype == DT_F32)
-        OFC_LAUNCH(kmeans_relocate_kernel<float>, dim3(batch), dim3(1024), smem, stream, (const float*)X, n, d, k, mean, labels,
+        OFC_LAUNCH(kmeans_relocate_kernel<float>, dim3(batch), dim3(1024), smem, stream, (const float*)X, x_stride, n, d, k, mean, labels,
                    centres_old, sums, counts, raw_sums, active);
     else
-        OFC_LAUNCH(kmeans_relocate_kernel<double>, dim3(batch), dim3(1024), smem, stream, (const double*)X, n, d, k, mean, labels,
+        OFC_LAUNCH(kmeans_relocate_kernel<double>, dim3(batch), dim3(1024), smem, stream, (const double*)X, x_stride, n, d, k, mean, labels,
                    centres_old, sums, counts, raw_sums, active);
     OFC_CHECK_LAUNCH("kmeans_relocate");
     return OFC_OK;
@@ -1699,9 +1699,9 @@ int launch_kmeans_far_payload(const void* X, int dtype, int batch, int64_t n, in
     ProfScope prof(PK_KMEANS, stream);
     int rc = OFC_OK;
     if (n > 0) {
-        if (dtype == DT_U8) rc = launch_rowdist<unsigned char>(X, batch, n, d, k, mean, labels, centres_old, counts, scratch, 0, active, stream);
-        else if (dtype == DT_F32) rc = launch_rowdist<float>(X, batch, n, d, k, mean, labels, centres_old, counts, scratch, 0, active, stream);
-        else rc = launch_rowdist<double>(X, batch, n, d, k, mean, labels, centres_old, counts, scratch, 0, active, stream);
+        if (dtype == DT_U8) rc = launch_rowdist<unsigned char>(X, (int64_t)n * d, batch, n, d, k, mean, labels, centres_old, counts, scratch, 0, active, stream);
+        else if (dtype == DT_F32) rc = launch_rowdist<float>(X, (int64_t)n * d, batch, n, d, k, mean, labels, centres_old, counts, scratch, 0, active, stream);
+        else rc = launch_rowdist<double>(X, (int64_t)n * d, batch, n, d, k, mean, labels, centres_old, counts, scratch, 0, active, stream);
         if (rc != OFC_OK) return rc;
     }
     if (dtype == DT_U8)
@@ -1735,9 +1735,9 @@ int launch_kmeans_far_points(const void* X, int dtype, int batch, int64_t n, int
     ProfScope prof(PK_KMEANS, stream);
     if (scratch) {
         int rc;
-        if (dtype == DT_U8) rc = launch_rowdist<unsigned char>(X, batch, n, d, k, mean, labels, centres_old, nullptr, scratch, 1, nullptr, stream);
-        else if (dtype == DT_F32) rc = launch_rowdist<float>(X, batch, n, d, k, mean, labels, centres_old, nullptr, scratch, 1, nullptr, stream);
-        else rc = launch_rowdist<double>(X, batch, n, d, k, mean, labels, centres_old, nullptr, scratch, 1, nullptr, stream);
+        if (dtype == DT_U8) rc = launch_rowdist<unsigned char>(X, (int64_t)n * d, batch, n, d, k, mean, labels, centres_old, nullptr, scratch, 1, nullptr, stream);
+        else if (dtype == DT_F32) rc = launch_rowdist<float>(X, (int64_t)n * d, batch, n, d, k, mean, labels, centres_old, nullptr, scratch, 1, nullptr, stream);
+        else rc = launch_rowdist<double>(X, (int64_t)n * d, batch, n, d, k, mean, labels, centres_old, nullptr, scratch, 1, nullptr, stream);
         if (rc != OFC_OK) return rc;
         OFC_LAUNCH(kmeans_far_list_kernel, dim3(batch), dim3(1024), 0, stream, n, scratch, n_far, out_val, out_idx);
         OFC_CHECK_LAUNCH("kmeans_far_list");

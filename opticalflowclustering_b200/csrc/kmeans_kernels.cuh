@@ -9,7 +9,8 @@ enum { DT_U8 = 0, DT_F32 = 1, DT_F64 = 2 };
 static inline size_t dtype_size(int dtype) { return dtype == DT_U8 ? 1 : (dtype == DT_F32 ? 4 : 8); }
 
 struct KmAssignParams {
-    const void* X;               // [batch][n][d]
+    const void* X;               // [batch][n][d], or one [n][d] for every problem (x_stride = 0)
+    int64_t x_stride;            // elements between two problems' rows: n * d, or 0 (OFC_KMEANS_SHARED_ROWS)
     int dtype;
     int64_t n;
     int d, k;
@@ -26,6 +27,7 @@ struct KmAssignParams {
 
 struct KmSumsParams {
     const void* X;
+    int64_t x_stride;            // as in KmAssignParams
     int dtype;
     int64_t n;
     int d, k;
@@ -57,7 +59,7 @@ int launch_kmeans_update(int batch, int d, int k, const double* sums, const long
                          int32_t* labels_other, int* it_counter, void* stream);
 int launch_minibatch_update(const void* Xb, int dtype, int bs, int d, int k, const int32_t* labels, const double* centres_old,
                             double* centres_new, double* weight_sums, void* stream);
-int launch_kmeans_relocate(const void* X, int dtype, int batch, int64_t n, int d, int k, const double* mean,
+int launch_kmeans_relocate(const void* X, int64_t x_stride, int dtype, int batch, int64_t n, int d, int k, const double* mean,
                            const int32_t* labels, const double* centres_old, double* sums, long long* counts,
                            int raw_sums, const unsigned char* active, double* scratch, void* stream);
 int launch_kmeans_far_payload(const void* X, int dtype, int batch, int64_t n, int d, int k, const double* mean, const int32_t* labels,

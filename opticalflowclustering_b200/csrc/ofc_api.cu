@@ -685,10 +685,13 @@ struct KmWorkspace {
     size_t assign_total;         // the prefix ofc_kmeans_assign / ofc_kmeans_centres need (no M-step partials)
     int parts, splits, dt, kt;
 };
-KmWorkspace km_layout(int batch, int64_t n, int d, int k) {
+// shared: the problems read one X (OFC_KMEANS_SHARED_ROWS).  Their M-step then uses the split count of ONE problem, so
+// the float sums of a problem are folded in the same order whatever the batch (uint8 sums are exact in any order);
+// the layout stays within batch * km_layout(1, n, d, k).total, which is what the header promises the caller.
+KmWorkspace km_layout(int batch, int64_t n, int d, int k, bool shared = false) {
     KmWorkspace w;
     w.parts = kmeans_assign_grid(n);
-    w.splits = kmeans_sums_splits(n, batch);
+    w.splits = kmeans_sums_splits(n, shared ? 1 : batch);
     w.dt = 1;
     while (w.dt < 32 && w.dt < d) w.dt <<= 1;
     w.kt = k < 32 ? k : 32;
@@ -718,7 +721,10 @@ size_t ofc_kmeans_assign_workspace_bytes(int batch, int64_t n, int d, int k) {
     return km_layout(batch, n, d, k).assign_total;
 }
 
-static int km_check(const void* X, int dtype, int batch, int64_t n, int d, int k) {
+// splits the dtype argument of the stepwise calls into the element type and the OFC_KMEANS_SHARED_ROWS flag
+static int km_check(const void* X, int& dtype, bool& shared, int batch, int64_t n, int d, int k) {
+    shared = (dtype & OFC_KMEANS_SHARED_ROWS) != 0;
+    dtype &= ~OFC_KMEANS_SHARED_ROWS;
     OFC_REQUIRE(dtype == OFC_U8 || dtype == OFC_F32 || dtype == OFC_F64, "bad dtype %d", dtype);
     OFC_REQUIRE(batch >= 0 && n >= 0 && d >= 1 && k >= 1, "bad k-means shape batch=%d n=%lld d=%d k=%d", batch, (long long)n, d, k);
     OFC_REQUIRE(batch == 0 || n == 0 || X != nullptr, "null data");
@@ -729,15 +735,16 @@ int ofc_kmeans_assign(const void* X, int dtype, int batch, int64_t n, int d, int
                       const double* centres, int32_t* labels, const int32_t* prev_labels, uint64_t* n_changed,
                       double* inertia, double* min_dist, const uint8_t* active, void* workspace, size_t workspace_bytes,
                       void* stream) {
-    int rc = km_check(X, dtype, batch, n, d, k);
+    bool shared;
+    int rc = km_check(X, dtype, shared, batch, n, d, k);
     if (rc != OFC_OK) return rc;
     if (batch == 0 || n == 0) return OFC_OK;
     OFC_REQUIRE(centres && labels, "null centres / labels");
-    KmWorkspace w = km_layout(batch, n, d, k);
+    KmWorkspace w = km_layout(batch, n, d, k, shared);
     if (!workspace || workspace_bytes < w.assign_total) { set_error("k-means workspace too small: %zu < %zu", workspace_bytes, w.assign_total); return OFC_ERR_WORKSPACE; }
     char* ws = (char*)workspace;
     KmAssignParams p;
-    p.X = X; p.dtype = dtype; p.n = n; p.d = d; p.k = k; p.mean = mean; p.centres = centres; p.c2 = nullptr;
+    p.X = X; p.x_stride = shared ? 0 : n * d; p.dtype = dtype; p.n = n; p.d = d; p.k = k; p.mean = mean; p.centres = centres; p.c2 = nullptr;
     p.labels = labels; p.prev_labels = prev_labels; p.n_changed = (unsigned long long*)n_changed;
     p.inertia_partial = inertia ? (double*)(ws + w.off_inertia) : nullptr;
     p.min_dist = min_dist; p.active = active;
@@ -751,29 +758,31 @@ int ofc_kmeans_assign(const void* X, int dtype, int batch, int64_t n, int d, int
 int ofc_kmeans_sums(const void* X, int dtype, int batch, int64_t n, int d, int k, const double* mean,
                     const int32_t* labels, int square, double* sums, int64_t* counts, const uint8_t* active,
                     void* workspace, size_t workspace_bytes, void* stream) {
-    int rc = km_check(X, dtype, batch, n, d, k);
+    bool shared;
+    int rc = km_check(X, dtype, shared, batch, n, d, k);
     if (rc != OFC_OK) return rc;
     if (batch == 0) return OFC_OK;
     OFC_REQUIRE(sums != nullptr, "null sums");
     OFC_REQUIRE(n > 0, "empty data");
-    KmWorkspace w = km_layout(batch, n, d, k);
+    KmWorkspace w = km_layout(batch, n, d, k, shared);
     if (!workspace || workspace_bytes < w.total) { set_error("k-means workspace too small: %zu < %zu", workspace_bytes, w.total); return OFC_ERR_WORKSPACE; }
     char* ws = (char*)workspace;
     KmSumsParams p;
-    p.X = X; p.dtype = dtype; p.n = n; p.d = d; p.k = k; p.mean = mean; p.labels = labels; p.square = square;
+    p.X = X; p.x_stride = shared ? 0 : n * d; p.dtype = dtype; p.n = n; p.d = d; p.k = k; p.mean = mean; p.labels = labels; p.square = square;
     p.partial = (double*)(ws + w.off_partial); p.cnt_partial = (long long*)(ws + w.off_cnt);
     p.splits = w.splits; p.dt = w.dt; p.kt = w.kt; p.active = active;
     return launch_kmeans_sums(p, batch, sums, (long long*)counts, stream);
 }
 
 int ofc_kmeans_step_supported(int dtype, int d, int k) {
-    return dtype == OFC_U8 && d >= 1 && d <= 32 && k >= 1 && kmeans_step_smem(d, k) <= 200 * 1024;
+    return (dtype & ~OFC_KMEANS_SHARED_ROWS) == OFC_U8 && d >= 1 && d <= 32 && k >= 1 && kmeans_step_smem(d, k) <= 200 * 1024;
 }
 
 int ofc_kmeans_step(const void* X, int dtype, int batch, int64_t n, int d, int k, const double* mean, const double* centres,
                     int32_t* labels, const int32_t* prev_labels, uint64_t* n_changed, double* sums, int64_t* counts,
                     const uint8_t* active, void* workspace, size_t workspace_bytes, void* stream) {
-    int rc = km_check(X, dtype, batch, n, d, k);
+    bool shared;
+    int rc = km_check(X, dtype, shared, batch, n, d, k);
     if (rc != OFC_OK) return rc;
     if (!ofc_kmeans_step_supported(dtype, d, k)) {
         set_error("fused k-means step needs uint8 rows, d <= 32 and [k][d] accumulators that fit shared memory (dtype=%d d=%d k=%d)", dtype, d, k);
@@ -781,11 +790,11 @@ int ofc_kmeans_step(const void* X, int dtype, int batch, int64_t n, int d, int k
     }
     if (batch == 0 || n == 0) return OFC_OK;
     OFC_REQUIRE(centres && labels && sums && counts, "null buffer");
-    KmWorkspace w = km_layout(batch, n, d, k);
+    KmWorkspace w = km_layout(batch, n, d, k, shared);
     if (!workspace || workspace_bytes < w.total) { set_error("k-means workspace too small: %zu < %zu", workspace_bytes, w.total); return OFC_ERR_WORKSPACE; }
     char* ws = (char*)workspace;
     KmAssignParams p;
-    p.X = X; p.dtype = dtype; p.n = n; p.d = d; p.k = k; p.mean = mean; p.centres = centres; p.c2 = nullptr;
+    p.X = X; p.x_stride = shared ? 0 : n * d; p.dtype = dtype; p.n = n; p.d = d; p.k = k; p.mean = mean; p.centres = centres; p.c2 = nullptr;
     p.labels = labels; p.prev_labels = prev_labels; p.n_changed = (unsigned long long*)n_changed;
     p.inertia_partial = nullptr; p.min_dist = nullptr; p.active = active;
     if (n_changed) OFC_CUDA(cudaMemsetAsync(n_changed, 0, sizeof(uint64_t) * batch, (cudaStream_t)stream));
@@ -829,18 +838,21 @@ int ofc_minibatch_update(const void* Xb, int dtype, int batch_rows, int d, int k
 int ofc_kmeans_relocate(const void* X, int dtype, int batch, int64_t n, int d, int k, const double* mean,
                         const int32_t* labels, const double* centres_old, double* sums, int64_t* counts,
                         int raw_sums, const uint8_t* active, double* scratch, void* stream) {
-    int rc = km_check(X, dtype, batch, n, d, k);
+    bool shared;
+    int rc = km_check(X, dtype, shared, batch, n, d, k);
     if (rc != OFC_OK) return rc;
     if (batch == 0 || n == 0) return OFC_OK;
     OFC_REQUIRE(labels && centres_old && sums && counts, "null buffer");
-    return launch_kmeans_relocate(X, dtype, batch, n, d, k, mean, labels, centres_old, sums, (long long*)counts, raw_sums, active, scratch,
+    return launch_kmeans_relocate(X, shared ? 0 : n * d, dtype, batch, n, d, k, mean, labels, centres_old, sums, (long long*)counts, raw_sums, active, scratch,
                                   stream);
 }
 
 int ofc_kmeans_far_points(const void* X, int dtype, int batch, int64_t n, int d, int k, const double* mean, const int32_t* labels,
                           const double* centres_old, int n_far, double* out_val, int64_t* out_idx, double* scratch, void* stream) {
-    int rc = km_check(X, dtype, batch, n, d, k);
+    bool shared;
+    int rc = km_check(X, dtype, shared, batch, n, d, k);
     if (rc != OFC_OK) return rc;
+    if (shared) { set_error("ofc_kmeans_far_points: row-sharded fits take one X per problem (no OFC_KMEANS_SHARED_ROWS)"); return OFC_ERR_UNSUPPORTED; }
     OFC_REQUIRE(n_far >= 1 && n_far <= k, "n_far=%d outside [1, k]", n_far);
     if (batch == 0) return OFC_OK;
     OFC_REQUIRE(n > 0 && labels && centres_old && out_val && out_idx, "null buffer / empty shard");
@@ -851,6 +863,10 @@ int ofc_kmeans_far_points(const void* X, int dtype, int batch, int64_t n, int d,
 int ofc_kmeans_far_payload(const void* X, int dtype, int batch, int64_t n, int d, int k, const double* mean, const int32_t* labels,
                            const double* centres_old, const int64_t* counts, int raw_sums, int n_far, int64_t row_offset,
                            double* payload, double* scratch, const uint8_t* active, void* stream) {
+    if (dtype & OFC_KMEANS_SHARED_ROWS) {
+        set_error("ofc_kmeans_far_payload: row-sharded fits take one X per problem (no OFC_KMEANS_SHARED_ROWS)");
+        return OFC_ERR_UNSUPPORTED;
+    }
     OFC_REQUIRE(dtype == OFC_U8 || dtype == OFC_F32 || dtype == OFC_F64, "bad dtype %d", dtype);
     OFC_REQUIRE(batch >= 0 && n >= 0 && d >= 1 && k >= 1, "bad shape");
     OFC_REQUIRE(n_far >= 1 && n_far <= k, "n_far=%d outside [1, k]", n_far);

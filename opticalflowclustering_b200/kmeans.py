@@ -12,7 +12,9 @@ E-step when the stop was not strict.  uint8 rows are worked in float64 like skle
 
 Everything is batched: ``X`` may be ``[n, d]`` (one problem) or ``[B, n, d]`` (B independent
 problems of equal shape -- the reference runs one fit per grid cell).  Problems that have
-converged are frozen by an ``active`` mask while the others keep iterating.
+converged are frozen by an ``active`` mask while the others keep iterating.  ``X [n, d]`` with
+``init [R, k, d]`` runs R starts of one fit (``KMeans(n_init=R)``) as R problems that read the
+same rows (``OFC_KMEANS_SHARED_ROWS``: no copy of X per start).
 
 Multi-GPU: rows sharded over the ranks of ``group``; the only exchange is an all-reduce
 of ``[k*d sums | k counts | n_changed]`` per iteration (NCCL over NVLink on GPUs).  For
@@ -111,22 +113,28 @@ def _as_batch(X, device=None):
 class LloydState:
     """Buffers of one batched Lloyd run (all on the data's device)."""
 
-    def __init__(self, ctx: _Ctx, X: torch.Tensor, k: int, ws_k: int | None = None):
+    def __init__(self, ctx: _Ctx, X: torch.Tensor, k: int, ws_k: int | None = None, shared_batch: int | None = None):
         """``ws_k``: cluster count the stepwise workspace is sized for (1 when the tensor-core path does
-        the E/M steps and only the column statistics run through the stepwise kernels)."""
+        the E/M steps and only the column statistics run through the stepwise kernels).  ``shared_batch``: run that
+        many problems over the one problem of ``X`` ([1, n, d]) without copying it (OFC_KMEANS_SHARED_ROWS)."""
         self.ctx, self.X, self.k = ctx, X, int(k)
         self.B, self.n, self.d = (int(s) for s in X.shape)
         self.dtype = _DT[X.dtype]
+        self.flags = 0                  # OR-ed into the dtype of the calls that read X
+        per = self.B                    # problems the workspace queries are asked for; a shared batch needs B times one
+        if shared_batch is not None:
+            self.B, self.flags, per = int(shared_batch), _lib.OFC_KMEANS_SHARED_ROWS, 1
         dev = X.device
         lib = ctx.lib
         lib.ofc_kmeans_workspace_bytes.restype = C.c_size_t
         lib.ofc_kmeans_workspace_bytes.argtypes = [C.c_int, C.c_int64, C.c_int, C.c_int]
-        self.ws_bytes = int(lib.ofc_kmeans_workspace_bytes(self.B, self.n, self.d, max(self.k if ws_k is None else int(ws_k), 1)))
+        mul = self.B // per
+        self.ws_bytes = mul * int(lib.ofc_kmeans_workspace_bytes(per, self.n, self.d, max(self.k if ws_k is None else int(ws_k), 1)))
         if ws_k is not None and hasattr(lib, "ofc_kmeans_assign_workspace_bytes"):
             # the E-step / centre kernels still run for all k clusters (final inertia, relocation, new centres)
             lib.ofc_kmeans_assign_workspace_bytes.restype = C.c_size_t
             lib.ofc_kmeans_assign_workspace_bytes.argtypes = [C.c_int, C.c_int64, C.c_int, C.c_int]
-            self.ws_bytes = max(self.ws_bytes, int(lib.ofc_kmeans_assign_workspace_bytes(self.B, self.n, self.d, max(self.k, 1))))
+            self.ws_bytes = max(self.ws_bytes, mul * int(lib.ofc_kmeans_assign_workspace_bytes(per, self.n, self.d, max(self.k, 1))))
         self.ws = torch.empty(max(self.ws_bytes, 256), dtype=torch.uint8, device=dev)
         self.labels = [torch.full((self.B, self.n), -1, dtype=torch.int32, device=dev) for _ in range(2)]
         # the kernels write straight into the buffers the all-reduces move: float64 sums, and ONE int64 buffer holding
@@ -145,7 +153,7 @@ class LloydState:
     # -- thin wrappers over the C-ABI -----------------------------------------------------
     def assign(self, mean, centres, labels, prev=None, n_changed=None, inertia=None, min_dist=None, active=None):
         c = self.ctx
-        c.check(c.lib.ofc_kmeans_assign(_ptr(self.X), self.dtype, self.B, C.c_int64(self.n), self.d, int(centres.shape[1]),
+        c.check(c.lib.ofc_kmeans_assign(_ptr(self.X), self.dtype | self.flags, self.B, C.c_int64(self.n), self.d, int(centres.shape[1]),
                                         _ptr(mean), _ptr(centres), _ptr(labels), _ptr(prev), _ptr(n_changed),
                                         _ptr(inertia), _ptr(min_dist), _ptr(active), _ptr(self.ws),
                                         C.c_size_t(self.ws.numel()), c.stream()))
@@ -158,13 +166,13 @@ class LloydState:
 
     def step(self, mean, centres, labels, prev, n_changed, sums, counts, active=None):
         c = self.ctx
-        c.check(c.lib.ofc_kmeans_step(_ptr(self.X), self.dtype, self.B, C.c_int64(self.n), self.d, self.k, _ptr(mean),
+        c.check(c.lib.ofc_kmeans_step(_ptr(self.X), self.dtype | self.flags, self.B, C.c_int64(self.n), self.d, self.k, _ptr(mean),
                                       _ptr(centres), _ptr(labels), _ptr(prev), _ptr(n_changed), _ptr(sums), _ptr(counts),
                                       _ptr(active), _ptr(self.ws), C.c_size_t(self.ws.numel()), c.stream()))
 
     def sums_(self, mean, labels, sums, counts, k, square=0, active=None):
         c = self.ctx
-        c.check(c.lib.ofc_kmeans_sums(_ptr(self.X), self.dtype, self.B, C.c_int64(self.n), self.d, int(k), _ptr(mean),
+        c.check(c.lib.ofc_kmeans_sums(_ptr(self.X), self.dtype | self.flags, self.B, C.c_int64(self.n), self.d, int(k), _ptr(mean),
                                       _ptr(labels), int(square), _ptr(sums), _ptr(counts), _ptr(active), _ptr(self.ws),
                                       C.c_size_t(self.ws.numel()), c.stream()))
 
@@ -186,7 +194,7 @@ class LloydState:
 
     def relocate(self, mean, labels, centres_old, sums, counts, raw_sums, active=None):
         c = self.ctx
-        c.check(c.lib.ofc_kmeans_relocate(_ptr(self.X), self.dtype, self.B, C.c_int64(self.n), self.d, self.k, _ptr(mean),
+        c.check(c.lib.ofc_kmeans_relocate(_ptr(self.X), self.dtype | self.flags, self.B, C.c_int64(self.n), self.d, self.k, _ptr(mean),
                                           _ptr(labels), _ptr(centres_old), _ptr(sums), _ptr(counts), int(raw_sums),
                                           _ptr(active), _ptr(self.row_scratch()), c.stream()))
 
@@ -363,6 +371,12 @@ def lloyd(X, init, max_iter: int = 300, tol: float = 1e-4, group=None, _host_rel
     init ``[k,d]`` or ``[B,k,d]``.  With ``group`` every rank passes its own rows (same B, d, k)
     and receives the global centres / inertia and the labels of its rows.
 
+    ``X [n,d]`` with ``init [R,k,d]``: R starts over the same rows, returned as ``[R, ...]``.  Every start gives the
+    bits it gives alone (``lloyd(X, init[r])``): the batch reads X with a batch stride of 0 and the M-step sums
+    of a start are folded in the order of a single problem.  The column statistics are computed once.  Where a
+    single start runs on the tensor cores, the starts run one after another (a batch would take the CUDA-core
+    M-step, whose float32 sums are ordered differently).  Not with ``group``.
+
     The loop keeps the host out of the data path: every iteration is a handful of kernel launches (E-step +
     M-step sums, empty-cluster relocation, ``ofc_kmeans_update`` = new centres + stopping rule on the device);
     the only thing the host reads is the "problems still running" counter, asynchronously and ``_POLL_LAG``
@@ -378,17 +392,27 @@ def lloyd(X, init, max_iter: int = 300, tol: float = 1e-4, group=None, _host_rel
     """
     Xb, single = _as_batch(X, _target_device(X))
     ctx = _Ctx(Xb.device)
+    init_arg = init
     init = torch.as_tensor(np.asarray(init) if not isinstance(init, torch.Tensor) else init)
     init = init.to(device=Xb.device, dtype=torch.float64)
-    if init.dim() == 2:
+    shared = single and init.dim() == 3                           # several starts over one X
+    if shared:
+        if group is not None:
+            raise NotImplementedError("several starts (init [R, k, d]) of a row-sharded fit")
+        if _tc_wanted(Xb, int(init.shape[1])):
+            runs = [lloyd(Xb[0], init[r], max_iter, tol) for r in range(int(init.shape[0]))]
+            return tuple(torch.stack(t) for t in zip(*runs))
+    elif init.dim() == 2:
         init = init.unsqueeze(0).expand(Xb.shape[0], -1, -1)
     init = init.contiguous()
     B, n, d = (int(s) for s in Xb.shape)
+    if shared:
+        B = int(init.shape[0])
     k = int(init.shape[1])
-    if init.shape[0] != B or init.shape[2] != d:
+    if init.dim() != 3 or init.shape[0] != B or init.shape[2] != d:
         raise ValueError(f"init shape {tuple(init.shape)} does not match X {tuple(Xb.shape)}")
-    use_tc = _tc_wanted(Xb, k)
-    st = LloydState(ctx, Xb, k, ws_k=1 if use_tc else None)
+    use_tc = not shared and _tc_wanted(Xb, k)
+    st = LloydState(ctx, Xb, k, ws_k=1 if use_tc else None, shared_batch=B if shared else None)
     dev = Xb.device
     row_offset, n_total = 0, n
     if group is not None:
@@ -400,8 +424,10 @@ def lloyd(X, init, max_iter: int = 300, tol: float = 1e-4, group=None, _host_rel
         row_offset, n_total = sum(ns[:dist.get_rank(group)]), sum(ns)
     if n_total < k:
         raise ValueError(f"n_samples={n_total} should be >= n_clusters={k}.")   # _kmeans.py:876-879
-    mean, var, _ = column_mean_var(st, group)
-    tol_ = (var.mean(dim=1) * tol).contiguous()                  # stays on the device
+    # a shared batch: the statistics once, as a single fit computes them, then the same values for every start
+    mean, var, _ = column_mean_var(LloydState(ctx, Xb, 1) if shared else st, group)
+    tol_ = (var.mean(dim=1) * tol).expand(B).contiguous()        # stays on the device
+    mean = mean.expand(B, d).contiguous()
     is_u8 = st.dtype == 0
     is_f32 = st.dtype == 1
     if is_f32:
@@ -578,7 +604,7 @@ def lloyd(X, init, max_iter: int = 300, tol: float = 1e-4, group=None, _host_rel
         if int(overflow.item()):
             # more clusters empty at once than the device-side candidate list holds: redo the fit with the host-merged
             # relocation (every rank takes this branch: the all-reduced counts are the same everywhere)
-            return lloyd(X, init, max_iter, tol, group, _host_relocation=True)
+            return lloyd(X, init_arg, max_iter, tol, group, _host_relocation=True)
     final = st.labels[0]
     # strict stops already hold the labels of the final centres; the rest get one more E-step
     # (_kmeans.py:745-755).  Re-running it for everyone is idempotent for the strict ones and
@@ -592,7 +618,7 @@ def lloyd(X, init, max_iter: int = 300, tol: float = 1e-4, group=None, _host_rel
         _all_reduce(inertia, group)
     out_centres = centres + mean.unsqueeze(1)
     n_iter_t = st.n_iter.to(torch.int64)
-    if single:
+    if single and not shared:
         return final[0], out_centres[0], inertia[0], n_iter_t[0]
     return final, out_centres, inertia, n_iter_t
 
@@ -695,11 +721,125 @@ def kmeans_plusplus(X, n_clusters: int, random_state=None):
     return centres, indices
 
 
+def kmeans_plusplus_starts(X, n_clusters: int, n_starts: int, random_state):
+    """The k-means++ seeds of ``n_starts`` starts of one fit, the same as ``n_starts`` calls of
+    :func:`kmeans_plusplus` one after another on one ``RandomState`` -- computed in lockstep on the device, without
+    a host round trip until the seeds are done.  X ``[n, d]`` on the compute device; returns ``(centres float64
+    [R, k, d] tensor, indices int64 [R, k])``.
+
+    The host first makes every start's RNG calls in sklearn's order (one ``choice`` and k - 1 ``uniform(size=T)``
+    per start: how many numbers they draw does not depend on the data).  Each of the k - 1 steps then computes the
+    distances of all R*T candidates in ONE E-step call (a shared-row batch of one-centre problems), and every start
+    runs the torch operations of :func:`kmeans_plusplus` on tensors of the same shapes, each in an allocation of its
+    own (a reduction may order its sum by the data's alignment), so a start's seeds do not depend on R."""
+    Xb, single = _as_batch(X, _target_device(X))
+    if not single:
+        raise ValueError("kmeans_plusplus_starts takes one problem [n, d]")
+    ctx = _Ctx(Xb.device)
+    rs = random_state if isinstance(random_state, np.random.RandomState) else np.random.RandomState(random_state)
+    n, d = int(Xb.shape[1]), int(Xb.shape[2])
+    k, R = int(n_clusters), int(n_starts)
+    trials = 2 + int(math.log(k))
+    dev = Xb.device
+    first = np.empty(R, np.int64)
+    uni = np.empty((R, max(k - 1, 1), trials))
+    for r in range(R):
+        first[r] = rs.choice(n, p=np.full(n, 1.0 / n))
+        for c in range(1, k):
+            uni[r, c - 1] = rs.uniform(size=trials)
+    uni = torch.from_numpy(uni).to(dev)
+    Xf = Xb[0]
+    idx = torch.empty((R, k), dtype=torch.int64, device=dev)
+    idx[:, 0] = torch.from_numpy(first).to(dev)
+    st = LloydState(ctx, Xb, 1, shared_batch=R)
+    dist0 = torch.empty((R, n), dtype=torch.float64, device=dev)
+    st.assign(None, Xf[idx[:, 0]].to(torch.float64).view(R, 1, d).contiguous(), st.labels[0], min_dist=dist0)
+    closest = [dist0[r:r + 1].clone() for r in range(R)]
+    pot = [cl.sum() for cl in closest]
+    if k > 1:
+        cst = LloydState(ctx, Xb, 1, shared_batch=R * trials)
+        cand = torch.empty((R * trials, n), dtype=torch.float64, device=dev)
+    for c in range(1, k):
+        ids = []
+        for r in range(R):
+            rand_vals = uni[r, c - 1] * pot[r]
+            cum = torch.cumsum(closest[r][0], dim=0)
+            ids.append(torch.searchsorted(cum, rand_vals).clamp_(max=n - 1))
+        ids = torch.cat(ids)
+        cst.assign(None, Xf[ids].to(torch.float64).view(R * trials, 1, d).contiguous(), cst.labels[0], min_dist=cand)
+        for r in range(R):
+            dmin = [torch.minimum(closest[r], cand[r * trials + t:r * trials + t + 1]) for t in range(trials)]
+            p = torch.stack([dm.sum() for dm in dmin])
+            best = torch.argmin(p).view(1)                     # the first of the smallest, as the strict `<` of the loop
+            pot[r] = p[best][0]
+            closest[r] = torch.stack(dmin).index_select(0, best)[0]
+            idx[r, c] = ids[r * trials:(r + 1) * trials][best][0]
+    return Xf[idx].to(torch.float64), idx.cpu().numpy()
+
+
+def _is_same_clustering(labels1, labels2, k: int) -> bool:
+    """sklearn's ``_is_same_clustering`` (_k_means_common.pyx:314-328): the map from ``labels1`` to ``labels2``, taken
+    at the first row of every cluster of ``labels1``, is a function on all rows (not necessarily a bijection)."""
+    n = int(labels1.shape[0])
+    a = labels1.long()
+    first = torch.full((k,), n, dtype=torch.int64, device=a.device)
+    first.scatter_reduce_(0, a, torch.arange(n, device=a.device), reduce="amin")
+    return bool(torch.equal(labels2[first[a]], labels2))
+
+
+def best_start(labels, inertia, k: int) -> int:
+    """sklearn's choice among the starts of one fit (_kmeans.py:1534-1543): start i replaces the best so far only if its
+    inertia is strictly lower and its clustering is not the same (:func:`_is_same_clustering`)."""
+    inert = inertia.cpu().numpy()
+    best = 0
+    for i in range(1, len(inert)):
+        if inert[i] < inert[best] and not _is_same_clustering(labels[i], labels[best], k):
+            best = i
+    return best
+
+
+def _resolve_n_init(n_init, init) -> int:
+    """sklearn's ``_check_params_vs_input`` (_kmeans.py:884-907): "auto" is 1 for k-means++ and an array, 10 for
+    "random"; an array with n_init != 1 warns and runs one start."""
+    if isinstance(n_init, str):
+        if n_init != "auto":
+            raise ValueError(f"n_init must be 'auto' or an int >= 1, got {n_init!r}")
+        r = 10 if isinstance(init, str) and init == "random" else 1
+    else:
+        if isinstance(n_init, bool) or not isinstance(n_init, (int, np.integer)) or n_init < 1:
+            raise ValueError(f"n_init must be 'auto' or an int >= 1, got {n_init!r}")
+        r = int(n_init)
+    if not isinstance(init, str) and r != 1:
+        import warnings
+        warnings.warn("Explicit initial center position passed: performing only one init in KMeans instead of "
+                      f"n_init={r}.", RuntimeWarning, stacklevel=3)
+        r = 1
+    return r
+
+
+def random_starts(X, n_clusters: int, n_starts: int, random_state):
+    """``init="random"`` (_kmeans.py:1030-1036): per start, ``choice(n, size=k, replace=False, p=w / w.sum())`` with
+    ``w`` = ones in the data's working dtype (float32 for float32 rows, else float64).  Returns (centres float64
+    [R, k, d] tensor on X's device, indices int64 [R, k])."""
+    Xb, _ = _as_batch(X, _target_device(X))
+    rs = random_state if isinstance(random_state, np.random.RandomState) else np.random.RandomState(random_state)
+    n = int(Xb.shape[1])
+    w = np.ones(n, dtype=np.float32 if Xb.dtype == torch.float32 else np.float64)
+    idx = np.stack([rs.choice(n, size=int(n_clusters), replace=False, p=w / w.sum()) for _ in range(int(n_starts))])
+    return Xb[0][torch.from_numpy(idx).to(Xb.device)].to(torch.float64), idx.astype(np.int64)
+
+
 class KMeans:
     """The subset of ``sklearn.cluster.KMeans`` the reference uses (KmeanGrids.py:299-304,
     color_kmeans.py:65-78): ``KMeans(n_clusters=k).fit(X)``, ``.predict(X)``,
     ``.cluster_centers_``, ``.labels_``, ``.inertia_``, ``.n_iter_``.  ``init`` may be
-    ``'k-means++'`` (default, see :func:`kmeans_plusplus`) or an array ``[k, d]``."""
+    ``'k-means++'`` (default, see :func:`kmeans_plusplus`), ``'random'`` or an array ``[k, d]``.
+
+    ``n_init`` as scikit-learn 1.9: ``"auto"`` is one start for k-means++ and an array, 10 for ``"random"``.
+    The starts draw their seeds one after another from one ``RandomState`` (so ``random_state=int`` reproduces
+    sklearn), run as one batched Lloyd fit over a single copy of the rows, and the result is the start sklearn
+    keeps: the first one, replaced by a later one only if that has a strictly lower inertia and a different
+    clustering."""
 
     def __init__(self, n_clusters=8, *, init="k-means++", n_init="auto", max_iter=300, tol=1e-4, random_state=None):
         self.n_clusters, self.init, self.n_init = int(n_clusters), init, n_init
@@ -711,16 +851,30 @@ class KMeans:
             raise ValueError("Expected 2D array")
         if Xa.shape[0] < self.n_clusters:
             raise ValueError(f"n_samples={Xa.shape[0]} should be >= n_clusters={self.n_clusters}.")
-        if isinstance(self.init, str):
-            if self.init != "k-means++":
-                raise NotImplementedError(f"init={self.init!r}")
-            if self.n_clusters == 1:
-                init = (Xa[:1].to(torch.float64) if isinstance(Xa, torch.Tensor) else Xa[:1].astype(np.float64))
+        if isinstance(self.init, str) and self.init not in ("k-means++", "random"):
+            raise ValueError(f"init={self.init!r}: 'k-means++', 'random' or an array")
+        n_init = _resolve_n_init(self.n_init, self.init)
+        if isinstance(self.init, str) and self.n_clusters > 1 and (n_init > 1 or self.init == "random"):
+            rs = (self.random_state if isinstance(self.random_state, np.random.RandomState)
+                  else np.random.RandomState(self.random_state))
+            Xd, _ = _as_batch(Xa, _target_device(Xa))
+            Xd = Xd[0]
+            if self.init == "random":
+                init, _ = random_starts(Xd, self.n_clusters, n_init, rs)
             else:
-                init, _ = kmeans_plusplus(Xa, self.n_clusters, self.random_state)
+                init, _ = kmeans_plusplus_starts(Xd, self.n_clusters, n_init, rs)
+            labels, centres, inertia, n_iter = lloyd(Xd, init, self.max_iter, self.tol)
+            b = best_start(labels, inertia, self.n_clusters)
+            labels, centres, inertia, n_iter = labels[b], centres[b], inertia[b], n_iter[b]
         else:
-            init = self.init
-        labels, centres, inertia, n_iter = lloyd(Xa, init, self.max_iter, self.tol)
+            if isinstance(self.init, str):
+                if self.n_clusters == 1:
+                    init = (Xa[:1].to(torch.float64) if isinstance(Xa, torch.Tensor) else Xa[:1].astype(np.float64))
+                else:
+                    init, _ = kmeans_plusplus(Xa, self.n_clusters, self.random_state)
+            else:
+                init = self.init
+            labels, centres, inertia, n_iter = lloyd(Xa, init, self.max_iter, self.tol)
         self._centres_t = centres
         self.cluster_centers_ = centres.cpu().numpy()
         if not isinstance(X, torch.Tensor) and np.asarray(X).dtype == np.float32:
