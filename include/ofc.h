@@ -253,6 +253,39 @@ int ofc_kmeans_relocate(const void* X, int dtype, int batch, int64_t n, int d, i
                         const int32_t* labels, const double* centres_old, double* sums, int64_t* counts,
                         int raw_sums, const uint8_t* active, double* scratch, void* stream);
 
+/* ---- weighted fits: KMeans.fit(X, sample_weight=w) ----
+ * The weighted twins of ofc_kmeans_assign / _sums / _update / _relocate.  weights f64 [batch][n] (>= 0, not all 0;
+ * the caller validates them), or ONE [n] vector for every problem under OFC_KMEANS_SHARED_ROWS, like X.  Where the
+ * unweighted calls have int64 member counts these take float64 weight sums `weight_sums [batch][k]`.  Labels do not
+ * depend on the weights.  Every weighted form folds in the unweighted order, so weights of all ones give exactly the
+ * unweighted bits.  Real-valued weights are summed deterministically (fixed order, no floating-point atomics).  uint8
+ * rows with integer-valued weights keep exact sums: every x w and every partial sum stays below 2^53.
+ *
+ * ofc_kmeans_assign_weighted: ofc_kmeans_assign with inertia = sum_i w_i ||x_i - c_label||^2
+ *   (_inertia_dense, _k_means_common.pyx:94-124); min_dist stays unweighted. */
+int ofc_kmeans_assign_weighted(const void* X, int dtype, int batch, int64_t n, int d, int k, const double* mean,
+                               const double* centres, const double* weights, int32_t* labels, const int32_t* prev_labels,
+                               uint64_t* n_changed, double* inertia, double* min_dist, const uint8_t* active, void* workspace,
+                               size_t workspace_bytes, void* stream);
+/* M-step: sums[b][j][:] = sum over members of (x - mean) w, weight_sums[b][j] = sum of their weights
+ * (_k_means_lloyd.pyx:216-218).  Same workspace as ofc_kmeans_sums. */
+int ofc_kmeans_sums_weighted(const void* X, int dtype, int batch, int64_t n, int d, int k, const double* mean,
+                             const int32_t* labels, const double* weights, double* sums, double* weight_sums,
+                             const uint8_t* active, void* workspace, size_t workspace_bytes, void* stream);
+/* ofc_kmeans_update on weight sums (_average_centers, _k_means_common.pyx:264-286): centres = sums / weight where
+ * weight > 0, otherwise the centre of the heaviest cluster by weight (the first on ties).  Stopping rule unchanged. */
+int ofc_kmeans_update_weighted(int batch, int64_t n, int d, int k, const double* sums, const double* weight_sums,
+                               const double* mean_sub, int use_reciprocal, int round_f32, double* centres, double* shift_tot,
+                               const uint64_t* n_changed, const double* tol, int iteration, uint8_t* active, uint8_t* just_done,
+                               int32_t* n_iter, int32_t* n_active, const int32_t* labels_cur, int32_t* labels_other,
+                               int32_t* it_counter, void* workspace, size_t workspace_bytes, void* stream);
+/* ofc_kmeans_relocate on weight sums (_relocate_empty_clusters_dense, _k_means_common.pyx:167-211): a cluster is
+ * empty when its WEIGHT is 0 (members of weight 0 only count as empty); the farthest rows are chosen by unweighted
+ * distance; the moved row carries x w and w.  scratch (f64 [batch][n]) is required. */
+int ofc_kmeans_relocate_weighted(const void* X, int dtype, int batch, int64_t n, int d, int k, const double* mean,
+                                 const int32_t* labels, const double* centres_old, const double* weights, double* sums,
+                                 double* weight_sums, int raw_sums, const uint8_t* active, double* scratch, void* stream);
+
 /* Row-sharded data (one shard per GPU): the search half of that relocation.  out_val / out_idx [batch][n_far] =
  * this shard's n_far farthest rows (squared distance to the old centre of their label; largest first, lowest
  * index on ties; idx -1 past the shard's size).  The host merges the ranks' lists and applies the moves to the
@@ -362,6 +395,20 @@ int ofc_kmeans_tc_assign_u8(const uint8_t* X, const double* mean, const float* X
                             void* workspace, size_t workspace_bytes, void* stream);
 int ofc_kmeans_tc_sums_u8(const uint8_t* X, int64_t n, int d, int k, const int32_t* labels,
                           double* sums, int64_t* counts, void* workspace, size_t workspace_bytes, void* stream);
+/* Weighted fits on the tensor cores (weights f64 [n], as for ofc_kmeans_sums_weighted); the E-step's labels do not
+ * depend on the weights.  _assign_weighted: inertia = sum_i w_i ||x_i - c_label||^2 (_inertia_dense).  _sums_weighted /
+ * _sums_u8_weighted: sums of x w and weight_sums[j] = sum of the members' weights (_k_means_lloyd.pyx:216-218), in the
+ * member list's order; counts = members as before. */
+int ofc_kmeans_tc_assign_weighted(const float* Xh, const float* Xl, const float* xnorm, int64_t n, int d, int k,
+                                  const double* centres, const double* weights, int32_t* labels, const int32_t* prev_labels,
+                                  uint64_t* n_changed, double* inertia, uint32_t* n_rechecked,
+                                  void* workspace, size_t workspace_bytes, void* stream);
+int ofc_kmeans_tc_sums_weighted(const float* Xh, const float* Xl, int64_t n, int d, int k, const int32_t* labels,
+                                const double* weights, double* sums, int64_t* counts, double* weight_sums,
+                                void* workspace, size_t workspace_bytes, void* stream);
+int ofc_kmeans_tc_sums_u8_weighted(const uint8_t* X, int64_t n, int d, int k, const int32_t* labels, const double* weights,
+                                   double* sums, int64_t* counts, double* weight_sums, void* workspace, size_t workspace_bytes,
+                                   void* stream);
 
 /* image_dict ROIs (KmeanGrids.py:85,113) + preprocess_image (:269-286) for every cell:
  * out u8 [n_frames][rows*cols][ (H/rows)*(W/cols) ][4] = (c0, c1, c2, alpha).  draw_lines:

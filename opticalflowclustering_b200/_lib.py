@@ -54,6 +54,11 @@ SIGNATURES = {
                                _sz, _vp]),
     "ofc_minibatch_update": (_i, [_vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp]),
     "ofc_kmeans_relocate": (_i, [_vp, _i, _i, _i64, _i, _i, _vp, _vp, _vp, _vp, _vp, _i, _vp, _vp, _vp]),
+    "ofc_kmeans_assign_weighted": (_i, [_vp, _i, _i, _i64, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "ofc_kmeans_sums_weighted": (_i, [_vp, _i, _i, _i64, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "ofc_kmeans_update_weighted": (_i, [_i, _i64, _i, _i, _vp, _vp, _vp, _i, _i, _vp, _vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp,
+                                        _vp, _vp, _sz, _vp]),
+    "ofc_kmeans_relocate_weighted": (_i, [_vp, _i, _i, _i64, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _i, _vp, _vp, _vp]),
     "ofc_kmeans_far_points": (_i, [_vp, _i, _i, _i64, _i, _i, _vp, _vp, _vp, _i, _vp, _vp, _vp, _vp]),
     "ofc_kmeans_far_payload": (_i, [_vp, _i, _i, _i64, _i, _i, _vp, _vp, _vp, _vp, _i, _i, _i64, _vp, _vp, _vp, _vp]),
     "ofc_kmeans_relocate_merge": (_i, [_i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp]),
@@ -75,6 +80,9 @@ SIGNATURES = {
     "ofc_kmeans_tc_prepare_u8": (_i, [_vp, _vp, _i64, _i, _vp, _vp, _vp, _vp]),
     "ofc_kmeans_tc_assign_u8": (_i, [_vp, _vp, _vp, _vp, _vp, _i64, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
     "ofc_kmeans_tc_sums_u8": (_i, [_vp, _i64, _i, _i, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "ofc_kmeans_tc_assign_weighted": (_i, [_vp, _vp, _vp, _i64, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "ofc_kmeans_tc_sums_weighted": (_i, [_vp, _vp, _i64, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "ofc_kmeans_tc_sums_u8_weighted": (_i, [_vp, _i64, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
     "ofc_grid_extract_cells": (_i, [_vp, _i, _i, _i, _i, _i, _i, _i, _i, _vp, _vp]),
     "ofc_sliding_cosine": (_i, [_vp, _i, _vp, _i64, _vp, _vp, _vp, _vp]),
     "ofc_row_cosine": (_i, [_vp, _i, _i64, _i, _vp, _vp, _vp]),

@@ -17,6 +17,7 @@
 // All kernels take a batch dimension (independent problems of equal shape): the
 // reference runs one fit per grid cell per frame (350 per frame).
 #include <stdlib.h>
+#include <type_traits>
 #include "ofc_common.cuh"
 #include "kmeans_kernels.cuh"
 
@@ -57,7 +58,9 @@ __device__ __forceinline__ double block_sum_256(double v, double* s_red) {
 // E-step, one thread per point: the row lives in registers (d <= DP), the
 // centres and their squared norms in shared memory.
 // ---------------------------------------------------------------------------
-template <typename T, typename W, int DP>
+// WT: p.weights is set and the inertia is sum_i w_i ||x_i - c||^2 (sklearn's _inertia_dense); labels and min_dist do
+// not depend on the weights.  Every weighted form below keeps the unweighted fold order, so unit weights give its bits.
+template <typename T, typename W, int DP, bool WT>
 __global__ void __launch_bounds__(256) kmeans_assign_small_kernel(KmAssignParams p) {
     OFC_DYN_SMEM(unsigned char, raw);
     W* sc = reinterpret_cast<W*>(raw);               // [k][d]
@@ -76,6 +79,7 @@ __global__ void __launch_bounds__(256) kmeans_assign_small_kernel(KmAssignParams
     const T* X = reinterpret_cast<const T*>(p.X) + (int64_t)b * p.x_stride;
     int32_t* labels = p.labels + (int64_t)b * p.n;
     const int32_t* prev = p.prev_labels ? p.prev_labels + (int64_t)b * p.n : nullptr;
+    const double* wt = WT ? p.weights + (int64_t)b * p.w_stride : nullptr;
     double inert = 0.0;
     unsigned changed = 0;
     for (int64_t base = (int64_t)blockIdx.x * 256; base < p.n; base += (int64_t)gridDim.x * 256) {
@@ -112,7 +116,7 @@ __global__ void __launch_bounds__(256) kmeans_assign_small_kernel(KmAssignParams
 #pragma unroll
                 for (int t = 0; t < DP; ++t)
                     if (t < d) { W df = x[t] - c[t]; sq = fma_w<W>(df, df, sq); }
-                inert += (double)sq;
+                inert += WT ? (double)sq * wt[i] : (double)sq;
                 if (p.min_dist) p.min_dist[(int64_t)b * p.n + i] = (double)sq;
             }
         }
@@ -133,7 +137,7 @@ __global__ void __launch_bounds__(256) kmeans_assign_small_kernel(KmAssignParams
 // E-step, generic shape (large d, or k*d beyond shared memory): one warp per
 // point, lanes stride over the features, centres read through L1/L2.
 // ---------------------------------------------------------------------------
-template <typename T, typename W>
+template <typename T, typename W, bool WT>
 __global__ void __launch_bounds__(256) kmeans_assign_generic_kernel(KmAssignParams p) {
     __shared__ double s_red[8];
     const int b = blockIdx.y, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, d = p.d, k = p.k;
@@ -144,6 +148,7 @@ __global__ void __launch_bounds__(256) kmeans_assign_generic_kernel(KmAssignPara
     const T* X = reinterpret_cast<const T*>(p.X) + (int64_t)b * p.x_stride;
     int32_t* labels = p.labels + (int64_t)b * p.n;
     const int32_t* prev = p.prev_labels ? p.prev_labels + (int64_t)b * p.n : nullptr;
+    const double* wt = WT ? p.weights + (int64_t)b * p.w_stride : nullptr;
     double inert = 0.0;
     unsigned changed = 0;
     for (int64_t i = (int64_t)blockIdx.x * 8 + warp; i < p.n; i += (int64_t)gridDim.x * 8) {
@@ -176,7 +181,7 @@ __global__ void __launch_bounds__(256) kmeans_assign_generic_kernel(KmAssignPara
 #pragma unroll
             for (int o = 16; o > 0; o >>= 1) sq += __shfl_xor_sync(0xffffffffu, sq, o);
             if (lane == 0) {
-                inert += (double)sq;
+                inert += WT ? (double)sq * wt[i] : (double)sq;
                 if (p.min_dist) p.min_dist[(int64_t)b * p.n + i] = (double)sq;
             }
         }
@@ -194,7 +199,7 @@ __global__ void __launch_bounds__(256) kmeans_assign_generic_kernel(KmAssignPara
 // but the centred row is loaded ONCE into registers and the centres (in the working precision) and their
 // norms live in shared memory -- X is read once per iteration and nothing else leaves the SM.
 // ---------------------------------------------------------------------------
-template <typename T, typename W, int NT>
+template <typename T, typename W, int NT, bool WT>
 __global__ void __launch_bounds__(256) kmeans_assign_medium_kernel(KmAssignParams p) {
     OFC_DYN_SMEM(unsigned char, raw);
     W* sc = reinterpret_cast<W*>(raw);                        // [k][d]
@@ -214,6 +219,7 @@ __global__ void __launch_bounds__(256) kmeans_assign_medium_kernel(KmAssignParam
     const T* X = reinterpret_cast<const T*>(p.X) + (int64_t)b * p.x_stride;
     int32_t* labels = p.labels + (int64_t)b * p.n;
     const int32_t* prev = p.prev_labels ? p.prev_labels + (int64_t)b * p.n : nullptr;
+    const double* wt = WT ? p.weights + (int64_t)b * p.w_stride : nullptr;
     double inert = 0.0;
     unsigned changed = 0;
     for (int64_t i = (int64_t)blockIdx.x * 8 + warp; i < p.n; i += (int64_t)gridDim.x * 8) {
@@ -245,7 +251,7 @@ __global__ void __launch_bounds__(256) kmeans_assign_medium_kernel(KmAssignParam
 #pragma unroll
             for (int o = 16; o > 0; o >>= 1) sq += __shfl_xor_sync(0xffffffffu, sq, o);
             if (lane == 0) {
-                inert += (double)sq;
+                inert += WT ? (double)sq * wt[i] : (double)sq;
                 if (p.min_dist) p.min_dist[(int64_t)b * p.n + i] = (double)sq;
             }
         }
@@ -286,12 +292,16 @@ __global__ void inertia_reduce_kernel(const double* partial, int parts, double* 
 // into G = 32/dt lane groups, group g of warp w owns accumulator copy (w, g) of
 // [kt][dt] doubles and walks its own subsequence of the split's points, so no
 // two lanes ever touch the same word.  Copies are folded in index order.
+// WT (weighted, _k_means_lloyd.pyx:216-218): every member adds (x - mean) w and
+// its weight w to a float64 weight accumulator in place of the integer count.
 // ---------------------------------------------------------------------------
-template <typename T>
+template <typename T, bool WT>
 __global__ void __launch_bounds__(256) kmeans_sums_kernel(KmSumsParams p) {
+    using Cnt = typename std::conditional<WT, double, int>::type;
+    using CntSum = typename std::conditional<WT, double, long long>::type;
     OFC_DYN_SMEM(double, acc);                         // [8*G][kt][dt]
     const int dt = p.dt, G = 32 / dt, kt = p.kt, d = p.d, k = p.k;
-    int* cnt = reinterpret_cast<int*>(acc + (size_t)8 * G * kt * dt);   // [8*G][kt]
+    Cnt* cnt = reinterpret_cast<Cnt*>(acc + (size_t)8 * G * kt * dt);   // [8*G][kt]
     const int split = blockIdx.x, dtile = blockIdx.y, b = blockIdx.z;
     if (p.active && !p.active[b]) return;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -301,10 +311,11 @@ __global__ void __launch_bounds__(256) kmeans_sums_kernel(KmSumsParams p) {
     const int64_t lo = (int64_t)split * chunk, hi = lo + chunk < p.n ? lo + chunk : p.n;
     const int copy = warp * G + g;
     double* my = acc + (size_t)copy * kt * dt + t;
-    int* mycnt = cnt + copy * kt;
+    Cnt* mycnt = cnt + copy * kt;
     const double m = (p.mean && dim_ok) ? p.mean[(int64_t)b * d + dim] : 0.0;
     const T* X = reinterpret_cast<const T*>(p.X) + (int64_t)b * p.x_stride;
     const int32_t* labels = p.labels ? p.labels + (int64_t)b * p.n : nullptr;
+    const double* wt = WT ? p.weights + (int64_t)b * p.w_stride : nullptr;
 
     for (int k0 = 0; k0 < k; k0 += kt) {
         const int kk = k - k0 < kt ? k - k0 : kt;
@@ -319,9 +330,13 @@ __global__ void __launch_bounds__(256) kmeans_sums_kernel(KmSumsParams p) {
                 if (dim_ok) {
                     double v = (double)X[i * d + dim] - m;
                     if (p.square) v *= v;
+                    if (WT) v *= wt[i];
                     my[j * dt] += v;
                 }
-                if (t == 0) mycnt[j] += 1;
+                if (t == 0) {
+                    if constexpr (WT) mycnt[j] += wt[i];
+                    else mycnt[j] += 1;
+                }
             }
         }
         __syncthreads();
@@ -334,9 +349,10 @@ __global__ void __launch_bounds__(256) kmeans_sums_kernel(KmSumsParams p) {
         }
         if (dtile == 0) {
             for (int j = tid; j < kk; j += 256) {
-                long long c = 0;
+                CntSum c = 0;
                 for (int q = 0; q < 8 * G; ++q) c += cnt[q * kt + j];
-                p.cnt_partial[((int64_t)b * p.splits + split) * k + k0 + j] = c;
+                if (WT) p.wcnt_partial[((int64_t)b * p.splits + split) * k + k0 + j] = (double)c;
+                else p.cnt_partial[((int64_t)b * p.splits + split) * k + k0 + j] = (long long)c;
             }
         }
         __syncthreads();
@@ -430,9 +446,10 @@ __global__ void __launch_bounds__(256) kmeans_step_u8_kernel(KmAssignParams p, d
     }
 }
 
-// sums[b][j][t] = sum over splits (in split order) of the partials; counts likewise
-__global__ void kmeans_fold_kernel(const double* partial, const long long* cnt_partial, int splits, int k, int d,
-                                   double* sums, long long* counts, const unsigned char* active) {
+// sums[b][j][t] = sum over splits (in split order) of the partials; counts (or weight sums) likewise
+template <typename C>
+__global__ void kmeans_fold_kernel(const double* partial, const C* cnt_partial, int splits, int k, int d,
+                                   double* sums, C* counts, const unsigned char* active) {
     const int b = blockIdx.y;
     if (active && !active[b]) return;
     const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -443,7 +460,7 @@ __global__ void kmeans_fold_kernel(const double* partial, const long long* cnt_p
         sums[(int64_t)b * kd + e] = s;
     }
     if (e < k && counts) {
-        long long c = 0;
+        C c = 0;
         for (int sp = 0; sp < splits; ++sp) c += cnt_partial[((int64_t)b * splits + sp) * k + e];
         counts[(int64_t)b * k + e] = c;
     }
@@ -504,9 +521,11 @@ __global__ void __launch_bounds__(256) kmeans_centres_kernel(int d, int k, const
 // <= tol.  Stopped problems clear their `active` byte (every kernel skips them from then on) and raise
 // `just_done` (their labels are copied into both label buffers by kmeans_freeze_labels_kernel); the number
 // of problems still running is accumulated in *n_active, which the host reads asynchronously, a few
-// iterations behind, to know when to stop enqueuing.  One CTA per problem.
+// iterations behind, to know when to stop enqueuing.  One CTA per problem.  CW = double: `counts` are the float64
+// weight sums of a weighted fit (_average_centers: empty = weight 0, np.argmax of the weights).
 // ---------------------------------------------------------------------------
-__global__ void __launch_bounds__(256) kmeans_update_kernel(int d, int k, const double* sums, const long long* counts,
+template <typename CW>
+__global__ void __launch_bounds__(256) kmeans_update_kernel(int d, int k, const double* sums, const CW* counts,
                                                             const double* mean_sub, int use_reciprocal, int round_f32,
                                                             double* centres, double* shift_tot, double* shift_ws,
                                                             const unsigned long long* n_changed, const double* tol, int it_arg,
@@ -520,7 +539,7 @@ __global__ void __launch_bounds__(256) kmeans_update_kernel(int d, int k, const 
     if (just_done && tid == 0) just_done[b] = 0;
     if (active && !active[b]) return;
     const double* S = sums + (int64_t)b * k * d;
-    const long long* Cn = counts + (int64_t)b * k;
+    const CW* Cn = counts + (int64_t)b * k;
     double* C = centres + (int64_t)b * k * d;
     double* sh = shift_ws + (int64_t)b * k;
     __shared__ int s_heavy;
@@ -709,11 +728,13 @@ __global__ void __launch_bounds__(1024) kmeans_relocate_kernel(const T* Xall, in
 // cluster in index order, the farthest remaining row from the scratch (ties: lowest index), marks it taken and moves
 // it in the sums.  kmeans_relocate_kernel re-reads all of X once per empty cluster through ONE CTA: 369 ms per
 // launch on 1 M x 128 float32 rows with a handful of empty clusters (ncu r02e) against ~1 ms this way.
+// C = double: a weighted fit (_relocate_empty_clusters_dense): `counts` are the clusters' weight sums, a cluster is
+// empty when its weight is 0, the distances stay unweighted and the moved row carries x w and w.
 // ---------------------------------------------------------------------------
-template <typename T>
+template <typename T, typename C>
 __global__ void __launch_bounds__(256) kmeans_rowdist_kernel(const T* Xall, int64_t x_stride, int64_t n, int d, int k, const double* mean_all,
                                                              const int32_t* labels_all, const double* centres_all,
-                                                             const long long* counts_all, double* scratch_all, int force,
+                                                             const C* counts_all, double* scratch_all, int force,
                                                              const unsigned char* active) {
     const int b = blockIdx.y, tid = threadIdx.x;
     if (active && !active[b]) return;
@@ -721,7 +742,7 @@ __global__ void __launch_bounds__(256) kmeans_rowdist_kernel(const T* Xall, int6
     if (!force) {
         if (tid == 0) s_any = 0;
         __syncthreads();
-        const long long* counts = counts_all + (int64_t)b * k;
+        const C* counts = counts_all + (int64_t)b * k;
         int any = 0;
         for (int j = tid; j < k; j += 256) any |= counts[j] == 0;
         if (any) s_any = 1;
@@ -772,13 +793,15 @@ __device__ __forceinline__ void block_argmax_1024(const double* scratch, int64_t
     out_i = idx;
 }
 
-template <typename T>
+template <typename T, typename C>
 __global__ void __launch_bounds__(1024) kmeans_relocate_apply_kernel(const T* Xall, int64_t x_stride, int64_t n, int d, int k, const double* mean_all,
                                                                       const int32_t* labels_all, double* scratch_all, double* sums_all,
-                                                                      long long* counts_all, int raw_sums, const unsigned char* active) {
+                                                                      C* counts_all, int raw_sums, const unsigned char* active,
+                                                                      const double* weights_all, int64_t w_stride) {
+    constexpr bool WT = std::is_same<C, double>::value;
     const int b = blockIdx.x, tid = threadIdx.x;
     if (active && !active[b]) return;
-    long long* counts = counts_all + (int64_t)b * k;
+    C* counts = counts_all + (int64_t)b * k;
     __shared__ int s_any;
     __shared__ double s_val[32];
     __shared__ long long s_idx[32];
@@ -806,14 +829,21 @@ __global__ void __launch_bounds__(1024) kmeans_relocate_apply_kernel(const T* Xa
         if (fi < 0) return;
         ++n_taken;
         const int old = labels[fi];
+        const double wf = WT ? weights_all[(int64_t)b * w_stride + fi] : 1.0;
         for (int t = tid; t < d; t += 1024) {
-            const double x = (double)X[fi * d + t] - ((mean && !raw_sums) ? mean[t] : 0.0);
+            double x = (double)X[fi * d + t] - ((mean && !raw_sums) ? mean[t] : 0.0);
+            if (WT) x *= wf;
             sums[(int64_t)old * d + t] -= x;
             sums[(int64_t)e * d + t] = x;
         }
         if (tid == 0) {
-            counts[e] = 1;
-            counts[old] -= 1;
+            if constexpr (WT) {
+                counts[e] = wf;
+                counts[old] -= wf;
+            } else {
+                counts[e] = 1;
+                counts[old] -= 1;
+            }
             scratch[fi] = -1.0;                        // taken
         }
         __syncthreads();
@@ -1399,12 +1429,12 @@ int kmeans_sums_splits(int64_t n, int batch) {
     return (int)(want < 1 ? 1 : want);
 }
 
-template <typename T, typename W>
+template <typename T, typename W, bool WT>
 static int assign_small_dispatch(const KmAssignParams& p, dim3 grid, size_t smem, void* stream) {
 #define OFC_KM_CASE(DPV)                                                                                     \
     {                                                                                                        \
-        OFC_SMEM_OPTIN((kmeans_assign_small_kernel<T, W, DPV>), smem);                                       \
-        OFC_LAUNCH((kmeans_assign_small_kernel<T, W, DPV>), grid, dim3(256), smem, stream, p);               \
+        OFC_SMEM_OPTIN((kmeans_assign_small_kernel<T, W, DPV, WT>), smem);                                   \
+        OFC_LAUNCH((kmeans_assign_small_kernel<T, W, DPV, WT>), grid, dim3(256), smem, stream, p);           \
     }
     if (p.d <= 4) OFC_KM_CASE(4)
     else if (p.d <= 8) OFC_KM_CASE(8)
@@ -1414,8 +1444,8 @@ static int assign_small_dispatch(const KmAssignParams& p, dim3 grid, size_t smem
     return OFC_OK;
 }
 
-int launch_kmeans_assign(KmAssignParams p, int batch, double* c2_ws, void* stream) {
-    if (batch <= 0 || p.n <= 0) return OFC_OK;
+template <bool WT>
+static int launch_assign(KmAssignParams p, int batch, double* c2_ws, void* stream) {
     if (batch > 65535) { set_error("batch=%d exceeds 65535", batch); return OFC_ERR_UNSUPPORTED; }
     const size_t wsz = p.dtype == DT_F32 ? 4 : 8;
     const size_t smem = ((size_t)p.k * p.d + p.k + p.d) * wsz;
@@ -1423,9 +1453,9 @@ int launch_kmeans_assign(KmAssignParams p, int batch, double* c2_ws, void* strea
     if (p.d <= 32 && smem <= 200 * 1024) {
         dim3 grid(kmeans_assign_grid(p.n), batch);
         int rc;
-        if (p.dtype == DT_U8) rc = assign_small_dispatch<unsigned char, double>(p, grid, smem, stream);
-        else if (p.dtype == DT_F32) rc = assign_small_dispatch<float, float>(p, grid, smem, stream);
-        else rc = assign_small_dispatch<double, double>(p, grid, smem, stream);
+        if (p.dtype == DT_U8) rc = assign_small_dispatch<unsigned char, double, WT>(p, grid, smem, stream);
+        else if (p.dtype == DT_F32) rc = assign_small_dispatch<float, float, WT>(p, grid, smem, stream);
+        else rc = assign_small_dispatch<double, double, WT>(p, grid, smem, stream);
         if (rc != OFC_OK) return rc;
         OFC_CHECK_LAUNCH("kmeans_assign_small");
         return OFC_OK;
@@ -1448,8 +1478,8 @@ int launch_kmeans_assign(KmAssignParams p, int batch, double* c2_ws, void* strea
     if (!seam_off("OFC_KMEANS_MEDIUM") && p.d <= 512 && msmem <= 200 * 1024) {
 #define OFC_KM_MED(TT, WW, NTV)                                                                                        \
     {                                                                                                                  \
-        OFC_SMEM_OPTIN((kmeans_assign_medium_kernel<TT, WW, NTV>), msmem);                                             \
-        OFC_LAUNCH((kmeans_assign_medium_kernel<TT, WW, NTV>), grid, dim3(256), msmem, stream, p);                     \
+        OFC_SMEM_OPTIN((kmeans_assign_medium_kernel<TT, WW, NTV, WT>), msmem);                                         \
+        OFC_LAUNCH((kmeans_assign_medium_kernel<TT, WW, NTV, WT>), grid, dim3(256), msmem, stream, p);                 \
     }
 #define OFC_KM_MED_NT(TT, WW)                                                                                          \
     {                                                                                                                  \
@@ -1469,11 +1499,17 @@ int launch_kmeans_assign(KmAssignParams p, int batch, double* c2_ws, void* strea
         OFC_CHECK_LAUNCH("kmeans_assign_medium");
         return OFC_OK;
     }
-    if (p.dtype == DT_U8) OFC_LAUNCH((kmeans_assign_generic_kernel<unsigned char, double>), grid, dim3(256), 0, stream, p);
-    else if (p.dtype == DT_F32) OFC_LAUNCH((kmeans_assign_generic_kernel<float, float>), grid, dim3(256), 0, stream, p);
-    else OFC_LAUNCH((kmeans_assign_generic_kernel<double, double>), grid, dim3(256), 0, stream, p);
+    if (p.dtype == DT_U8) OFC_LAUNCH((kmeans_assign_generic_kernel<unsigned char, double, WT>), grid, dim3(256), 0, stream, p);
+    else if (p.dtype == DT_F32) OFC_LAUNCH((kmeans_assign_generic_kernel<float, float, WT>), grid, dim3(256), 0, stream, p);
+    else OFC_LAUNCH((kmeans_assign_generic_kernel<double, double, WT>), grid, dim3(256), 0, stream, p);
     OFC_CHECK_LAUNCH("kmeans_assign_generic");
     return OFC_OK;
+}
+
+// p.weights set: the weighted-inertia instantiations (the labels are the same)
+int launch_kmeans_assign(KmAssignParams p, int batch, double* c2_ws, void* stream) {
+    if (batch <= 0 || p.n <= 0) return OFC_OK;
+    return p.weights ? launch_assign<true>(p, batch, c2_ws, stream) : launch_assign<false>(p, batch, c2_ws, stream);
 }
 
 // fold of the fused step's per-CTA partials: integers held exactly in float64, so a warp per element can
@@ -1554,17 +1590,20 @@ int launch_inertia_reduce(const double* partial, int parts, int batch, double* i
     return OFC_OK;
 }
 
-int launch_kmeans_sums(const KmSumsParams& p, int batch, double* sums, long long* counts, void* stream) {
+// C = long long: member counts; C = double: weight sums (p.weights set)
+template <typename C>
+static int launch_sums(const KmSumsParams& p, int batch, double* sums, C* counts, void* stream) {
+    constexpr bool WT = std::is_same<C, double>::value;
     if (batch <= 0) return OFC_OK;
     if (batch > 65535) { set_error("batch=%d exceeds 65535", batch); return OFC_ERR_UNSUPPORTED; }
     const int G = 32 / p.dt;
-    const size_t smem = (size_t)8 * G * p.kt * p.dt * sizeof(double) + (size_t)8 * G * p.kt * sizeof(int);
+    const size_t smem = (size_t)8 * G * p.kt * p.dt * sizeof(double) + (size_t)8 * G * p.kt * (WT ? sizeof(double) : sizeof(int));
     dim3 grid(p.splits, cdiv(p.d, p.dt), batch);
     ProfScope prof(PK_KMEANS, stream);
 #define OFC_KM_SUMS(TT)                                                                                      \
     {                                                                                                        \
-        OFC_SMEM_OPTIN(kmeans_sums_kernel<TT>, smem);                                                        \
-        OFC_LAUNCH(kmeans_sums_kernel<TT>, grid, dim3(256), smem, stream, p);                                \
+        OFC_SMEM_OPTIN((kmeans_sums_kernel<TT, WT>), smem);                                                  \
+        OFC_LAUNCH((kmeans_sums_kernel<TT, WT>), grid, dim3(256), smem, stream, p);                          \
     }
     if (p.dtype == DT_U8) OFC_KM_SUMS(unsigned char)
     else if (p.dtype == DT_F32) OFC_KM_SUMS(float)
@@ -1572,10 +1611,21 @@ int launch_kmeans_sums(const KmSumsParams& p, int batch, double* sums, long long
 #undef OFC_KM_SUMS
     OFC_CHECK_LAUNCH("kmeans_sums");
     const int64_t kd = (int64_t)p.k * p.d;
-    OFC_LAUNCH(kmeans_fold_kernel, dim3((unsigned)((kd + 255) / 256), batch), dim3(256), 0, stream, p.partial,
-               p.cnt_partial, p.splits, p.k, p.d, sums, counts, p.active);
+    const C* cnt_partial;
+    if constexpr (WT) cnt_partial = p.wcnt_partial;
+    else cnt_partial = p.cnt_partial;
+    OFC_LAUNCH(kmeans_fold_kernel<C>, dim3((unsigned)((kd + 255) / 256), batch), dim3(256), 0, stream, p.partial,
+               cnt_partial, p.splits, p.k, p.d, sums, counts, p.active);
     OFC_CHECK_LAUNCH("kmeans_fold");
     return OFC_OK;
+}
+
+int launch_kmeans_sums(const KmSumsParams& p, int batch, double* sums, long long* counts, void* stream) {
+    return launch_sums<long long>(p, batch, sums, counts, stream);
+}
+
+int launch_kmeans_sums_weighted(const KmSumsParams& p, int batch, double* sums, double* weight_sums, void* stream) {
+    return launch_sums<double>(p, batch, sums, weight_sums, stream);
 }
 
 int launch_kmeans_centres(int batch, int d, int k, const double* sums, const long long* counts, const double* mean_sub,
@@ -1589,14 +1639,15 @@ int launch_kmeans_centres(int batch, int d, int k, const double* sums, const lon
     return OFC_OK;
 }
 
-int launch_kmeans_update(int batch, int d, int k, const double* sums, const long long* counts, const double* mean_sub,
+template <typename C>
+static int launch_update(int batch, int d, int k, const double* sums, const C* counts, const double* mean_sub,
                          int use_reciprocal, int round_f32, double* centres, double* shift_tot, double* shift_ws,
                          const unsigned long long* n_changed, const double* tol, int it, unsigned char* active,
                          unsigned char* just_done, int* n_iter, int* n_active, int64_t n, const int32_t* labels_cur,
                          int32_t* labels_other, int* it_counter, void* stream) {
     if (batch <= 0) return OFC_OK;
     ProfScope prof(PK_KMEANS, stream);
-    OFC_LAUNCH(kmeans_update_kernel, dim3(batch), dim3(256), 0, stream, d, k, sums, counts, mean_sub, use_reciprocal, round_f32,
+    OFC_LAUNCH(kmeans_update_kernel<C>, dim3(batch), dim3(256), 0, stream, d, k, sums, counts, mean_sub, use_reciprocal, round_f32,
                centres, shift_tot, shift_ws, n_changed, tol, it, active, just_done, n_iter, n_active, it_counter);
     OFC_CHECK_LAUNCH("kmeans_update");
     if (it_counter) {
@@ -1610,6 +1661,24 @@ int launch_kmeans_update(int batch, int d, int k, const double* sums, const long
         OFC_CHECK_LAUNCH("kmeans_freeze_labels");
     }
     return OFC_OK;
+}
+
+int launch_kmeans_update(int batch, int d, int k, const double* sums, const long long* counts, const double* mean_sub,
+                         int use_reciprocal, int round_f32, double* centres, double* shift_tot, double* shift_ws,
+                         const unsigned long long* n_changed, const double* tol, int it, unsigned char* active,
+                         unsigned char* just_done, int* n_iter, int* n_active, int64_t n, const int32_t* labels_cur,
+                         int32_t* labels_other, int* it_counter, void* stream) {
+    return launch_update(batch, d, k, sums, counts, mean_sub, use_reciprocal, round_f32, centres, shift_tot, shift_ws, n_changed, tol,
+                         it, active, just_done, n_iter, n_active, n, labels_cur, labels_other, it_counter, stream);
+}
+
+int launch_kmeans_update(int batch, int d, int k, const double* sums, const double* weight_sums, const double* mean_sub,
+                         int use_reciprocal, int round_f32, double* centres, double* shift_tot, double* shift_ws,
+                         const unsigned long long* n_changed, const double* tol, int it, unsigned char* active,
+                         unsigned char* just_done, int* n_iter, int* n_active, int64_t n, const int32_t* labels_cur,
+                         int32_t* labels_other, int* it_counter, void* stream) {
+    return launch_update(batch, d, k, sums, weight_sums, mean_sub, use_reciprocal, round_f32, centres, shift_tot, shift_ws, n_changed,
+                         tol, it, active, just_done, n_iter, n_active, n, labels_cur, labels_other, it_counter, stream);
 }
 
 int launch_minibatch_update(const void* Xb, int dtype, int bs, int d, int k, const int32_t* labels, const double* centres_old,
@@ -1638,11 +1707,11 @@ static int rowdist_grid(int64_t n, int batch) {
     return (int)(g < cap ? (g < 1 ? 1 : g) : cap);
 }
 
-template <typename T>
+template <typename T, typename C>
 static int launch_rowdist(const void* X, int64_t x_stride, int batch, int64_t n, int d, int k, const double* mean, const int32_t* labels,
-                          const double* centres_old, const long long* counts, double* scratch, int force,
+                          const double* centres_old, const C* counts, double* scratch, int force,
                           const unsigned char* active, void* stream) {
-    OFC_LAUNCH(kmeans_rowdist_kernel<T>, dim3(rowdist_grid(n, batch), batch), dim3(256), 0, stream, (const T*)X, x_stride, n, d, k, mean, labels,
+    OFC_LAUNCH((kmeans_rowdist_kernel<T, C>), dim3(rowdist_grid(n, batch), batch), dim3(256), 0, stream, (const T*)X, x_stride, n, d, k, mean, labels,
                centres_old, counts, scratch, force, active);
     OFC_CHECK_LAUNCH("kmeans_rowdist");
     return OFC_OK;
@@ -1662,14 +1731,14 @@ int launch_kmeans_relocate(const void* X, int64_t x_stride, int dtype, int batch
         else rc = launch_rowdist<double>(X, x_stride, batch, n, d, k, mean, labels, centres_old, counts, scratch, 0, active, stream);
         if (rc != OFC_OK) return rc;
         if (dtype == DT_U8)
-            OFC_LAUNCH(kmeans_relocate_apply_kernel<unsigned char>, dim3(batch), dim3(1024), 0, stream, (const unsigned char*)X, x_stride, n, d, k, mean,
-                       labels, scratch, sums, counts, raw_sums, active);
+            OFC_LAUNCH((kmeans_relocate_apply_kernel<unsigned char, long long>), dim3(batch), dim3(1024), 0, stream, (const unsigned char*)X,
+                       x_stride, n, d, k, mean, labels, scratch, sums, counts, raw_sums, active, nullptr, 0);
         else if (dtype == DT_F32)
-            OFC_LAUNCH(kmeans_relocate_apply_kernel<float>, dim3(batch), dim3(1024), 0, stream, (const float*)X, x_stride, n, d, k, mean, labels,
-                       scratch, sums, counts, raw_sums, active);
+            OFC_LAUNCH((kmeans_relocate_apply_kernel<float, long long>), dim3(batch), dim3(1024), 0, stream, (const float*)X, x_stride, n, d, k,
+                       mean, labels, scratch, sums, counts, raw_sums, active, nullptr, 0);
         else
-            OFC_LAUNCH(kmeans_relocate_apply_kernel<double>, dim3(batch), dim3(1024), 0, stream, (const double*)X, x_stride, n, d, k, mean, labels,
-                       scratch, sums, counts, raw_sums, active);
+            OFC_LAUNCH((kmeans_relocate_apply_kernel<double, long long>), dim3(batch), dim3(1024), 0, stream, (const double*)X, x_stride, n, d,
+                       k, mean, labels, scratch, sums, counts, raw_sums, active, nullptr, 0);
         OFC_CHECK_LAUNCH("kmeans_relocate_apply");
         return OFC_OK;
     }
@@ -1690,6 +1759,35 @@ int launch_kmeans_relocate(const void* X, int64_t x_stride, int dtype, int batch
                    centres_old, sums, counts, raw_sums, active);
     OFC_CHECK_LAUNCH("kmeans_relocate");
     return OFC_OK;
+}
+
+template <typename T>
+static int relocate_weighted(const void* X, int64_t x_stride, int batch, int64_t n, int d, int k, const double* mean, const int32_t* labels,
+                             const double* centres_old, const double* weights, int64_t w_stride, double* sums, double* weight_sums,
+                             int raw_sums, const unsigned char* active, double* scratch, void* stream) {
+    int rc = launch_rowdist<T, double>(X, x_stride, batch, n, d, k, mean, labels, centres_old, weight_sums, scratch, 0, active, stream);
+    if (rc != OFC_OK) return rc;
+    OFC_LAUNCH((kmeans_relocate_apply_kernel<T, double>), dim3(batch), dim3(1024), 0, stream, (const T*)X, x_stride, n, d, k, mean, labels,
+               scratch, sums, weight_sums, raw_sums, active, weights, w_stride);
+    OFC_CHECK_LAUNCH("kmeans_relocate_apply");
+    return OFC_OK;
+}
+
+int launch_kmeans_relocate_weighted(const void* X, int64_t x_stride, int dtype, int batch, int64_t n, int d, int k, const double* mean,
+                                    const int32_t* labels, const double* centres_old, const double* weights, int64_t w_stride,
+                                    double* sums, double* weight_sums, int raw_sums, const unsigned char* active, double* scratch,
+                                    void* stream) {
+    if (batch <= 0) return OFC_OK;
+    if (batch > 65535) { set_error("batch=%d exceeds 65535", batch); return OFC_ERR_UNSUPPORTED; }
+    ProfScope prof(PK_KMEANS, stream);
+    if (dtype == DT_U8)
+        return relocate_weighted<unsigned char>(X, x_stride, batch, n, d, k, mean, labels, centres_old, weights, w_stride, sums, weight_sums,
+                                                raw_sums, active, scratch, stream);
+    if (dtype == DT_F32)
+        return relocate_weighted<float>(X, x_stride, batch, n, d, k, mean, labels, centres_old, weights, w_stride, sums, weight_sums,
+                                        raw_sums, active, scratch, stream);
+    return relocate_weighted<double>(X, x_stride, batch, n, d, k, mean, labels, centres_old, weights, w_stride, sums, weight_sums,
+                                     raw_sums, active, scratch, stream);
 }
 
 int launch_kmeans_far_payload(const void* X, int dtype, int batch, int64_t n, int d, int k, const double* mean, const int32_t* labels,
@@ -1735,9 +1833,9 @@ int launch_kmeans_far_points(const void* X, int dtype, int batch, int64_t n, int
     ProfScope prof(PK_KMEANS, stream);
     if (scratch) {
         int rc;
-        if (dtype == DT_U8) rc = launch_rowdist<unsigned char>(X, (int64_t)n * d, batch, n, d, k, mean, labels, centres_old, nullptr, scratch, 1, nullptr, stream);
-        else if (dtype == DT_F32) rc = launch_rowdist<float>(X, (int64_t)n * d, batch, n, d, k, mean, labels, centres_old, nullptr, scratch, 1, nullptr, stream);
-        else rc = launch_rowdist<double>(X, (int64_t)n * d, batch, n, d, k, mean, labels, centres_old, nullptr, scratch, 1, nullptr, stream);
+        if (dtype == DT_U8) rc = launch_rowdist<unsigned char>(X, (int64_t)n * d, batch, n, d, k, mean, labels, centres_old, (const long long*)nullptr, scratch, 1, nullptr, stream);
+        else if (dtype == DT_F32) rc = launch_rowdist<float>(X, (int64_t)n * d, batch, n, d, k, mean, labels, centres_old, (const long long*)nullptr, scratch, 1, nullptr, stream);
+        else rc = launch_rowdist<double>(X, (int64_t)n * d, batch, n, d, k, mean, labels, centres_old, (const long long*)nullptr, scratch, 1, nullptr, stream);
         if (rc != OFC_OK) return rc;
         OFC_LAUNCH(kmeans_far_list_kernel, dim3(batch), dim3(1024), 0, stream, n, scratch, n_far, out_val, out_idx);
         OFC_CHECK_LAUNCH("kmeans_far_list");

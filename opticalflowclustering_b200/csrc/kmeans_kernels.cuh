@@ -23,6 +23,8 @@ struct KmAssignParams {
     double* inertia_partial;     // [batch][gridDim.x] or null
     double* min_dist;            // [batch][n] squared distance to the chosen centre, or null
     const unsigned char* active; // [batch] problems to process (null = all)
+    const double* weights = nullptr;   // [batch][n] sample weights (inertia = sum w_i d_i), or null (unweighted)
+    int64_t w_stride = 0;        // n, or 0 when every problem reads one [n] vector (OFC_KMEANS_SHARED_ROWS)
 };
 
 struct KmSumsParams {
@@ -40,10 +42,15 @@ struct KmSumsParams {
     int dt;                      // dims per lane group (power of two <= 32)
     int kt;                      // clusters per shared-memory pass
     const unsigned char* active; // [batch] or null
+    const double* weights = nullptr;   // as in KmAssignParams: sums of x w and weight sums instead of member counts
+    int64_t w_stride = 0;
+    double* wcnt_partial = nullptr;    // [batch][splits][k] weight partials (weighted only; in place of cnt_partial)
 };
 
 int launch_kmeans_assign(KmAssignParams p, int batch, double* c2_ws, void* stream);
 int launch_kmeans_sums(const KmSumsParams& p, int batch, double* sums, long long* counts, void* stream);
+// p.weights set: weight_sums[b][j] = sum of the members' weights (float64) in place of the member counts
+int launch_kmeans_sums_weighted(const KmSumsParams& p, int batch, double* sums, double* weight_sums, void* stream);
 // fused E-step + M-step sums for uint8 rows whose [k][d] accumulators fit shared memory (one pass over X)
 int kmeans_step_grid(int64_t n, int batch);
 size_t kmeans_step_smem(int d, int k);
@@ -57,11 +64,23 @@ int launch_kmeans_update(int batch, int d, int k, const double* sums, const long
                          const unsigned long long* n_changed, const double* tol, int it, unsigned char* active,
                          unsigned char* just_done, int* n_iter, int* n_active, int64_t n, const int32_t* labels_cur,
                          int32_t* labels_other, int* it_counter, void* stream);
+// the same driven by float64 cluster weights (empty = weight 0, the heaviest cluster by weight)
+int launch_kmeans_update(int batch, int d, int k, const double* sums, const double* weight_sums, const double* mean_sub,
+                         int use_reciprocal, int round_f32, double* centres, double* shift_tot, double* shift_ws,
+                         const unsigned long long* n_changed, const double* tol, int it, unsigned char* active,
+                         unsigned char* just_done, int* n_iter, int* n_active, int64_t n, const int32_t* labels_cur,
+                         int32_t* labels_other, int* it_counter, void* stream);
 int launch_minibatch_update(const void* Xb, int dtype, int bs, int d, int k, const int32_t* labels, const double* centres_old,
                             double* centres_new, double* weight_sums, void* stream);
 int launch_kmeans_relocate(const void* X, int64_t x_stride, int dtype, int batch, int64_t n, int d, int k, const double* mean,
                            const int32_t* labels, const double* centres_old, double* sums, long long* counts,
                            int raw_sums, const unsigned char* active, double* scratch, void* stream);
+// weighted: a cluster is empty when its weight is 0; the moved row carries x w and w (weights [batch][n], w_stride n or 0);
+// always the two-kernel form (scratch required)
+int launch_kmeans_relocate_weighted(const void* X, int64_t x_stride, int dtype, int batch, int64_t n, int d, int k, const double* mean,
+                                    const int32_t* labels, const double* centres_old, const double* weights, int64_t w_stride,
+                                    double* sums, double* weight_sums, int raw_sums, const unsigned char* active, double* scratch,
+                                    void* stream);
 int launch_kmeans_far_payload(const void* X, int dtype, int batch, int64_t n, int d, int k, const double* mean, const int32_t* labels,
                               const double* centres_old, const long long* counts, int raw_sums, int n_far, long long row_offset,
                               double* payload, double* scratch, const unsigned char* active, void* stream);

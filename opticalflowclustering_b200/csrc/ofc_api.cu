@@ -755,6 +755,31 @@ int ofc_kmeans_assign(const void* X, int dtype, int batch, int64_t n, int d, int
     return OFC_OK;
 }
 
+int ofc_kmeans_assign_weighted(const void* X, int dtype, int batch, int64_t n, int d, int k, const double* mean,
+                               const double* centres, const double* weights, int32_t* labels, const int32_t* prev_labels,
+                               uint64_t* n_changed, double* inertia, double* min_dist, const uint8_t* active, void* workspace,
+                               size_t workspace_bytes, void* stream) {
+    bool shared;
+    int rc = km_check(X, dtype, shared, batch, n, d, k);
+    if (rc != OFC_OK) return rc;
+    if (batch == 0 || n == 0) return OFC_OK;
+    OFC_REQUIRE(centres && labels && weights, "null centres / labels / weights");
+    KmWorkspace w = km_layout(batch, n, d, k, shared);
+    if (!workspace || workspace_bytes < w.assign_total) { set_error("k-means workspace too small: %zu < %zu", workspace_bytes, w.assign_total); return OFC_ERR_WORKSPACE; }
+    char* ws = (char*)workspace;
+    KmAssignParams p;
+    p.X = X; p.x_stride = shared ? 0 : n * d; p.dtype = dtype; p.n = n; p.d = d; p.k = k; p.mean = mean; p.centres = centres; p.c2 = nullptr;
+    p.labels = labels; p.prev_labels = prev_labels; p.n_changed = (unsigned long long*)n_changed;
+    p.inertia_partial = inertia ? (double*)(ws + w.off_inertia) : nullptr;
+    p.min_dist = min_dist; p.active = active;
+    p.weights = weights; p.w_stride = shared ? 0 : n;
+    if (n_changed) OFC_CUDA(cudaMemsetAsync(n_changed, 0, sizeof(uint64_t) * batch, (cudaStream_t)stream));
+    rc = launch_kmeans_assign(p, batch, (double*)(ws + w.off_c2), stream);
+    if (rc != OFC_OK) return rc;
+    if (inertia) return launch_inertia_reduce((const double*)(ws + w.off_inertia), w.parts, batch, inertia, active, stream);
+    return OFC_OK;
+}
+
 int ofc_kmeans_sums(const void* X, int dtype, int batch, int64_t n, int d, int k, const double* mean,
                     const int32_t* labels, int square, double* sums, int64_t* counts, const uint8_t* active,
                     void* workspace, size_t workspace_bytes, void* stream) {
@@ -772,6 +797,27 @@ int ofc_kmeans_sums(const void* X, int dtype, int batch, int64_t n, int d, int k
     p.partial = (double*)(ws + w.off_partial); p.cnt_partial = (long long*)(ws + w.off_cnt);
     p.splits = w.splits; p.dt = w.dt; p.kt = w.kt; p.active = active;
     return launch_kmeans_sums(p, batch, sums, (long long*)counts, stream);
+}
+
+int ofc_kmeans_sums_weighted(const void* X, int dtype, int batch, int64_t n, int d, int k, const double* mean,
+                             const int32_t* labels, const double* weights, double* sums, double* weight_sums,
+                             const uint8_t* active, void* workspace, size_t workspace_bytes, void* stream) {
+    bool shared;
+    int rc = km_check(X, dtype, shared, batch, n, d, k);
+    if (rc != OFC_OK) return rc;
+    if (batch == 0) return OFC_OK;
+    OFC_REQUIRE(sums && weight_sums && labels && weights, "null sums / weight_sums / labels / weights");
+    OFC_REQUIRE(n > 0, "empty data");
+    KmWorkspace w = km_layout(batch, n, d, k, shared);
+    if (!workspace || workspace_bytes < w.total) { set_error("k-means workspace too small: %zu < %zu", workspace_bytes, w.total); return OFC_ERR_WORKSPACE; }
+    char* ws = (char*)workspace;
+    KmSumsParams p;
+    p.X = X; p.x_stride = shared ? 0 : n * d; p.dtype = dtype; p.n = n; p.d = d; p.k = k; p.mean = mean; p.labels = labels; p.square = 0;
+    p.partial = (double*)(ws + w.off_partial); p.cnt_partial = nullptr;
+    p.splits = w.splits; p.dt = w.dt; p.kt = w.kt; p.active = active;
+    // the weight partials take the place of the count partials (8 bytes each as well)
+    p.weights = weights; p.w_stride = shared ? 0 : n; p.wcnt_partial = (double*)(ws + w.off_cnt);
+    return launch_kmeans_sums_weighted(p, batch, sums, weight_sums, stream);
 }
 
 int ofc_kmeans_step_supported(int dtype, int d, int k) {
@@ -827,6 +873,20 @@ int ofc_kmeans_update(int batch, int64_t n, int d, int k, const double* sums, co
                                 n_active, n, labels_cur, labels_other, it_counter, stream);
 }
 
+int ofc_kmeans_update_weighted(int batch, int64_t n, int d, int k, const double* sums, const double* weight_sums,
+                               const double* mean_sub, int use_reciprocal, int round_f32, double* centres, double* shift_tot,
+                               const uint64_t* n_changed, const double* tol, int iteration, uint8_t* active, uint8_t* just_done,
+                               int32_t* n_iter, int32_t* n_active, const int32_t* labels_cur, int32_t* labels_other,
+                               int32_t* it_counter, void* workspace, size_t workspace_bytes, void* stream) {
+    OFC_REQUIRE(batch >= 0 && d >= 1 && k >= 1 && n >= 0, "bad shape");
+    if (batch == 0) return OFC_OK;
+    OFC_REQUIRE(sums && weight_sums && centres, "null buffer");
+    OFC_REQUIRE(workspace && workspace_bytes >= align_up((size_t)batch * k * 8, 256), "k-means workspace too small");
+    return launch_kmeans_update(batch, d, k, sums, weight_sums, mean_sub, use_reciprocal, round_f32, centres, shift_tot,
+                                (double*)workspace, (const unsigned long long*)n_changed, tol, iteration, active, just_done, n_iter,
+                                n_active, n, labels_cur, labels_other, it_counter, stream);
+}
+
 int ofc_minibatch_update(const void* Xb, int dtype, int batch_rows, int d, int k, const int32_t* labels, const double* centres_old,
                          double* centres_new, double* weight_sums, void* stream) {
     OFC_REQUIRE(dtype == OFC_U8 || dtype == OFC_F32 || dtype == OFC_F64, "bad dtype %d", dtype);
@@ -845,6 +905,18 @@ int ofc_kmeans_relocate(const void* X, int dtype, int batch, int64_t n, int d, i
     OFC_REQUIRE(labels && centres_old && sums && counts, "null buffer");
     return launch_kmeans_relocate(X, shared ? 0 : n * d, dtype, batch, n, d, k, mean, labels, centres_old, sums, (long long*)counts, raw_sums, active, scratch,
                                   stream);
+}
+
+int ofc_kmeans_relocate_weighted(const void* X, int dtype, int batch, int64_t n, int d, int k, const double* mean,
+                                 const int32_t* labels, const double* centres_old, const double* weights, double* sums,
+                                 double* weight_sums, int raw_sums, const uint8_t* active, double* scratch, void* stream) {
+    bool shared;
+    int rc = km_check(X, dtype, shared, batch, n, d, k);
+    if (rc != OFC_OK) return rc;
+    if (batch == 0 || n == 0) return OFC_OK;
+    OFC_REQUIRE(labels && centres_old && weights && sums && weight_sums && scratch, "null buffer");
+    return launch_kmeans_relocate_weighted(X, shared ? 0 : n * d, dtype, batch, n, d, k, mean, labels, centres_old, weights, shared ? 0 : n,
+                                           sums, weight_sums, raw_sums, active, scratch, stream);
 }
 
 int ofc_kmeans_far_points(const void* X, int dtype, int batch, int64_t n, int d, int k, const double* mean, const int32_t* labels,

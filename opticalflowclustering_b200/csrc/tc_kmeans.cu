@@ -560,10 +560,12 @@ __global__ void __launch_bounds__(256) labels_changed_kernel(const int32_t* __re
 }
 
 // inertia partials: sum over the rows of a CTA of ||x - c_label||^2 (float32 per row like the assign kernels,
-// float64 across rows), one warp per row, fixed order inside the CTA; folded in CTA order afterwards
+// float64 across rows), one warp per row, fixed order inside the CTA; folded in CTA order afterwards.
+// WT: each row's term times its weight (unit weights give the unweighted bits)
+template <bool WT>
 __global__ void __launch_bounds__(256) inertia_rows_kernel(const float* __restrict__ Xh, const float* __restrict__ Xl, int64_t n, int d,
-                                                           const float* __restrict__ C,
-                                                           const int32_t* __restrict__ labels, double* __restrict__ partial) {
+                                                           const float* __restrict__ C, const int32_t* __restrict__ labels,
+                                                           const double* __restrict__ weights, double* __restrict__ partial) {
     __shared__ double s_w[8];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     double acc = 0.0;
@@ -575,7 +577,7 @@ __global__ void __launch_bounds__(256) inertia_rows_kernel(const float* __restri
         for (int t = lane; t < d; t += 32) { const float df = (rh[t] + rl[t]) - c[t]; sq = fmaf(df, df, sq); }
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) sq += __shfl_xor_sync(0xffffffffu, sq, o);
-        acc += (double)sq;
+        acc += WT ? (double)sq * weights[i] : (double)sq;
     }
     if (lane == 0) s_w[warp] = acc;
     __syncthreads();
@@ -601,6 +603,8 @@ __global__ void fold_partials_kernel(const double* __restrict__ partial, int par
 //   3  csr_scatter: the same walk as (1) writes the row indices -- ascending inside every cluster
 //   4  seg_sums:    grid (segment, 128-feature tile): float64 sums of the segment's rows, in list order
 //   5  seg_fold:    sums[j][t] = the cluster's segment partials in order; counts[j]
+// Weighted (WT, _k_means_lloyd.pyx:216-218): every row adds x w, and one more column (t == d) sums the weights, folded
+// into weight_sums[j]; same list order, so unit weights give the unweighted bits.
 // ---------------------------------------------------------------------------
 constexpr int CHUNK = 1024;
 constexpr int SEG = 512;
@@ -689,14 +693,25 @@ __global__ void __launch_bounds__(1024) csr_scan_kernel(unsigned* __restrict__ t
     }
 }
 
-// uint8 rows: sums of the raw bytes (exact integers in float64, what ofc_kmeans_sums gives for OFC_U8)
+// uint8 rows: sums of the raw bytes (exact integers in float64, what ofc_kmeans_sums gives for OFC_U8); weighted: float64
+// sums of x w in list order (exact for integer weights while the sums stay below 2^53)
+template <bool WT>
 __global__ void __launch_bounds__(128) seg_sums_u8_kernel(const unsigned char* __restrict__ X, int d, const int32_t* __restrict__ order,
                                                           const int4* __restrict__ seg_info, const int* __restrict__ n_segs,
-                                                          double* __restrict__ partial) {
+                                                          const double* __restrict__ weights, double* __restrict__ partial) {
     const int t = blockIdx.y * 128 + threadIdx.x;
     for (int s = blockIdx.x; s < *n_segs; s += gridDim.x) {
         const int4 si = seg_info[s];
-        if (t < d) {
+        if constexpr (WT) {
+            if (t <= d) {
+                double acc = 0.0;
+                for (int m = si.y; m < si.z; ++m) {
+                    const int64_t r = order[m];
+                    acc += t == d ? weights[r] : (double)X[r * d + t] * weights[r];
+                }
+                partial[(int64_t)s * (d + 1) + t] = acc;
+            }
+        } else if (t < d) {
             unsigned long long acc = 0;
             int m = si.y;
             for (; m + 4 <= si.z; m += 4) {
@@ -710,36 +725,45 @@ __global__ void __launch_bounds__(128) seg_sums_u8_kernel(const unsigned char* _
     }
 }
 
+template <bool WT>
 __global__ void __launch_bounds__(128) seg_sums_kernel(const float* __restrict__ Xh, const float* __restrict__ Xl, int d,
                                                        const int32_t* __restrict__ order,
                                                        const int4* __restrict__ seg_info, const int* __restrict__ n_segs,
-                                                       double* __restrict__ partial) {
+                                                       const double* __restrict__ weights, double* __restrict__ partial) {
     const int t = blockIdx.y * 128 + threadIdx.x;
+    const int dp = WT ? d + 1 : d;                   // partial columns: the features (+ the weight)
+    // one member's term: x (h + l exactly), x w, or (column d) w
+    auto term = [&](int64_t r) -> double {
+        if (WT && t == d) return weights[r];
+        const int64_t o = r * d + t;
+        const double x = (double)(Xh[o] + Xl[o]);
+        return WT ? x * weights[r] : x;
+    };
     for (int s = blockIdx.x; s < *n_segs; s += gridDim.x) {
         const int4 si = seg_info[s];
         double acc = 0.0;
-        if (t < d) {
+        if (t < dp) {
             int m = si.y;
             for (; m + 4 <= si.z; m += 4) {
-                const int64_t o0 = (int64_t)order[m] * d + t, o1 = (int64_t)order[m + 1] * d + t;
-                const int64_t o2 = (int64_t)order[m + 2] * d + t, o3 = (int64_t)order[m + 3] * d + t;
-                const float h0 = Xh[o0], h1 = Xh[o1], h2 = Xh[o2], h3 = Xh[o3];
-                const float l0 = Xl[o0], l1 = Xl[o1], l2 = Xl[o2], l3 = Xl[o3];
-                acc += (double)(h0 + l0); acc += (double)(h1 + l1); acc += (double)(h2 + l2); acc += (double)(h3 + l3);
+                const double a0 = term(order[m]), a1 = term(order[m + 1]), a2 = term(order[m + 2]), a3 = term(order[m + 3]);
+                acc += a0; acc += a1; acc += a2; acc += a3;
             }
-            for (; m < si.z; ++m) { const int64_t o = (int64_t)order[m] * d + t; acc += (double)(Xh[o] + Xl[o]); }
-            partial[(int64_t)s * d + t] = acc;
+            for (; m < si.z; ++m) acc += term(order[m]);
+            partial[(int64_t)s * dp + t] = acc;
         }
     }
 }
 
+template <bool WT>
 __global__ void __launch_bounds__(128) seg_fold_kernel(const double* __restrict__ partial, int d, const int* __restrict__ seg_first,
-                                                       double* __restrict__ sums) {
+                                                       double* __restrict__ sums, double* __restrict__ weight_sums) {
     const int j = blockIdx.x, t = blockIdx.y * 128 + threadIdx.x;
-    if (t >= d) return;
+    const int dp = WT ? d + 1 : d;
+    if (t >= dp) return;
     double s = 0.0;
-    for (int g = seg_first[j]; g < seg_first[j + 1]; ++g) s += partial[(int64_t)g * d + t];
-    sums[(int64_t)j * d + t] = s;
+    for (int g = seg_first[j]; g < seg_first[j + 1]; ++g) s += partial[(int64_t)g * dp + t];
+    if (WT && t == d) weight_sums[j] = s;
+    else sums[(int64_t)j * d + t] = s;
 }
 
 // ---------------------------------------------------------------------------
@@ -810,7 +834,7 @@ TcLayout tc_layout(int64_t n, int d, int k) {
     w.off_segfirst = take((size_t)(k + 1) * 4);
     w.off_seginfo = take((size_t)w.max_segs * 16);
     w.off_nsegs = take(4);
-    w.off_segpart = take((size_t)w.max_segs * d * 8);
+    w.off_segpart = take((size_t)w.max_segs * (d + 1) * 8);     // + 1: the weight column of a weighted M-step
     w.off_fixrows = take((size_t)148 * 4 * 8 * d * 8);
     w.total = off;
     return w;
@@ -879,7 +903,8 @@ int ofc_kmeans_tc_prepare(const float* X, const double* mean, int64_t n, int d, 
 // X8 != null: the rows are uint8 (worked in float64): float64 squared norms, float64 re-evaluation on the bytes
 static int tc_assign_impl(const float* Xh, const float* Xl, const float* xnorm, int64_t n, int d, int k, const double* centres,
                           int32_t* labels, const int32_t* prev_labels, uint64_t* n_changed, double* inertia, uint32_t* n_rechecked,
-                          void* workspace, size_t workspace_bytes, void* stream, const uint8_t* X8, const double* mean8) {
+                          void* workspace, size_t workspace_bytes, void* stream, const uint8_t* X8, const double* mean8,
+                          const double* weights) {
     int rc = tc_shape_ok(n, d, k);
     if (rc != OFC_OK) return rc;
     OFC_REQUIRE(Xh && Xl && xnorm && centres && labels, "null buffer");
@@ -959,7 +984,8 @@ static int tc_assign_impl(const float* Xh, const float* Xl, const float* xnorm, 
     if (inertia) {
         int64_t g = (n + 7) / 8;
         if (g > w.parts) g = w.parts;
-        inertia_rows_kernel<<<(int)g, 256, 0, st>>>(Xh, Xl, n, d, c32, labels, (double*)(ws + w.off_part));
+        if (weights) inertia_rows_kernel<true><<<(int)g, 256, 0, st>>>(Xh, Xl, n, d, c32, labels, weights, (double*)(ws + w.off_part));
+        else inertia_rows_kernel<false><<<(int)g, 256, 0, st>>>(Xh, Xl, n, d, c32, labels, nullptr, (double*)(ws + w.off_part));
         OFC_CHECK_LAUNCH("inertia_rows");
         fold_partials_kernel<<<1, 32, 0, st>>>((const double*)(ws + w.off_part), (int)g, inertia);
         OFC_CHECK_LAUNCH("fold_partials");
@@ -971,7 +997,15 @@ int ofc_kmeans_tc_assign(const float* Xh, const float* Xl, const float* xnorm, i
                          const int32_t* prev_labels, uint64_t* n_changed, double* inertia, uint32_t* n_rechecked,
                          void* workspace, size_t workspace_bytes, void* stream) {
     return tc_assign_impl(Xh, Xl, xnorm, n, d, k, centres, labels, prev_labels, n_changed, inertia, n_rechecked, workspace,
-                          workspace_bytes, stream, nullptr, nullptr);
+                          workspace_bytes, stream, nullptr, nullptr, nullptr);
+}
+
+int ofc_kmeans_tc_assign_weighted(const float* Xh, const float* Xl, const float* xnorm, int64_t n, int d, int k, const double* centres,
+                                  const double* weights, int32_t* labels, const int32_t* prev_labels, uint64_t* n_changed,
+                                  double* inertia, uint32_t* n_rechecked, void* workspace, size_t workspace_bytes, void* stream) {
+    OFC_REQUIRE(weights != nullptr, "null weights");
+    return tc_assign_impl(Xh, Xl, xnorm, n, d, k, centres, labels, prev_labels, n_changed, inertia, n_rechecked, workspace,
+                          workspace_bytes, stream, nullptr, nullptr, weights);
 }
 
 int ofc_kmeans_tc_assign_u8(const uint8_t* X, const double* mean, const float* Xh, const float* Xl, const float* xnorm, int64_t n, int d,
@@ -979,7 +1013,7 @@ int ofc_kmeans_tc_assign_u8(const uint8_t* X, const double* mean, const float* X
                             uint32_t* n_rechecked, void* workspace, size_t workspace_bytes, void* stream) {
     OFC_REQUIRE(X != nullptr, "null rows");
     return tc_assign_impl(Xh, Xl, xnorm, n, d, k, centres, labels, prev_labels, n_changed, nullptr, n_rechecked, workspace,
-                          workspace_bytes, stream, X, mean);
+                          workspace_bytes, stream, X, mean, nullptr);
 }
 
 int ofc_kmeans_tc_prepare_u8(const uint8_t* X, const double* mean, int64_t n, int d, float* Xh, float* Xl, float* xnorm, void* stream) {
@@ -993,7 +1027,8 @@ int ofc_kmeans_tc_prepare_u8(const uint8_t* X, const double* mean, int64_t n, in
 }
 
 static int tc_sums_impl(const float* Xh, const float* Xl, const uint8_t* X8, int64_t n, int d, int k, const int32_t* labels, double* sums,
-                        int64_t* counts, void* workspace, size_t workspace_bytes, void* stream);
+                        int64_t* counts, void* workspace, size_t workspace_bytes, void* stream, const double* weights = nullptr,
+                        double* weight_sums = nullptr);
 
 int ofc_kmeans_tc_sums(const float* Xh, const float* Xl, int64_t n, int d, int k, const int32_t* labels, double* sums, int64_t* counts,
                        void* workspace, size_t workspace_bytes, void* stream) {
@@ -1007,8 +1042,22 @@ int ofc_kmeans_tc_sums_u8(const uint8_t* X, int64_t n, int d, int k, const int32
     return tc_sums_impl(nullptr, nullptr, X, n, d, k, labels, sums, counts, workspace, workspace_bytes, stream);
 }
 
+int ofc_kmeans_tc_sums_weighted(const float* Xh, const float* Xl, int64_t n, int d, int k, const int32_t* labels, const double* weights,
+                                double* sums, int64_t* counts, double* weight_sums, void* workspace, size_t workspace_bytes,
+                                void* stream) {
+    OFC_REQUIRE(Xh && Xl && weights && weight_sums, "null buffer");
+    return tc_sums_impl(Xh, Xl, nullptr, n, d, k, labels, sums, counts, workspace, workspace_bytes, stream, weights, weight_sums);
+}
+
+int ofc_kmeans_tc_sums_u8_weighted(const uint8_t* X, int64_t n, int d, int k, const int32_t* labels, const double* weights, double* sums,
+                                   int64_t* counts, double* weight_sums, void* workspace, size_t workspace_bytes, void* stream) {
+    OFC_REQUIRE(X && weights && weight_sums, "null buffer");
+    return tc_sums_impl(nullptr, nullptr, X, n, d, k, labels, sums, counts, workspace, workspace_bytes, stream, weights, weight_sums);
+}
+
 static int tc_sums_impl(const float* Xh, const float* Xl, const uint8_t* X8, int64_t n, int d, int k, const int32_t* labels, double* sums,
-                        int64_t* counts, void* workspace, size_t workspace_bytes, void* stream) {
+                        int64_t* counts, void* workspace, size_t workspace_bytes, void* stream, const double* weights,
+                        double* weight_sums) {
     int rc = tc_shape_ok(n, d, k);
     if (rc != OFC_OK) return rc;
     OFC_REQUIRE(labels && sums && counts, "null buffer");
@@ -1035,14 +1084,19 @@ static int tc_sums_impl(const float* Xh, const float* Xl, const uint8_t* X8, int
     OFC_CHECK_LAUNCH("csr_scan");
     csr_walk_kernel<true><<<walk_ctas, 256, walk_smem, st>>>(labels, n, k, table, order);
     OFC_CHECK_LAUNCH("csr_scatter");
-    const int dt = cdiv(d, 128);
+    const bool wt = weights != nullptr;
+    const int dt = cdiv(wt ? d + 1 : d, 128);
     int64_t gx = w.max_segs;
     const int64_t cap = (int64_t)sm_count() * 32 / dt + 1;
     if (gx > cap) gx = cap;
-    if (X8) seg_sums_u8_kernel<<<dim3((unsigned)gx, dt), 128, 0, st>>>(X8, d, order, seg_info, n_segs, partial);
-    else seg_sums_kernel<<<dim3((unsigned)gx, dt), 128, 0, st>>>(Xh, Xl, d, order, seg_info, n_segs, partial);
+    const dim3 sgrid((unsigned)gx, dt);
+    if (X8 && wt) seg_sums_u8_kernel<true><<<sgrid, 128, 0, st>>>(X8, d, order, seg_info, n_segs, weights, partial);
+    else if (X8) seg_sums_u8_kernel<false><<<sgrid, 128, 0, st>>>(X8, d, order, seg_info, n_segs, nullptr, partial);
+    else if (wt) seg_sums_kernel<true><<<sgrid, 128, 0, st>>>(Xh, Xl, d, order, seg_info, n_segs, weights, partial);
+    else seg_sums_kernel<false><<<sgrid, 128, 0, st>>>(Xh, Xl, d, order, seg_info, n_segs, nullptr, partial);
     OFC_CHECK_LAUNCH("seg_sums");
-    seg_fold_kernel<<<dim3(k, dt), 128, 0, st>>>(partial, d, seg_first, sums);
+    if (wt) seg_fold_kernel<true><<<dim3(k, dt), 128, 0, st>>>(partial, d, seg_first, sums, weight_sums);
+    else seg_fold_kernel<false><<<dim3(k, dt), 128, 0, st>>>(partial, d, seg_first, sums, nullptr);
     OFC_CHECK_LAUNCH("seg_fold");
     return OFC_OK;
 }

@@ -110,14 +110,43 @@ def _as_batch(X, device=None):
     return X.contiguous(), single
 
 
+def _check_sample_weight(sample_weight, n: int, x_dtype, rows: int = 1):
+    """sklearn's ``_check_sample_weight(sample_weight, X, dtype=X.dtype)`` as KMeans uses it: ``None`` stays None, a number
+    is that weight for every row, anything else must be ``(n,)`` (or ``(rows, n)`` for a batch of problems).  The weights
+    are cast to the working dtype (float32 for float32 rows, float64 otherwise, uint8 rows included).  All-zero weights,
+    NaN and inf raise ValueError as in sklearn; negative weights raise ValueError too (sklearn accepts them in ``fit``,
+    but its seeding then fails and an "empty" cluster means nothing).  Returns the numpy array in the working dtype."""
+    if sample_weight is None:
+        return None
+    wdt = np.float32 if x_dtype in (torch.float32, np.float32) else np.float64
+    if isinstance(sample_weight, torch.Tensor):
+        sample_weight = sample_weight.detach().cpu().numpy()
+    if np.ndim(sample_weight) == 0:
+        return np.full(n, sample_weight, dtype=wdt)
+    w = np.ascontiguousarray(np.asarray(sample_weight, dtype=wdt))
+    if w.shape != (n,) and not (rows > 1 and w.shape == (rows, n)):
+        raise ValueError(f"sample_weight.shape == {w.shape}, expected {(n,)}!")
+    if not np.isfinite(w).all():
+        raise ValueError("Input sample_weight contains NaN or infinity.")
+    if (w < 0).any():
+        raise ValueError("Negative values in sample_weight: KMeans takes non-negative weights.")
+    if (w.reshape(-1, n) == 0).all(axis=1).any():
+        raise ValueError("Sample weights must contain at least one non-zero number.")
+    return w
+
+
 class LloydState:
     """Buffers of one batched Lloyd run (all on the data's device)."""
 
-    def __init__(self, ctx: _Ctx, X: torch.Tensor, k: int, ws_k: int | None = None, shared_batch: int | None = None):
+    def __init__(self, ctx: _Ctx, X: torch.Tensor, k: int, ws_k: int | None = None, shared_batch: int | None = None,
+                 weights: torch.Tensor | None = None):
         """``ws_k``: cluster count the stepwise workspace is sized for (1 when the tensor-core path does
         the E/M steps and only the column statistics run through the stepwise kernels).  ``shared_batch``: run that
-        many problems over the one problem of ``X`` ([1, n, d]) without copying it (OFC_KMEANS_SHARED_ROWS)."""
+        many problems over the one problem of ``X`` ([1, n, d]) without copying it (OFC_KMEANS_SHARED_ROWS).
+        ``weights``: float64 sample weights (``[B, n]``, or ``[n]`` for a shared batch) -- every E-step's inertia is
+        weighted, and ``wsum`` holds the clusters' weight sums for the weighted M-step."""
         self.ctx, self.X, self.k = ctx, X, int(k)
+        self.w = weights
         self.B, self.n, self.d = (int(s) for s in X.shape)
         self.dtype = _DT[X.dtype]
         self.flags = 0                  # OR-ed into the dtype of the calls that read X
@@ -149,10 +178,17 @@ class LloydState:
         self.active = torch.ones(self.B, dtype=torch.uint8, device=dev)
         self.just_done = torch.zeros(self.B, dtype=torch.uint8, device=dev)
         self.n_iter = torch.zeros(self.B, dtype=torch.int32, device=dev)
+        self.wsum = torch.zeros((self.B, self.k), dtype=torch.float64, device=dev) if weights is not None else None
 
     # -- thin wrappers over the C-ABI -----------------------------------------------------
     def assign(self, mean, centres, labels, prev=None, n_changed=None, inertia=None, min_dist=None, active=None):
         c = self.ctx
+        if self.w is not None:
+            c.check(c.lib.ofc_kmeans_assign_weighted(_ptr(self.X), self.dtype | self.flags, self.B, C.c_int64(self.n), self.d,
+                                                     int(centres.shape[1]), _ptr(mean), _ptr(centres), _ptr(self.w), _ptr(labels),
+                                                     _ptr(prev), _ptr(n_changed), _ptr(inertia), _ptr(min_dist), _ptr(active),
+                                                     _ptr(self.ws), C.c_size_t(self.ws.numel()), c.stream()))
+            return
         c.check(c.lib.ofc_kmeans_assign(_ptr(self.X), self.dtype | self.flags, self.B, C.c_int64(self.n), self.d, int(centres.shape[1]),
                                         _ptr(mean), _ptr(centres), _ptr(labels), _ptr(prev), _ptr(n_changed),
                                         _ptr(inertia), _ptr(min_dist), _ptr(active), _ptr(self.ws),
@@ -176,6 +212,13 @@ class LloydState:
                                       _ptr(labels), int(square), _ptr(sums), _ptr(counts), _ptr(active), _ptr(self.ws),
                                       C.c_size_t(self.ws.numel()), c.stream()))
 
+    def sums_weighted(self, mean, labels, sums, wsum, active=None):
+        """weighted M-step: sums of (x - mean) w and the clusters' weight sums (float64) in place of the counts"""
+        c = self.ctx
+        c.check(c.lib.ofc_kmeans_sums_weighted(_ptr(self.X), self.dtype | self.flags, self.B, C.c_int64(self.n), self.d, self.k,
+                                               _ptr(mean), _ptr(labels), _ptr(self.w), _ptr(sums), _ptr(wsum), _ptr(active),
+                                               _ptr(self.ws), C.c_size_t(self.ws.numel()), c.stream()))
+
     def centres_(self, sums, counts, mean_sub, use_reciprocal, centres, shift, active=None):
         c = self.ctx
         c.check(c.lib.ofc_kmeans_centres(self.B, self.d, int(centres.shape[1]), _ptr(sums), _ptr(counts), _ptr(mean_sub),
@@ -184,16 +227,23 @@ class LloydState:
 
     def update_(self, sums, counts, mean_sub, use_reciprocal, round_f32, centres, n_changed, tol, it, n_active, lab, lab_other,
                 it_counter=None):
-        """new centres + sklearn's stopping rule on the device (no read-back): see ofc_kmeans_update"""
+        """new centres + sklearn's stopping rule on the device (no read-back): see ofc_kmeans_update.  float64 ``counts``
+        are the weight sums of a weighted fit (ofc_kmeans_update_weighted)"""
         c = self.ctx
-        c.check(c.lib.ofc_kmeans_update(self.B, C.c_int64(self.n), self.d, int(centres.shape[1]), _ptr(sums), _ptr(counts),
-                                        _ptr(mean_sub), int(use_reciprocal), int(round_f32), _ptr(centres), _ptr(self.shift),
-                                        _ptr(n_changed), _ptr(tol), int(it), _ptr(self.active), _ptr(self.just_done),
-                                        _ptr(self.n_iter), _ptr(n_active), _ptr(lab), _ptr(lab_other), _ptr(it_counter),
-                                        _ptr(self.ws), C.c_size_t(self.ws.numel()), c.stream()))
+        fn = c.lib.ofc_kmeans_update_weighted if counts.dtype == torch.float64 else c.lib.ofc_kmeans_update
+        c.check(fn(self.B, C.c_int64(self.n), self.d, int(centres.shape[1]), _ptr(sums), _ptr(counts), _ptr(mean_sub),
+                   int(use_reciprocal), int(round_f32), _ptr(centres), _ptr(self.shift), _ptr(n_changed), _ptr(tol), int(it),
+                   _ptr(self.active), _ptr(self.just_done), _ptr(self.n_iter), _ptr(n_active), _ptr(lab), _ptr(lab_other),
+                   _ptr(it_counter), _ptr(self.ws), C.c_size_t(self.ws.numel()), c.stream()))
 
     def relocate(self, mean, labels, centres_old, sums, counts, raw_sums, active=None):
         c = self.ctx
+        if counts.dtype == torch.float64:          # weight sums: a cluster is empty when its weight is 0
+            c.check(c.lib.ofc_kmeans_relocate_weighted(_ptr(self.X), self.dtype | self.flags, self.B, C.c_int64(self.n), self.d, self.k,
+                                                       _ptr(mean), _ptr(labels), _ptr(centres_old), _ptr(self.w), _ptr(sums),
+                                                       _ptr(counts), int(raw_sums), _ptr(active), _ptr(self.row_scratch()),
+                                                       c.stream()))
+            return
         c.check(c.lib.ofc_kmeans_relocate(_ptr(self.X), self.dtype | self.flags, self.B, C.c_int64(self.n), self.d, self.k, _ptr(mean),
                                           _ptr(labels), _ptr(centres_old), _ptr(sums), _ptr(counts), int(raw_sums),
                                           _ptr(active), _ptr(self.row_scratch()), c.stream()))
@@ -239,12 +289,29 @@ class TensorCoreSteps:
                 # inertia of the final (centres, labels): the float64 CUDA-core E-step (idempotent on the labels)
                 st.assign(self.mean.view(1, -1), centres, labels, inertia=inertia)
             return
+        if st.w is not None:
+            c.check(c.lib.ofc_kmeans_tc_assign_weighted(_ptr(self.Xh), _ptr(self.Xl), _ptr(self.xnorm), C.c_int64(st.n), st.d, st.k,
+                                                        _ptr(centres), _ptr(st.w), _ptr(labels), _ptr(prev), _ptr(n_changed),
+                                                        _ptr(inertia), _ptr(self.n_rechecked), _ptr(self.ws), C.c_size_t(self.ws_bytes),
+                                                        c.stream()))
+            return
         c.check(c.lib.ofc_kmeans_tc_assign(_ptr(self.Xh), _ptr(self.Xl), _ptr(self.xnorm), C.c_int64(st.n), st.d, st.k,
                                            _ptr(centres), _ptr(labels), _ptr(prev), _ptr(n_changed), _ptr(inertia),
                                            _ptr(self.n_rechecked), _ptr(self.ws), C.c_size_t(self.ws_bytes), c.stream()))
 
     def sums_(self, labels, sums, counts):
+        """member counts into ``counts``; a weighted fit also writes the weight sums into ``st.wsum``"""
         st, c = self.st, self.st.ctx
+        if st.w is not None:
+            if self.u8:
+                c.check(c.lib.ofc_kmeans_tc_sums_u8_weighted(_ptr(st.X), C.c_int64(st.n), st.d, st.k, _ptr(labels), _ptr(st.w),
+                                                             _ptr(sums), _ptr(counts), _ptr(st.wsum), _ptr(self.ws),
+                                                             C.c_size_t(self.ws_bytes), c.stream()))
+            else:
+                c.check(c.lib.ofc_kmeans_tc_sums_weighted(_ptr(self.Xh), _ptr(self.Xl), C.c_int64(st.n), st.d, st.k, _ptr(labels),
+                                                          _ptr(st.w), _ptr(sums), _ptr(counts), _ptr(st.wsum), _ptr(self.ws),
+                                                          C.c_size_t(self.ws_bytes), c.stream()))
+            return
         if self.u8:         # raw (exact integer) sums like the stepwise uint8 path
             c.check(c.lib.ofc_kmeans_tc_sums_u8(_ptr(st.X), C.c_int64(st.n), st.d, st.k, _ptr(labels), _ptr(sums), _ptr(counts),
                                                 _ptr(self.ws), C.c_size_t(self.ws_bytes), c.stream()))
@@ -364,8 +431,8 @@ _POLL_LAG = 4
 _EAGER_ITERATIONS = 8
 
 
-def lloyd(X, init, max_iter: int = 300, tol: float = 1e-4, group=None, _host_relocation: bool = False):
-    """Batched ``KMeans(n_clusters=k, init=init, n_init=1, max_iter=max_iter, tol=tol).fit(X)``.
+def lloyd(X, init, max_iter: int = 300, tol: float = 1e-4, group=None, sample_weight=None, _host_relocation: bool = False):
+    """Batched ``KMeans(n_clusters=k, init=init, n_init=1, max_iter=max_iter, tol=tol).fit(X, sample_weight=sample_weight)``.
 
     X ``[n,d]`` or ``[B,n,d]`` (uint8 / float32 / float64; torch on the compute device, or numpy);
     init ``[k,d]`` or ``[B,k,d]``.  With ``group`` every rank passes its own rows (same B, d, k)
@@ -387,11 +454,19 @@ def lloyd(X, init, max_iter: int = 300, tol: float = 1e-4, group=None, _host_rel
     rank applies the same moves (``ofc_kmeans_relocate_merge``).  Should more clusters be empty at once than the
     list holds (16), the fit is redone with the host-merged relocation (``_relocate_across_ranks``).
 
+    ``sample_weight`` (``[n]``, or ``[B, n]`` for a batch; numpy or torch; see :func:`_check_sample_weight`): the weighted
+    fit of sklearn -- M-step sums of x w and float64 weight sums (a cluster is empty when its weight is 0), weighted
+    relocation and inertia.  The column mean, the tolerance and the stopping rule stay unweighted, as in sklearn.  The
+    weighted fit never takes the fused uint8 step.  ``None`` runs the unweighted kernels.  Not with ``group``.
+
     Returns ``(labels int32, centres float64, inertia float64, n_iter int64)`` as torch
     tensors on X's device, squeezed when X was ``[n,d]``.
     """
+    if sample_weight is not None and group is not None:
+        raise NotImplementedError("sample_weight with a row-sharded fit (group)")
     Xb, single = _as_batch(X, _target_device(X))
     ctx = _Ctx(Xb.device)
+    w_host = _check_sample_weight(sample_weight, int(Xb.shape[1]), Xb.dtype, rows=int(Xb.shape[0]))
     init_arg = init
     init = torch.as_tensor(np.asarray(init) if not isinstance(init, torch.Tensor) else init)
     init = init.to(device=Xb.device, dtype=torch.float64)
@@ -400,7 +475,7 @@ def lloyd(X, init, max_iter: int = 300, tol: float = 1e-4, group=None, _host_rel
         if group is not None:
             raise NotImplementedError("several starts (init [R, k, d]) of a row-sharded fit")
         if _tc_wanted(Xb, int(init.shape[1])):
-            runs = [lloyd(Xb[0], init[r], max_iter, tol) for r in range(int(init.shape[0]))]
+            runs = [lloyd(Xb[0], init[r], max_iter, tol, sample_weight=w_host) for r in range(int(init.shape[0]))]
             return tuple(torch.stack(t) for t in zip(*runs))
     elif init.dim() == 2:
         init = init.unsqueeze(0).expand(Xb.shape[0], -1, -1)
@@ -412,7 +487,13 @@ def lloyd(X, init, max_iter: int = 300, tol: float = 1e-4, group=None, _host_rel
     if init.dim() != 3 or init.shape[0] != B or init.shape[2] != d:
         raise ValueError(f"init shape {tuple(init.shape)} does not match X {tuple(Xb.shape)}")
     use_tc = not shared and _tc_wanted(Xb, k)
-    st = LloydState(ctx, Xb, k, ws_k=1 if use_tc else None, shared_batch=B if shared else None)
+    weighted = w_host is not None
+    w_dev = None
+    if weighted:                     # float64 on the device: [n] read by every start of a shared batch, else [B, n]
+        w_dev = torch.from_numpy(w_host.astype(np.float64)).to(Xb.device)
+        if not shared:
+            w_dev = w_dev.view(-1, n).expand(B, n).contiguous()
+    st = LloydState(ctx, Xb, k, ws_k=1 if use_tc else None, shared_batch=B if shared else None, weights=w_dev)
     dev = Xb.device
     row_offset, n_total = 0, n
     if group is not None:
@@ -438,7 +519,9 @@ def lloyd(X, init, max_iter: int = 300, tol: float = 1e-4, group=None, _host_rel
         centres = centres.to(torch.float32).to(torch.float64).contiguous()
     # dense float32 corner (d > 32): E/M steps on the tensor-core path, same labels as the float32 kernels
     tc = TensorCoreSteps(st, mean[0].contiguous()) if use_tc else None
-    fused = tc is None and is_u8 and st.step_supported()
+    # the fused step's exact integer accumulators do not hold real-valued x w: a weighted uint8 fit takes two kernels
+    fused = tc is None and is_u8 and not weighted and st.step_supported()
+    counts_or_w = st.wsum if weighted else st.counts            # what the relocation and the centre update run on
 
     active = st.active
     n_active = torch.zeros(max(max_iter, 1), dtype=torch.int32, device=dev)        # problems still running after iteration i
@@ -490,7 +573,10 @@ def lloyd(X, init, max_iter: int = 300, tol: float = 1e-4, group=None, _host_rel
         else:
             st.assign(mean, centres, lab, prev=lab_old, n_changed=changed_w, active=active)
             # uint8: raw (exact integer) sums; floats: sums of the centred rows like sklearn
-            st.sums_(None if is_u8 else mean, lab, sums_w, counts_w, k, active=active)
+            if weighted:
+                st.sums_weighted(None if is_u8 else mean, lab, sums_w, st.wsum, active=active)
+            else:
+                st.sums_(None if is_u8 else mean, lab, sums_w, counts_w, k, active=active)
         if group is not None:
             if B > 1:
                 # stopped problems contribute nothing (their buffers hold already-reduced values)
@@ -524,8 +610,8 @@ def lloyd(X, init, max_iter: int = 300, tol: float = 1e-4, group=None, _host_rel
                 ctx.check(ctx.lib.ofc_kmeans_relocate_merge(B, d, k, world, n_far, _ptr(allpay), _ptr(st.sums), _ptr(st.counts),
                                                             _ptr(overflow), _ptr(active), ctx.stream()))
         else:
-            st.relocate(mean, lab, centres, st.sums, st.counts, is_u8, active=active)
-        st.update_(st.sums, st.counts, mean if is_u8 else None, 0 if is_u8 else 1, 1 if is_f32 else 0, centres, st.n_changed,
+            st.relocate(mean, lab, centres, st.sums, counts_or_w, is_u8, active=active)
+        st.update_(st.sums, counts_or_w, mean if is_u8 else None, 0 if is_u8 else 1, 1 if is_f32 else 0, centres, st.n_changed,
                    tol_, 0, n_active, lab, lab_old, it_counter=it_counter)
 
     def stopped(upto):
@@ -604,7 +690,7 @@ def lloyd(X, init, max_iter: int = 300, tol: float = 1e-4, group=None, _host_rel
         if int(overflow.item()):
             # more clusters empty at once than the device-side candidate list holds: redo the fit with the host-merged
             # relocation (every rank takes this branch: the all-reduced counts are the same everywhere)
-            return lloyd(X, init_arg, max_iter, tol, group, _host_relocation=True)
+            return lloyd(X, init_arg, max_iter, tol, group, sample_weight, _host_relocation=True)
     final = st.labels[0]
     # strict stops already hold the labels of the final centres; the rest get one more E-step
     # (_kmeans.py:745-755).  Re-running it for everyone is idempotent for the strict ones and
@@ -675,13 +761,15 @@ def predict(X, centres):
     return st.labels[0][0] if single else st.labels[0]
 
 
-def kmeans_plusplus(X, n_clusters: int, random_state=None):
+def kmeans_plusplus(X, n_clusters: int, random_state=None, sample_weight=None):
     """k-means++ seeding with sklearn's procedure and RNG call sequence
     (sklearn/cluster/_kmeans.py:181-268): first centre by ``random_state.choice``, then
     ``2 + int(log(k))`` candidates per step sampled in proportion to the squared distance to
     the closest chosen centre, keeping the candidate that lowers the potential most.
     Distances come from the E-step kernel (one candidate = a one-centre problem).
-    X ``[n, d]``; returns ``(centres float64 [k,d] tensor, indices)``.
+    X ``[n, d]``; returns ``(centres float64 [k,d] tensor, indices)``.  ``sample_weight`` ``[n]``: the first centre is
+    drawn with ``p = w / w.sum()``, the potentials are ``closest @ w`` and the candidates are sampled from
+    ``cumsum(w * closest)``, as sklearn does (a row of weight 0 is never a seed).
 
     The reference leaves ``random_state`` unset (KmeanGrids.py:300), so this seeding is not
     pinned by any reference output (SURVEY.md Q9)."""
@@ -692,27 +780,29 @@ def kmeans_plusplus(X, n_clusters: int, random_state=None):
     rs = random_state if isinstance(random_state, np.random.RandomState) else np.random.RandomState(random_state)
     n, d = int(Xb.shape[1]), int(Xb.shape[2])
     k = int(n_clusters)
+    w_host = _check_sample_weight(sample_weight, n, Xb.dtype)
+    w = None if w_host is None else torch.from_numpy(w_host.astype(np.float64)).to(Xb.device)
     st = LloydState(ctx, Xb, 1)
     trials = 2 + int(math.log(k))
     Xf = Xb[0]
     centres = torch.empty((k, d), dtype=torch.float64, device=Xb.device)
     indices = np.full(k, -1, dtype=np.int64)
-    cid = int(rs.choice(n, p=np.full(n, 1.0 / n)))
+    cid = int(rs.choice(n, p=np.full(n, 1.0 / n) if w is None else w_host / w_host.sum()))
     centres[0] = Xf[cid].to(torch.float64)
     indices[0] = cid
     closest = torch.empty((1, n), dtype=torch.float64, device=Xb.device)
     cand = torch.empty((1, n), dtype=torch.float64, device=Xb.device)
     st.assign(None, centres[0:1].unsqueeze(0).contiguous(), st.labels[0], min_dist=closest)
-    pot = float(closest.sum().item())
+    pot = float((closest.sum() if w is None else (closest * w).sum()).item())
     for c in range(1, k):
         rand_vals = rs.uniform(size=trials) * pot
-        cum = torch.cumsum(closest[0], dim=0)
+        cum = torch.cumsum(closest[0] if w is None else closest[0] * w, dim=0)
         ids = torch.searchsorted(cum, torch.from_numpy(rand_vals).to(Xb.device)).clamp_(max=n - 1).cpu().numpy()
         best = None
         for cidx in ids:
             st.assign(None, Xf[int(cidx)].to(torch.float64).view(1, 1, d).contiguous(), st.labels[0], min_dist=cand)
             dmin = torch.minimum(closest, cand)
-            p = float(dmin.sum().item())
+            p = float((dmin.sum() if w is None else (dmin * w).sum()).item())
             if best is None or p < best[0]:
                 best = (p, int(cidx), dmin)
         pot, cid, closest = best[0], best[1], best[2].contiguous()
@@ -721,7 +811,7 @@ def kmeans_plusplus(X, n_clusters: int, random_state=None):
     return centres, indices
 
 
-def kmeans_plusplus_starts(X, n_clusters: int, n_starts: int, random_state):
+def kmeans_plusplus_starts(X, n_clusters: int, n_starts: int, random_state, sample_weight=None):
     """The k-means++ seeds of ``n_starts`` starts of one fit, the same as ``n_starts`` calls of
     :func:`kmeans_plusplus` one after another on one ``RandomState`` -- computed in lockstep on the device, without
     a host round trip until the seeds are done.  X ``[n, d]`` on the compute device; returns ``(centres float64
@@ -731,7 +821,8 @@ def kmeans_plusplus_starts(X, n_clusters: int, n_starts: int, random_state):
     per start: how many numbers they draw does not depend on the data).  Each of the k - 1 steps then computes the
     distances of all R*T candidates in ONE E-step call (a shared-row batch of one-centre problems), and every start
     runs the torch operations of :func:`kmeans_plusplus` on tensors of the same shapes, each in an allocation of its
-    own (a reduction may order its sum by the data's alignment), so a start's seeds do not depend on R."""
+    own (a reduction may order its sum by the data's alignment), so a start's seeds do not depend on R.
+    ``sample_weight`` ``[n]``: the weighted seeding of :func:`kmeans_plusplus`, with the same operations."""
     Xb, single = _as_batch(X, _target_device(X))
     if not single:
         raise ValueError("kmeans_plusplus_starts takes one problem [n, d]")
@@ -741,10 +832,12 @@ def kmeans_plusplus_starts(X, n_clusters: int, n_starts: int, random_state):
     k, R = int(n_clusters), int(n_starts)
     trials = 2 + int(math.log(k))
     dev = Xb.device
+    w_host = _check_sample_weight(sample_weight, n, Xb.dtype)
+    w = None if w_host is None else torch.from_numpy(w_host.astype(np.float64)).to(dev)
     first = np.empty(R, np.int64)
     uni = np.empty((R, max(k - 1, 1), trials))
     for r in range(R):
-        first[r] = rs.choice(n, p=np.full(n, 1.0 / n))
+        first[r] = rs.choice(n, p=np.full(n, 1.0 / n) if w is None else w_host / w_host.sum())
         for c in range(1, k):
             uni[r, c - 1] = rs.uniform(size=trials)
     uni = torch.from_numpy(uni).to(dev)
@@ -755,7 +848,7 @@ def kmeans_plusplus_starts(X, n_clusters: int, n_starts: int, random_state):
     dist0 = torch.empty((R, n), dtype=torch.float64, device=dev)
     st.assign(None, Xf[idx[:, 0]].to(torch.float64).view(R, 1, d).contiguous(), st.labels[0], min_dist=dist0)
     closest = [dist0[r:r + 1].clone() for r in range(R)]
-    pot = [cl.sum() for cl in closest]
+    pot = [cl.sum() if w is None else (cl * w).sum() for cl in closest]
     if k > 1:
         cst = LloydState(ctx, Xb, 1, shared_batch=R * trials)
         cand = torch.empty((R * trials, n), dtype=torch.float64, device=dev)
@@ -763,13 +856,13 @@ def kmeans_plusplus_starts(X, n_clusters: int, n_starts: int, random_state):
         ids = []
         for r in range(R):
             rand_vals = uni[r, c - 1] * pot[r]
-            cum = torch.cumsum(closest[r][0], dim=0)
+            cum = torch.cumsum(closest[r][0] if w is None else closest[r][0] * w, dim=0)
             ids.append(torch.searchsorted(cum, rand_vals).clamp_(max=n - 1))
         ids = torch.cat(ids)
         cst.assign(None, Xf[ids].to(torch.float64).view(R * trials, 1, d).contiguous(), cst.labels[0], min_dist=cand)
         for r in range(R):
             dmin = [torch.minimum(closest[r], cand[r * trials + t:r * trials + t + 1]) for t in range(trials)]
-            p = torch.stack([dm.sum() for dm in dmin])
+            p = torch.stack([dm.sum() if w is None else (dm * w).sum() for dm in dmin])
             best = torch.argmin(p).view(1)                     # the first of the smallest, as the strict `<` of the loop
             pot[r] = p[best][0]
             closest[r] = torch.stack(dmin).index_select(0, best)[0]
@@ -817,14 +910,16 @@ def _resolve_n_init(n_init, init) -> int:
     return r
 
 
-def random_starts(X, n_clusters: int, n_starts: int, random_state):
+def random_starts(X, n_clusters: int, n_starts: int, random_state, sample_weight=None):
     """``init="random"`` (_kmeans.py:1030-1036): per start, ``choice(n, size=k, replace=False, p=w / w.sum())`` with
-    ``w`` = ones in the data's working dtype (float32 for float32 rows, else float64).  Returns (centres float64
-    [R, k, d] tensor on X's device, indices int64 [R, k])."""
+    ``w`` = ``sample_weight`` (ones when None) in the data's working dtype (float32 for float32 rows, else float64).
+    Returns (centres float64 [R, k, d] tensor on X's device, indices int64 [R, k])."""
     Xb, _ = _as_batch(X, _target_device(X))
     rs = random_state if isinstance(random_state, np.random.RandomState) else np.random.RandomState(random_state)
     n = int(Xb.shape[1])
-    w = np.ones(n, dtype=np.float32 if Xb.dtype == torch.float32 else np.float64)
+    w = _check_sample_weight(sample_weight, n, Xb.dtype)
+    if w is None:
+        w = np.ones(n, dtype=np.float32 if Xb.dtype == torch.float32 else np.float64)
     idx = np.stack([rs.choice(n, size=int(n_clusters), replace=False, p=w / w.sum()) for _ in range(int(n_starts))])
     return Xb[0][torch.from_numpy(idx).to(Xb.device)].to(torch.float64), idx.astype(np.int64)
 
@@ -839,18 +934,22 @@ class KMeans:
     The starts draw their seeds one after another from one ``RandomState`` (so ``random_state=int`` reproduces
     sklearn), run as one batched Lloyd fit over a single copy of the rows, and the result is the start sklearn
     keeps: the first one, replaced by a later one only if that has a strictly lower inertia and a different
-    clustering."""
+    clustering.
+
+    ``fit(X, sample_weight=w)`` is sklearn's weighted fit (seeding, M-step, relocation and inertia weighted; see
+    :func:`_check_sample_weight` for the accepted weights); :meth:`score` is its negative weighted inertia."""
 
     def __init__(self, n_clusters=8, *, init="k-means++", n_init="auto", max_iter=300, tol=1e-4, random_state=None):
         self.n_clusters, self.init, self.n_init = int(n_clusters), init, n_init
         self.max_iter, self.tol, self.random_state = int(max_iter), float(tol), random_state
 
-    def fit(self, X, y=None):
+    def fit(self, X, y=None, sample_weight=None):
         Xa = X if isinstance(X, torch.Tensor) else np.asarray(X)
         if Xa.ndim != 2:
             raise ValueError("Expected 2D array")
         if Xa.shape[0] < self.n_clusters:
             raise ValueError(f"n_samples={Xa.shape[0]} should be >= n_clusters={self.n_clusters}.")
+        sw = _check_sample_weight(sample_weight, int(Xa.shape[0]), Xa.dtype)
         if isinstance(self.init, str) and self.init not in ("k-means++", "random"):
             raise ValueError(f"init={self.init!r}: 'k-means++', 'random' or an array")
         n_init = _resolve_n_init(self.n_init, self.init)
@@ -860,10 +959,10 @@ class KMeans:
             Xd, _ = _as_batch(Xa, _target_device(Xa))
             Xd = Xd[0]
             if self.init == "random":
-                init, _ = random_starts(Xd, self.n_clusters, n_init, rs)
+                init, _ = random_starts(Xd, self.n_clusters, n_init, rs, sw)
             else:
-                init, _ = kmeans_plusplus_starts(Xd, self.n_clusters, n_init, rs)
-            labels, centres, inertia, n_iter = lloyd(Xd, init, self.max_iter, self.tol)
+                init, _ = kmeans_plusplus_starts(Xd, self.n_clusters, n_init, rs, sw)
+            labels, centres, inertia, n_iter = lloyd(Xd, init, self.max_iter, self.tol, sample_weight=sw)
             b = best_start(labels, inertia, self.n_clusters)
             labels, centres, inertia, n_iter = labels[b], centres[b], inertia[b], n_iter[b]
         else:
@@ -871,10 +970,10 @@ class KMeans:
                 if self.n_clusters == 1:
                     init = (Xa[:1].to(torch.float64) if isinstance(Xa, torch.Tensor) else Xa[:1].astype(np.float64))
                 else:
-                    init, _ = kmeans_plusplus(Xa, self.n_clusters, self.random_state)
+                    init, _ = kmeans_plusplus(Xa, self.n_clusters, self.random_state, sw)
             else:
                 init = self.init
-            labels, centres, inertia, n_iter = lloyd(Xa, init, self.max_iter, self.tol)
+            labels, centres, inertia, n_iter = lloyd(Xa, init, self.max_iter, self.tol, sample_weight=sw)
         self._centres_t = centres
         self.cluster_centers_ = centres.cpu().numpy()
         if not isinstance(X, torch.Tensor) and np.asarray(X).dtype == np.float32:
@@ -887,12 +986,26 @@ class KMeans:
     def predict(self, X):
         return predict(X, self._centres_t).cpu().numpy()
 
-    def fit_predict(self, X, y=None):
-        return self.fit(X).labels_
+    def fit_predict(self, X, y=None, sample_weight=None):
+        return self.fit(X, sample_weight=sample_weight).labels_
+
+    def score(self, X, y=None, sample_weight=None):
+        """sklearn's ``KMeans.score`` (_kmeans.py:1159-1187): minus the (weighted) inertia of X against the fitted centres,
+        on the un-centred rows as :meth:`predict` assigns them."""
+        Xb, single = _as_batch(X, _target_device(X))
+        if not single:
+            raise ValueError("Expected 2D array")
+        n = int(Xb.shape[1])
+        w = _check_sample_weight(sample_weight, n, Xb.dtype)
+        w = None if w is None else torch.from_numpy(w.astype(np.float64)).to(Xb.device)
+        c = self._centres_t.to(device=Xb.device, dtype=torch.float64).unsqueeze(0).contiguous()
+        st = LloydState(_Ctx(Xb.device), Xb, int(c.shape[1]), weights=w)
+        st.assign(None, c, st.labels[0], inertia=st.inertia)
+        return -float(st.inertia[0].item())
 
 
-def kmeans_fit(X, init, max_iter: int = 300, tol: float = 1e-4):
+def kmeans_fit(X, init, max_iter: int = 300, tol: float = 1e-4, sample_weight=None):
     """SURVEY.md §8(b) parity entry point: numpy in / numpy out
-    ``(labels int32[N], centers[k,D], inertia, n_iter)``."""
-    labels, centres, inertia, n_iter = lloyd(X, init, max_iter, tol)
+    ``(labels int32[N], centers[k,D], inertia, n_iter)``; ``sample_weight`` as in :func:`lloyd`."""
+    labels, centres, inertia, n_iter = lloyd(X, init, max_iter, tol, sample_weight=sample_weight)
     return labels.cpu().numpy(), centres.cpu().numpy(), float(inertia.item()), int(n_iter.item())
