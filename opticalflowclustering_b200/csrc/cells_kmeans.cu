@@ -118,7 +118,7 @@ __global__ void __launch_bounds__(256, KP <= 8 ? 3 : 2) kmeans_cells_fast_kernel
     __shared__ double s_tol;
     __shared__ double s_val[8];
     __shared__ int s_idx[8];
-    __shared__ int s_pick, s_stop, s_changed, s_nmoves;
+    __shared__ int s_pick, s_stop, s_changed, s_nmoves, s_exact;
     __shared__ int s_cand[8];
     if (!p.closest_in_smem) closest = p.closest_ws + b * n;
 
@@ -181,6 +181,7 @@ __global__ void __launch_bounds__(256, KP <= 8 ? 3 : 2) kmeans_cells_fast_kernel
             vs += (double)num / ((double)n * (double)n);
         }
         s_tol = vs / (double)D * p.tol;
+        s_exact = 0;
     }
     __syncthreads();
 
@@ -355,17 +356,44 @@ __global__ void __launch_bounds__(256, KP <= 8 ? 3 : 2) kmeans_cells_fast_kernel
             }
         }
     };
-    auto prepare_centres = [&]() {          // c2 (float64), float32 filter copies; padding clusters can never win
+    // Centres outside the data range (an empty cluster holding the heaviest cluster's centred sum, or such initial
+    // centres).  One farther than 2^19 (squared) from [0,255]^4 is farther from every row than any centre inside
+    // [-1,256]^4 can be (4 * 256^2 = 2^18): it never wins, so the filter leaves it out like a padding cluster (the float64
+    // chain of the near-ties still sees it).  That needs one centre inside the range, which every centre computed by an
+    // update has -- the heaviest cluster's mean -- but initial centres need not.  Any other centre outside [-1,256]^4
+    // voids the filter's bound: from then on every row takes the float64 chain -- the same rows per thread, in the same
+    // order.  s_exact is set in prepare_centres and sticky (no reset between barriers); the unit of slack keeps means
+    // that round a few ulp past 0 or 255 on the filter, and with |c'_t| <= 256 the bound above still stays below E.  The
+    // test is uniform and outside the row loop, so the filtered loop is unchanged.
+    auto lloyd_e_step = [&](auto&& on_label) {
+        if (s_exact) {
+            for (int i = tid; i < n; i += 256) { const unsigned w = xs[i]; on_label(i, w, exact_label(w)); }
+        } else {
+            e_step(on_label);
+        }
+    };
+    // c2 (float64), float32 filter copies; padding clusters can never win.  `updated`: the centres come from an update
+    auto prepare_centres = [&](bool updated) {
         for (int j = tid; j < KP; j += 256) {
             if (j < k) {
-                double squ = 0.0;
+                double squ = 0.0, out = 0.0;
+                bool inside = true;
                 const double sq = norm_sq_numpy_f64(cc + j * D, D);
                 for (int t = 0; t < D; ++t) {
                     const double u = cc[j * D + t] + mean[t];
                     squ += u * u;
                     s_cf[j * 5 + t] = (float)u;
+                    inside = inside && u >= -1.0 && u <= 256.0;
+                    const double o = fmax(fmax(-u, u - 255.0), 0.0);
+                    out += o * o;
                 }
                 c2[j] = sq;
+                if (updated && out > 524288.0) {
+                    for (int t = 0; t < D; ++t) s_cf[j * 5 + t] = 0.f;
+                    s_cf[j * 5 + 4] = 3.0e38f;
+                    continue;
+                }
+                if (!inside) s_exact = 1;
                 // + 2^18: ||c'||^2 - 2 x.c' >= -||x||^2 >= -260100, so every filtered distance is a positive float below 2^21
                 s_cf[j * 5 + 4] = (float)(squ + 262144.0);
             } else {
@@ -380,7 +408,7 @@ __global__ void __launch_bounds__(256, KP <= 8 ? 3 : 2) kmeans_cells_fast_kernel
     int iters = 0;
     bool strict = false;
     for (int it = 0; it < p.max_iter; ++it) {
-        prepare_centres();
+        prepare_centres(it > 0);
         if (tid == 0) { s_changed = 0; s_nmoves = 0; }
         // M-step of this iteration: the first E-step labels every row, so its sums are built from scratch in registers
         // (16-bit fields, warp reductions -- no contended atomics); every later iteration updates them from the rows
@@ -395,7 +423,7 @@ __global__ void __launch_bounds__(256, KP <= 8 ? 3 : 2) kmeans_cells_fast_kernel
         __syncthreads();
         int changed = 0;
         if (full) {
-            e_step([&](int i, unsigned, int label) {
+            lloyd_e_step([&](int i, unsigned, int label) {
                 if (lab[i] != label) { ++changed; lab[i] = (unsigned char)label; }
             });
             unsigned a0[KP], a1[KP], ac[KP];
@@ -427,7 +455,7 @@ __global__ void __launch_bounds__(256, KP <= 8 ? 3 : 2) kmeans_cells_fast_kernel
                 }
             }
         } else {
-            e_step([&](int i, unsigned w, int label) {
+            lloyd_e_step([&](int i, unsigned w, int label) {
                 const int old = lab[i];
                 if (old != label) {
                     ++changed;
@@ -449,12 +477,13 @@ __global__ void __launch_bounds__(256, KP <= 8 ? 3 : 2) kmeans_cells_fast_kernel
         __syncthreads();
         // empty clusters take the farthest points (squared distance to the old centre of their label); the labels
         // stay as they are (_k_means_common.pyx:167-211), so the moves are undone on the running sums below.
-        // The member counts are final behind the barrier above: every thread tests them itself (no flag, no barrier)
-        int any_empty = 0;
-        for (int j = 0; j < k; ++j) any_empty |= s_cnt[j] == 0;
-        if (any_empty) {
+        // The member counts are final behind the barrier above: every thread takes the set of empty clusters from them
+        // itself (no flag, no barrier), once -- a cluster that a move empties stays empty in this iteration
+        unsigned empty = 0u;
+        for (int j = 0; j < k; ++j) empty |= (s_cnt[j] == 0 ? 1u : 0u) << j;
+        if (empty) {
             for (int e = 0; e < k; ++e) {
-                if (s_cnt[e] != 0) continue;
+                if (!((empty >> e) & 1u)) continue;
                 const int n_taken = s_nmoves;
                 double bv = -1.0;
                 int bi = -1;
@@ -511,11 +540,12 @@ __global__ void __launch_bounds__(256, KP <= 8 ? 3 : 2) kmeans_cells_fast_kernel
             for (int j = 1; j < k; ++j) if (s_cnt[j] > s_cnt[heavy]) heavy = j;
             for (int j = lane; j < k; j += 32) {
                 const int srcj = s_cnt[j] > 0 ? j : heavy;
+                const bool as_sum = srcj != j && j < srcj;     // the heaviest cluster's centred sum (kmeans_cells_kernel)
                 const double wgt = (double)s_cnt[srcj];
                 double ss = 0.0;
                 for (int t = 0; t < D; ++t) {
-                    double v = (double)s_sum[srcj * D + t] / wgt;
-                    v -= mean[t];
+                    const double sv = (double)s_sum[srcj * D + t];
+                    const double v = as_sum ? fma(-wgt, mean[t], sv) : sv / wgt - mean[t];
                     const double df = v - cc[j * D + t];
                     ss = fma(df, df, ss);
                     cnew[j * D + t] = v;
@@ -559,11 +589,11 @@ __global__ void __launch_bounds__(256, KP <= 8 ? 3 : 2) kmeans_cells_fast_kernel
     const bool want_inertia = p.inertia != nullptr;
     const bool closing = !strict || want_inertia || labels_out != nullptr;
     if (closing) {
-        prepare_centres();
+        prepare_centres(iters > 0);
         for (int j = tid; j < KP; j += 256) s_cnt[j] = 0;
     }
     __syncthreads();
-    if (closing) e_step([&](int i, unsigned w, int label) {
+    if (closing) lloyd_e_step([&](int i, unsigned w, int label) {
         lab[i] = (unsigned char)label;
         if (labels_out) labels_out[i] = label;
         atomicAdd(&s_cnt[label], 1);

@@ -467,10 +467,12 @@ __global__ void kmeans_fold_kernel(const double* partial, const C* cnt_partial, 
 }
 
 // ---------------------------------------------------------------------------
-// centres from (all-reduced) sums and counts; empty clusters copy the heaviest
-// cluster's new centre (_k_means_common.pyx:274-295); shift_tot = sum_j ||new-old||^2
-// taken as (sqrt(.))^2 like sklearn's center_shift (:298-311, _kmeans.py:733).
-// One CTA per problem.
+// centres from (all-reduced) sums and counts; an empty cluster copies the heaviest
+// cluster's row as sklearn's in-place _average_centers (_k_means_common.pyx:274-295)
+// finds it: not yet divided -- the heaviest cluster's centred SUM -- when the empty
+// cluster's index is the lower one, its new centre otherwise (raw sums are centred
+// as S - W mean); shift_tot = sum_j ||new-old||^2 taken as (sqrt(.))^2 like
+// sklearn's center_shift (:298-311, _kmeans.py:733).  One CTA per problem.
 // ---------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) kmeans_centres_kernel(int d, int k, const double* sums, const long long* counts,
                                                              const double* mean_sub, int use_reciprocal,
@@ -495,13 +497,23 @@ __global__ void __launch_bounds__(256) kmeans_centres_kernel(int d, int k, const
         const double w = (double)Cn[src];
         const double alpha = 1.0 / w;
         double ss = 0.0;
-        for (int t = 0; t < d; ++t) {
-            double v = S[(int64_t)src * d + t];
-            v = use_reciprocal ? v * alpha : v / w;
-            if (mean_sub) v -= mean_sub[(int64_t)b * d + t];
-            const double df = v - C[(int64_t)j * d + t];
-            ss = fma(df, df, ss);
-            C[(int64_t)j * d + t] = v;
+        if (src != j && j < heavy) {                     // the heaviest cluster's centred sum
+            for (int t = 0; t < d; ++t) {
+                double v = S[(int64_t)src * d + t];
+                if (mean_sub) v = fma(-w, mean_sub[(int64_t)b * d + t], v);
+                const double df = v - C[(int64_t)j * d + t];
+                ss = fma(df, df, ss);
+                C[(int64_t)j * d + t] = v;
+            }
+        } else {
+            for (int t = 0; t < d; ++t) {
+                double v = S[(int64_t)src * d + t];
+                v = use_reciprocal ? v * alpha : v / w;
+                if (mean_sub) v -= mean_sub[(int64_t)b * d + t];
+                const double df = v - C[(int64_t)j * d + t];
+                ss = fma(df, df, ss);
+                C[(int64_t)j * d + t] = v;
+            }
         }
         const double s = sqrt(ss);
         sh[j] = s * s;
@@ -555,13 +567,23 @@ __global__ void __launch_bounds__(256) kmeans_update_kernel(int d, int k, const 
         const double w = (double)Cn[src];
         const double alpha = 1.0 / w;
         double ss = 0.0;
-        for (int t = 0; t < d; ++t) {
-            double v = S[(int64_t)src * d + t];
-            v = use_reciprocal ? v * alpha : v / w;
-            if (mean_sub) v -= mean_sub[(int64_t)b * d + t];
-            const double df = v - C[(int64_t)j * d + t];
-            ss = fma(df, df, ss);
-            C[(int64_t)j * d + t] = round_f32 ? (double)(float)v : v;
+        if (src != j && j < heavy) {                     // the heaviest cluster's centred sum (kmeans_centres_kernel)
+            for (int t = 0; t < d; ++t) {
+                double v = S[(int64_t)src * d + t];
+                if (mean_sub) v = fma(-w, mean_sub[(int64_t)b * d + t], v);
+                const double df = v - C[(int64_t)j * d + t];
+                ss = fma(df, df, ss);
+                C[(int64_t)j * d + t] = round_f32 ? (double)(float)v : v;
+            }
+        } else {
+            for (int t = 0; t < d; ++t) {
+                double v = S[(int64_t)src * d + t];
+                v = use_reciprocal ? v * alpha : v / w;
+                if (mean_sub) v -= mean_sub[(int64_t)b * d + t];
+                const double df = v - C[(int64_t)j * d + t];
+                ss = fma(df, df, ss);
+                C[(int64_t)j * d + t] = round_f32 ? (double)(float)v : v;
+            }
         }
         const double s = sqrt(ss);
         sh[j] = s * s;
@@ -637,19 +659,38 @@ __global__ void __launch_bounds__(256) kmeans_freeze_labels_kernel(int64_t n, co
         other[(int64_t)b * n + i] = cur[(int64_t)b * n + i];
 }
 
+// The empty clusters of a problem (count or weight sum 0) as a bit mask of (k + 31) / 32 words in shared memory, taken
+// by the CTA of NT threads before the first relocation move.  sklearn lists them once (_k_means_common.pyx:176): a
+// cluster that a move empties (its only member, or its only member of positive weight, was moved) stays empty for
+// this iteration, whatever its index.
+template <int NT, typename C>
+__device__ __forceinline__ void snapshot_empty(const C* counts, int k, unsigned* mask) {
+    for (int w = threadIdx.x; w < (k + 31) >> 5; w += NT) {
+        unsigned m = 0u;
+        for (int j = w * 32; j < min(k, w * 32 + 32); ++j) m |= (counts[j] == 0 ? 1u : 0u) << (j & 31);
+        mask[w] = m;
+    }
+    __syncthreads();
+}
+
+__device__ __forceinline__ bool in_mask(const unsigned* mask, int e) { return (mask[e >> 5] >> (e & 31)) & 1u; }
+
+static inline size_t empty_mask_bytes(int k) { return (size_t)((k + 31) / 32) * sizeof(unsigned); }
+
 // ---------------------------------------------------------------------------
-// empty-cluster relocation (_k_means_common.pyx:167-211): each empty cluster, in
-// index order, takes the farthest remaining point (squared distance to the OLD
-// centre of its label); labels are left untouched.  One CTA of 1024 threads per
-// problem; it returns at once when no cluster is empty, so the host launches it
-// unconditionally (no device->host round trip to decide).
+// empty-cluster relocation (_k_means_common.pyx:167-211): the clusters empty
+// before the first move, in index order, each take the farthest remaining point
+// (squared distance to the OLD centre of its label); labels are left untouched.
+// One CTA of 1024 threads per problem; it returns at once when no cluster is
+// empty, so the host launches it unconditionally (no device->host round trip).
 // ---------------------------------------------------------------------------
 template <typename T>
 __global__ void __launch_bounds__(1024) kmeans_relocate_kernel(const T* Xall, int64_t x_stride, int64_t n, int d, int k, const double* mean_all,
                                                                 const int32_t* labels_all, const double* centres_all,
                                                                 double* sums_all, long long* counts_all,
                                                                 int raw_sums, const unsigned char* active) {
-    OFC_DYN_SMEM(long long, s_taken);                  // [k] indices already given away
+    OFC_DYN_SMEM(long long, s_taken);                  // [k] indices already given away, then the empty-cluster mask
+    unsigned* s_empty = reinterpret_cast<unsigned*>(s_taken + k);
     const int b = blockIdx.x, tid = threadIdx.x;
     if (active && !active[b]) return;
     long long* counts = counts_all + (int64_t)b * k;
@@ -661,6 +702,7 @@ __global__ void __launch_bounds__(1024) kmeans_relocate_kernel(const T* Xall, in
     }
     __syncthreads();
     if (!s_any) return;
+    snapshot_empty<1024>(counts, k, s_empty);
     const T* X = Xall + (int64_t)b * x_stride;
     const int32_t* labels = labels_all + (int64_t)b * n;
     const double* cen = centres_all + (int64_t)b * k * d;
@@ -671,7 +713,7 @@ __global__ void __launch_bounds__(1024) kmeans_relocate_kernel(const T* Xall, in
     __shared__ long long s_pick;
     int n_taken = 0;
     for (int e = 0; e < k; ++e) {
-        if (counts[e] != 0) continue;                  // uniform: written only behind a barrier
+        if (!in_mask(s_empty, e)) continue;
         double bv = -1.0;
         long long bi = -1;
         for (int64_t i = tid; i < n; i += 1024) {
@@ -799,6 +841,7 @@ __global__ void __launch_bounds__(1024) kmeans_relocate_apply_kernel(const T* Xa
                                                                       C* counts_all, int raw_sums, const unsigned char* active,
                                                                       const double* weights_all, int64_t w_stride) {
     constexpr bool WT = std::is_same<C, double>::value;
+    OFC_DYN_SMEM(unsigned, s_empty);                   // [(k + 31) / 32] the empty-cluster mask
     const int b = blockIdx.x, tid = threadIdx.x;
     if (active && !active[b]) return;
     C* counts = counts_all + (int64_t)b * k;
@@ -814,6 +857,7 @@ __global__ void __launch_bounds__(1024) kmeans_relocate_apply_kernel(const T* Xa
     }
     __syncthreads();
     if (!s_any) return;
+    snapshot_empty<1024>(counts, k, s_empty);
     const T* X = Xall + (int64_t)b * x_stride;
     const int32_t* labels = labels_all + (int64_t)b * n;
     const double* mean = mean_all ? mean_all + (int64_t)b * d : nullptr;
@@ -821,7 +865,7 @@ __global__ void __launch_bounds__(1024) kmeans_relocate_apply_kernel(const T* Xa
     double* scratch = scratch_all + (int64_t)b * n;
     int n_taken = 0;
     for (int e = 0; e < k; ++e) {
-        if (counts[e] != 0) continue;                  // uniform: written only behind a barrier
+        if (!in_mask(s_empty, e)) continue;
         double v;
         long long fi;
         block_argmax_1024(scratch, n, s_val, s_idx, v, fi);
@@ -943,7 +987,8 @@ __global__ void __launch_bounds__(256) kmeans_relocate_merge_kernel(int batch, i
     const int rec = 3 + d, ncand = world * n_far;
     long long* counts = counts_all + (int64_t)b * k;
     double* sums = sums_all + (int64_t)b * k * d;
-    OFC_DYN_SMEM(unsigned char, s_used);                  // [ncand]
+    OFC_DYN_SMEM(unsigned char, s_used);                  // [ncand], then the empty-cluster mask (4-byte aligned)
+    unsigned* s_mask = reinterpret_cast<unsigned*>(s_used + ((ncand + 3) & ~3));
     __shared__ int s_pick, s_empty, s_state;
     if (tid == 0) {
         int ne = 0;
@@ -954,6 +999,7 @@ __global__ void __launch_bounds__(256) kmeans_relocate_merge_kernel(int batch, i
     for (int c = tid; c < ncand; c += 256) s_used[c] = 0;
     __syncthreads();
     if (s_state != 1) return;
+    snapshot_empty<256>(counts, k, s_mask);
     auto cand = [&](int c) -> const double* {
         const int r = c / n_far, e = c - r * n_far;
         return allpay + (((int64_t)r * batch + b) * n_far + e) * rec;
@@ -962,7 +1008,7 @@ __global__ void __launch_bounds__(256) kmeans_relocate_merge_kernel(int batch, i
     for (int round = 0;; ++round) {
         if (tid == 0) {
             int e = e_next;
-            while (e < k && counts[e] != 0) ++e;
+            while (e < k && !in_mask(s_mask, e)) ++e;
             s_empty = e;
             int best = -1;
             if (e < k) {
@@ -1093,7 +1139,8 @@ __global__ void __launch_bounds__(256) kmeans_cells_kernel(KmCellsParams p) {
     __shared__ unsigned long long s_stat[16];     // sum x, sum x^2 per dim (d <= 8)
     __shared__ double s_tol, s_val[8];
     __shared__ long long s_idx[8], s_pick;
-    __shared__ int s_any, s_heavy, s_stop, s_changed;     // one word per decision: no reuse between barriers
+    __shared__ int s_heavy, s_stop, s_changed;            // one word per decision: no reuse between barriers
+    __shared__ unsigned long long s_empty;                // the clusters empty before the first relocation move (k <= 64)
     const unsigned char* X = p.X + (int64_t)b * n * d;
     int32_t* labels = p.labels + (int64_t)b * n;
 
@@ -1267,18 +1314,18 @@ __global__ void __launch_bounds__(256) kmeans_cells_kernel(KmCellsParams p) {
         }
         if (changed) atomicAdd(&s_changed, changed);
         __syncthreads();
-        // empty clusters take the farthest points (distance to the old centre of their label)
+        // the clusters empty now, in index order, take the farthest points (distance to the old centre of their label)
         if (tid == 0) {
-            int any = 0;
-            for (int j = 0; j < k; ++j) any |= s_cnt[j] == 0;
-            s_any = any;
+            unsigned long long empty = 0ull;
+            for (int j = 0; j < k; ++j) empty |= (unsigned long long)(s_cnt[j] == 0) << j;
+            s_empty = empty;
         }
         __syncthreads();
-        if (s_any) {
+        if (s_empty) {
             long long* taken = reinterpret_cast<long long*>(cnew);     // scratch until the centre update
             int n_taken = 0;
             for (int e = 0; e < k; ++e) {
-                if (s_cnt[e] != 0) continue;
+                if (!((s_empty >> e) & 1ull)) continue;
                 double bv = -1.0;
                 long long bi = -1;
                 for (int i = tid; i < n; i += 256) {
@@ -1334,11 +1381,12 @@ __global__ void __launch_bounds__(256) kmeans_cells_kernel(KmCellsParams p) {
         __syncthreads();
         for (int j = tid; j < k; j += 256) {
             const int srcj = s_cnt[j] > 0 ? j : s_heavy;
+            const bool as_sum = srcj != j && j < srcj;         // the heaviest cluster's centred sum (kmeans_centres_kernel)
             const double wgt = (double)s_cnt[srcj];
             double ss = 0.0;
             for (int t = 0; t < d; ++t) {
-                double v = (double)s_sum[srcj * d + t] / wgt;
-                v -= mean[t];
+                const double sv = (double)s_sum[srcj * d + t];
+                const double v = as_sum ? fma(-wgt, mean[t], sv) : sv / wgt - mean[t];
                 const double df = v - cc[j * d + t];
                 ss = fma(df, df, ss);
                 cnew[j * d + t] = v;
@@ -1730,21 +1778,22 @@ int launch_kmeans_relocate(const void* X, int64_t x_stride, int dtype, int batch
         else if (dtype == DT_F32) rc = launch_rowdist<float>(X, x_stride, batch, n, d, k, mean, labels, centres_old, counts, scratch, 0, active, stream);
         else rc = launch_rowdist<double>(X, x_stride, batch, n, d, k, mean, labels, centres_old, counts, scratch, 0, active, stream);
         if (rc != OFC_OK) return rc;
+        const size_t smem = empty_mask_bytes(k);
         if (dtype == DT_U8)
-            OFC_LAUNCH((kmeans_relocate_apply_kernel<unsigned char, long long>), dim3(batch), dim3(1024), 0, stream, (const unsigned char*)X,
+            OFC_LAUNCH((kmeans_relocate_apply_kernel<unsigned char, long long>), dim3(batch), dim3(1024), smem, stream, (const unsigned char*)X,
                        x_stride, n, d, k, mean, labels, scratch, sums, counts, raw_sums, active, nullptr, 0);
         else if (dtype == DT_F32)
-            OFC_LAUNCH((kmeans_relocate_apply_kernel<float, long long>), dim3(batch), dim3(1024), 0, stream, (const float*)X, x_stride, n, d, k,
+            OFC_LAUNCH((kmeans_relocate_apply_kernel<float, long long>), dim3(batch), dim3(1024), smem, stream, (const float*)X, x_stride, n, d, k,
                        mean, labels, scratch, sums, counts, raw_sums, active, nullptr, 0);
         else
-            OFC_LAUNCH((kmeans_relocate_apply_kernel<double, long long>), dim3(batch), dim3(1024), 0, stream, (const double*)X, x_stride, n, d,
+            OFC_LAUNCH((kmeans_relocate_apply_kernel<double, long long>), dim3(batch), dim3(1024), smem, stream, (const double*)X, x_stride, n, d,
                        k, mean, labels, scratch, sums, counts, raw_sums, active, nullptr, 0);
         OFC_CHECK_LAUNCH("kmeans_relocate_apply");
         return OFC_OK;
     }
-    const size_t smem = (size_t)k * sizeof(long long);
-    // the list of rows already given away is k words of shared memory: opt in past 48 KB (k <= 25 600)
-    if (smem > 200 * 1024) { set_error("k=%d too large for the relocation kernel (k <= 25600)", k); return OFC_ERR_UNSUPPORTED; }
+    // the list of rows already given away (k words) and the empty-cluster mask in shared memory: opt in past 48 KB
+    if (k > 25600) { set_error("k=%d too large for the relocation kernel (k <= 25600)", k); return OFC_ERR_UNSUPPORTED; }
+    const size_t smem = (size_t)k * sizeof(long long) + empty_mask_bytes(k);
     OFC_SMEM_OPTIN(kmeans_relocate_kernel<unsigned char>, smem);
     OFC_SMEM_OPTIN(kmeans_relocate_kernel<float>, smem);
     OFC_SMEM_OPTIN(kmeans_relocate_kernel<double>, smem);
@@ -1767,8 +1816,8 @@ static int relocate_weighted(const void* X, int64_t x_stride, int batch, int64_t
                              int raw_sums, const unsigned char* active, double* scratch, void* stream) {
     int rc = launch_rowdist<T, double>(X, x_stride, batch, n, d, k, mean, labels, centres_old, weight_sums, scratch, 0, active, stream);
     if (rc != OFC_OK) return rc;
-    OFC_LAUNCH((kmeans_relocate_apply_kernel<T, double>), dim3(batch), dim3(1024), 0, stream, (const T*)X, x_stride, n, d, k, mean, labels,
-               scratch, sums, weight_sums, raw_sums, active, weights, w_stride);
+    OFC_LAUNCH((kmeans_relocate_apply_kernel<T, double>), dim3(batch), dim3(1024), empty_mask_bytes(k), stream, (const T*)X, x_stride, n, d,
+               k, mean, labels, scratch, sums, weight_sums, raw_sums, active, weights, w_stride);
     OFC_CHECK_LAUNCH("kmeans_relocate_apply");
     return OFC_OK;
 }
@@ -1819,7 +1868,7 @@ int launch_kmeans_relocate_merge(int batch, int d, int k, int world, int n_far, 
                                  int* overflow, const unsigned char* active, void* stream) {
     if (batch <= 0) return OFC_OK;
     ProfScope prof(PK_KMEANS, stream);
-    const size_t smem = (size_t)world * n_far;
+    const size_t smem = (((size_t)world * n_far + 3) & ~(size_t)3) + empty_mask_bytes(k);
     OFC_SMEM_OPTIN(kmeans_relocate_merge_kernel, smem);
     OFC_LAUNCH(kmeans_relocate_merge_kernel, dim3(batch), dim3(256), smem, stream, batch, d, k, world, n_far, allpay, sums, counts, overflow,
                active);

@@ -41,46 +41,59 @@ def _e_step(X, centers):
     return labels
 
 
-def _m_step(X, labels, centers_old):
+def _m_step(X, labels, centers_old, sw=None):
+    """sklearn's M-step on the centred rows: weighted sums and weight sums, _relocate_empty_clusters_dense, then
+    _average_centers.  ``sw`` None = unit weights (the same bits: x * 1 == x)."""
     k, D = centers_old.shape
-    w = np.bincount(labels, minlength=k).astype(X.dtype)
+    if sw is None:
+        w = np.bincount(labels, minlength=k).astype(X.dtype)
+    else:
+        w = np.bincount(labels, weights=sw, minlength=k).astype(X.dtype)
     sums = np.zeros((k, D), X.dtype)
     for d in range(D):
-        sums[:, d] = np.bincount(labels, weights=X[:, d], minlength=k)
-    # relocate empty clusters to the farthest points (_k_means_common.pyx:167-211)
+        sums[:, d] = np.bincount(labels, weights=X[:, d] if sw is None else X[:, d] * sw, minlength=k)
+    # relocate empty clusters to the farthest points (_k_means_common.pyx:167-211): the clusters of weight 0 are listed
+    # ONCE, before any move -- a cluster that a move empties stays empty -- and the n_empty farthest rows (unweighted
+    # distance to the old centre of their label; largest first, ties to the lowest row index, DESIGN.md section 3) move
+    # in, carrying x w and w
     empty = np.where(w == 0)[0]
     if empty.size:
         dist = ((X - centers_old[labels]) ** 2).sum(axis=1)
         if dist.max() > 0:
-            far = np.argpartition(dist, -empty.size)[:-empty.size - 1:-1]
-            for idx, new_id in enumerate(empty):
-                fi = far[idx]
+            far = np.lexsort((np.arange(dist.size), -dist))[:empty.size]
+            for fi, new_id in zip(far, empty):
                 old_id = labels[fi]
-                sums[old_id] -= X[fi]
-                sums[new_id] = X[fi]
-                w[new_id] = 1
-                w[old_id] -= 1
-    new = np.empty_like(sums)
+                wf = X.dtype.type(1.0) if sw is None else sw[fi]
+                xw = X[fi] if sw is None else X[fi] * wf
+                sums[old_id] -= xw
+                sums[new_id] = xw
+                w[new_id] = wf
+                w[old_id] -= wf
+    # _average_centers (:274-295) works in place in index order: an empty cluster copies row argmax(w) as it is at
+    # that moment -- still the heaviest cluster's SUM when the empty cluster's index is the lower one
+    new = sums.copy()
     amax = int(np.argmax(w))
     for j in range(k):
         if w[j] > 0:
-            new[j] = sums[j] * (X.dtype.type(1.0) / w[j])
-    for j in range(k):
-        if not w[j] > 0:
+            new[j] = new[j] * (X.dtype.type(1.0) / w[j])
+        else:
             new[j] = new[amax]
     shift = np.sqrt(((new - centers_old) ** 2).sum(axis=1))
     return new, w, shift
 
 
-def kmeans_fit(X, init, max_iter: int = 300, tol: float = 1e-4):
-    """KMeans(n_clusters=k, init=init, n_init=1, max_iter, tol).fit(X).
+def kmeans_fit(X, init, max_iter: int = 300, tol: float = 1e-4, sample_weight=None):
+    """KMeans(n_clusters=k, init=init, n_init=1, max_iter, tol).fit(X, sample_weight=sample_weight).
 
     Returns ``(labels int32[N], centers[k,D], inertia, n_iter)`` with the
     semantics of ``labels_``, ``cluster_centers_``, ``inertia_``, ``n_iter_``.
+    The weights enter the M-step sums, the relocation and the inertia; the
+    column mean, the tolerance and the E-step stay unweighted, as in sklearn.
     """
     X = np.asarray(X)
     dt = _work_dtype(X)
     X = X.astype(dt)                                      # uint8 -> float64
+    sw = None if sample_weight is None else np.asarray(sample_weight).astype(dt)
     centers = np.asarray(init).astype(dt).copy()
     tol_ = float(np.mean(np.var(X, axis=0)) * tol)        # _tolerance()
     mean = X.mean(axis=0)
@@ -92,7 +105,7 @@ def kmeans_fit(X, init, max_iter: int = 300, tol: float = 1e-4):
     labels = labels_old
     for it in range(max_iter):
         labels = _e_step(Xc, centers)
-        new, w, shift = _m_step(Xc, labels, centers)
+        new, w, shift = _m_step(Xc, labels, centers, sw)
         centers = new
         n_iter = it + 1
         if np.array_equal(labels, labels_old):
@@ -104,7 +117,10 @@ def kmeans_fit(X, init, max_iter: int = 300, tol: float = 1e-4):
     if not strict:
         labels = _e_step(Xc, centers)
     diff = Xc - centers[labels]
-    inertia = float((diff * diff).sum())
+    if sw is None:
+        inertia = float((diff * diff).sum())
+    else:
+        inertia = float(((diff * diff).sum(axis=1) * sw).sum())
     return labels, (centers + mean), inertia, n_iter
 
 
