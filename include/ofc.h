@@ -241,6 +241,18 @@ int ofc_kmeans_update(int batch, int64_t n, int d, int k, const double* sums, co
 int ofc_minibatch_update(const void* Xb, int dtype, int batch_rows, int d, int k, const int32_t* labels,
                          const double* centres_old, double* centres_new, double* weight_sums, void* stream);
 
+/* The same with sample weights, as MiniBatchKMeans.partial_fit(X, sample_weight=w) steps: per cluster,
+ * wsum = the members' weights in batch order; if wsum > 0, c_new = (c_old * weight_sum + x w of the members in batch
+ * order) / (weight_sum + wsum) and weight_sum += wsum, else the cluster keeps its centre and weight sum.  weights
+ * [batch_rows] are float64 holding values of the working type (float32 values for float32 rows).  Every product and
+ * sum is rounded on its own, as sklearn's loop; the result is that left fold's bits for every dtype and batch size.
+ * Both calls take any batch_rows >= 1 (a whole 1080p frame is one batch): one CTA per cluster streams the batch in
+ * order, on exact integer prefix sums where every increment is an integer, on the sequential fold elsewhere.
+ * centres_old and centres_new must not overlap. */
+int ofc_minibatch_update_weighted(const void* Xb, int dtype, int batch_rows, int d, int k, const int32_t* labels,
+                                  const double* weights, const double* centres_old, double* centres_new,
+                                  double* weight_sums, void* stream);
+
 /* Empty-cluster relocation on the sums/counts (_k_means_common.pyx:167-211): every empty
  * cluster, in index order, takes the point farthest from the (old) centre of its label.
  * Distances use (x - mean) against centres_old; raw_sums says whether `sums` holds sums of

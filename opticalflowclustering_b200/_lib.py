@@ -53,6 +53,7 @@ SIGNATURES = {
     "ofc_kmeans_update": (_i, [_i, _i64, _i, _i, _vp, _vp, _vp, _i, _i, _vp, _vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
                                _sz, _vp]),
     "ofc_minibatch_update": (_i, [_vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp]),
+    "ofc_minibatch_update_weighted": (_i, [_vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp]),
     "ofc_kmeans_relocate": (_i, [_vp, _i, _i, _i64, _i, _i, _vp, _vp, _vp, _vp, _vp, _i, _vp, _vp, _vp]),
     "ofc_kmeans_assign_weighted": (_i, [_vp, _i, _i, _i64, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
     "ofc_kmeans_sums_weighted": (_i, [_vp, _i, _i, _i64, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),

@@ -609,43 +609,157 @@ __global__ void __launch_bounds__(256) kmeans_update_kernel(int d, int k, const 
 // ---------------------------------------------------------------------------
 // MiniBatchKMeans centre update (reference color-quantization/quant.py:18-20 -> scikit-learn 1.9.0
 // sklearn/cluster/_k_means_minibatch.pyx:60-110, update_center_dense): per cluster, in the mini-batch's sample
-// order,  c_new = (c_old * weight_sum + sum of the members) / (weight_sum + n_members);  clusters without a member keep
-// their centre.  One thread per (cluster, feature) walks the batch sequentially -- the reference's accumulation
-// order, so the float result is the same; float32 data is worked in float32 like sklearn (W = float).
+// order,  wsum = the members' weights folded from 0;  if wsum > 0,  c_new = (c_old * weight_sum + x w of the members)
+// / (weight_sum + wsum)  and weight_sum += wsum;  else the cluster keeps its centre and weight sum (unit weights:
+// wsum = the member count).  Every product and sum is rounded on its own (no fma), as sklearn's C loop; float32 data
+// is worked in float32 like sklearn (W = float).
 // ---------------------------------------------------------------------------
-template <typename T, typename W>
-__global__ void __launch_bounds__(256) minibatch_update_kernel(const T* __restrict__ Xb, int bs, int d, int k,
-                                                               const int32_t* __restrict__ labels, const double* __restrict__ centres_old,
-                                                               double* __restrict__ centres_new, double* __restrict__ weight_sums) {
-    OFC_DYN_SMEM(int, s_lab);                            // [bs]
-    __shared__ int s_any;
-    for (int i = threadIdx.x; i < bs; i += 256) s_lab[i] = labels[i];
-    __syncthreads();
-    for (int e0 = 0; e0 < k * d; e0 += 256) {
-        const int e = e0 + threadIdx.x;
-        int cnt = 0, j = 0;
-        if (e < k * d) {
-            j = e / d;
-            const int t = e - j * d;
-            for (int i = 0; i < bs; ++i) cnt += s_lab[i] == j ? 1 : 0;
-            const W c_old = (W)centres_old[e];
-            W out = c_old;
-            if (cnt > 0) {
-                const W ws = (W)weight_sums[j];
-                W acc = c_old * ws;
-                for (int i = 0; i < bs; ++i)
-                    if (s_lab[i] == j) acc += (W)Xb[(int64_t)i * d + t];
-                const W ws_new = ws + (W)cnt;
-                const W alpha = (W)1 / ws_new;
-                out = acc * alpha;
+__device__ __forceinline__ double mul_rn(double a, double b) { return __dmul_rn(a, b); }
+__device__ __forceinline__ float mul_rn(float a, float b) { return __fmul_rn(a, b); }
+__device__ __forceinline__ double add_rn(double a, double b) { return __dadd_rn(a, b); }
+__device__ __forceinline__ float add_rn(float a, float b) { return __fadd_rn(a, b); }
+
+// One CTA of MB_NT threads per cluster j streams the batch in chunks of MB_NT rows, one row per thread, for
+// MB_FB features at a time plus one column for the weight fold (wsum, from 0).  Column c's running value lives in
+// thread c's register across the chunks.  Each chunk takes one of two paths, decided from its own values; both give
+// the bits of the sequential left fold acc <- acc + x w over the members in batch order:
+//  * exact-integer path: every member's increment x w (rounded in W) of every column is an integer in [0, 2^p) and
+//    acc + the chunk's total stays below 2^p (p = 53 for double, 24 for float).  Then the only adds that round are the
+//    ones where acc crosses a power of two (acc >= 0 grows monotonically, and below the next power of two B every sum
+//    acc + integer is representable as long as ulp(acc) <= 1).  The chunk keeps int64 inclusive prefix sums S of
+//    the increments per column; from acc, the first row i with S[i] - S[pos] >= B - acc (exact: Sterbenz) is the
+//    crossing one: acc + (S[i-1] - S[pos]) is exact, acc + inc[i-1] is the rounded add, as the sequential loop does
+//    it.  Once acc is an integer, acc + (the rest) is exact.  At most about p crossings per column per batch.
+//  * sequential path: otherwise (real weights, non-integer or negative rows), column c's thread folds the chunk's
+//    members in order, a chain of dependent adds as long as the member count.
+constexpr int MB_NT = 512;
+constexpr int MB_FB = 4;
+constexpr int MB_COLS = MB_FB + 1;
+
+template <typename W> struct fold_bits;
+template <> struct fold_bits<double> { static constexpr long long lim = 1ll << 53; };
+template <> struct fold_bits<float> { static constexpr long long lim = 1ll << 24; };
+
+template <typename T, typename W, bool WT>
+__global__ void __launch_bounds__(MB_NT) minibatch_stream_kernel(const T* __restrict__ Xb, int bs, int d, int k,
+                                                                 const int32_t* __restrict__ labels, const double* __restrict__ weights,
+                                                                 const double* __restrict__ centres_old,
+                                                                 double* __restrict__ centres_new, double* __restrict__ weight_sums) {
+    constexpr long long LIM = fold_bits<W>::lim;
+    __shared__ long long s_S[MB_COLS][MB_NT + 1];        // integer path: inclusive prefix sums; sequential path: W increments
+    __shared__ long long s_wtot[MB_COLS][MB_NT / 32];
+    __shared__ unsigned char s_mem[MB_NT];
+    __shared__ int s_any, s_frac, s_over;
+    const int j = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const W ws = (W)weight_sums[j];
+    W wsum_final = (W)0;
+    for (int f0 = 0; f0 < d; f0 += MB_FB) {
+        const int nf = min(MB_FB, d - f0);
+        // thread c < nf folds feature f0 + c from c_old * ws; thread MB_FB folds the weights from 0
+        W acc = (W)0;
+        if (tid < nf) acc = mul_rn((W)centres_old[(int64_t)j * d + f0 + tid], ws);
+        for (int i0 = 0; i0 < bs; i0 += MB_NT) {
+            const int i = i0 + tid;
+            const bool member = i < bs && labels[i] == j;
+            W inc[MB_COLS];
+            bool frac = false;
+            const W w = member ? (WT ? (W)weights[i] : (W)1) : (W)0;
+#pragma unroll
+            for (int c = 0; c < MB_COLS; ++c) {
+                W v = (W)0;
+                if (c == MB_FB) v = w;
+                else if (member && c < nf) v = mul_rn((W)Xb[(int64_t)i * d + f0 + c], w);      // exact when w = 1
+                inc[c] = v;
+                if (member && !(v >= (W)0 && v < (W)LIM && v == floor(v))) frac = true;
             }
+            if (tid == 0) { s_any = 0; s_frac = 0; s_over = 0; }
+            __syncthreads();
+            s_mem[tid] = member ? 1 : 0;
+            if (member) s_any = 1;
+            if (frac) s_frac = 1;
+            __syncthreads();
+            if (!s_any) continue;                          // uniform: no member of j in this chunk
+            bool integer = !s_frac;
+            if (integer) {
+#pragma unroll
+                for (int c = 0; c < MB_COLS; ++c) {
+                    long long v = (long long)inc[c];
+#pragma unroll
+                    for (int o = 1; o < 32; o <<= 1) {
+                        const long long u = __shfl_up_sync(0xffffffffu, v, o);
+                        if (lane >= o) v += u;
+                    }
+                    s_S[c][tid + 1] = v;
+                    if (lane == 31) s_wtot[c][warp] = v;
+                }
+                __syncthreads();
+#pragma unroll
+                for (int c = 0; c < MB_COLS; ++c) {
+                    long long off = 0;
+                    for (int q = 0; q < warp; ++q) off += s_wtot[c][q];
+                    s_S[c][tid + 1] += off;
+                }
+                if (tid < MB_COLS) s_S[tid][0] = 0;
+                __syncthreads();
+                if (tid < MB_COLS) {
+                    const long long tot = s_S[tid][MB_NT];
+                    if (!(acc >= (W)0 && tot < LIM && acc < (W)(LIM - tot))) s_over = 1;
+                }
+                __syncthreads();
+                integer = !s_over;                         // the readers of s_S are past the barrier above
+            }
+            if (!integer) {
+#pragma unroll
+                for (int c = 0; c < MB_COLS; ++c) {
+                    W* col = reinterpret_cast<W*>(&s_S[c][1]);
+                    col[tid] = inc[c];
+                }
+                __syncthreads();
+            }
+            if (tid < MB_COLS && (tid < nf || tid == MB_FB)) {
+                const long long* S = s_S[tid];
+                if (integer) {
+                    int pos = 0;
+                    while (true) {
+                        if (acc == floor(acc)) { acc = add_rn(acc, (W)(S[MB_NT] - S[pos])); break; }
+                        int e;
+                        frexp(acc, &e);
+                        const W gap = add_rn((W)ldexp((W)1, e), -acc);
+                        const long long need = S[pos] + (long long)ceil(gap);
+                        // first row index r in (pos, MB_NT] with S[r] >= need
+                        int lo = pos + 1, hi = MB_NT + 1;
+                        while (lo < hi) {
+                            const int mid = (lo + hi) >> 1;
+                            if (S[mid] >= need) hi = mid; else lo = mid + 1;
+                        }
+                        if (lo > MB_NT) { acc = add_rn(acc, (W)(S[MB_NT] - S[pos])); break; }
+                        acc = add_rn(acc, (W)(S[lo - 1] - S[pos]));
+                        acc = add_rn(acc, (W)(S[lo] - S[lo - 1]));
+                        pos = lo;
+                    }
+                } else {
+                    const W* col = reinterpret_cast<const W*>(&S[1]);
+                    for (int r = 0; r < MB_NT; ++r)
+                        if (s_mem[r]) acc = add_rn(acc, col[r]);
+                }
+            }
+            __syncthreads();                               // s_S and s_mem are rewritten by the next chunk
+        }
+        // thread MB_FB holds wsum; the features need it
+        __shared__ W s_wsum;
+        if (tid == MB_FB) s_wsum = acc;
+        __syncthreads();
+        const W wsum = s_wsum;
+        if (tid < nf) {
+            const int64_t e = (int64_t)j * d + f0 + tid;
+            W out = (W)centres_old[e];
+            if (wsum > (W)0) out = mul_rn(acc, (W)1 / add_rn(ws, wsum));
             centres_new[e] = (double)out;
         }
-        __syncthreads();                                  // every feature of a cluster has read its old weight
-        if (e < k * d && e - j * d == 0 && cnt > 0) weight_sums[j] = (double)((W)weight_sums[j] + (W)cnt);
-        if (threadIdx.x == 0) s_any = 0;
+        wsum_final = wsum;
         __syncthreads();
     }
+    if (tid == 0 && wsum_final > (W)0) weight_sums[j] = (double)(ws + wsum_final);
 }
 
 __global__ void kmeans_counter_inc_kernel(int* counter) { *counter += 1; }
@@ -1729,23 +1843,25 @@ int launch_kmeans_update(int batch, int d, int k, const double* sums, const doub
                          tol, it, active, just_done, n_iter, n_active, n, labels_cur, labels_other, it_counter, stream);
 }
 
-int launch_minibatch_update(const void* Xb, int dtype, int bs, int d, int k, const int32_t* labels, const double* centres_old,
-                            double* centres_new, double* weight_sums, void* stream) {
-    const size_t smem = (size_t)bs * sizeof(int);
-    if (smem > 200 * 1024) { set_error("mini-batch of %d rows is too large (<= 51200)", bs); return OFC_ERR_UNSUPPORTED; }
+template <bool WT>
+static int launch_minibatch(const void* Xb, int dtype, int bs, int d, int k, const int32_t* labels, const double* weights,
+                            const double* centres_old, double* centres_new, double* weight_sums, void* stream) {
     ProfScope prof(PK_KMEANS, stream);
 #define OFC_MB(TT, WW)                                                                                               \
-    {                                                                                                                \
-        OFC_SMEM_OPTIN((minibatch_update_kernel<TT, WW>), smem);                                                     \
-        OFC_LAUNCH((minibatch_update_kernel<TT, WW>), dim3(1), dim3(256), smem, stream, (const TT*)Xb, bs, d, k, labels, \
-                   centres_old, centres_new, weight_sums);                                                           \
-    }
-    if (dtype == DT_U8) OFC_MB(unsigned char, double)
-    else if (dtype == DT_F32) OFC_MB(float, float)
-    else OFC_MB(double, double)
+    OFC_LAUNCH((minibatch_stream_kernel<TT, WW, WT>), dim3(k), dim3(MB_NT), 0, stream, (const TT*)Xb, bs, d, k, labels, \
+               weights, centres_old, centres_new, weight_sums);
+    if (dtype == DT_U8) { OFC_MB(unsigned char, double) }
+    else if (dtype == DT_F32) { OFC_MB(float, float) }
+    else { OFC_MB(double, double) }
 #undef OFC_MB
     OFC_CHECK_LAUNCH("minibatch_update");
     return OFC_OK;
+}
+
+int launch_minibatch_update(const void* Xb, int dtype, int bs, int d, int k, const int32_t* labels, const double* weights,
+                            const double* centres_old, double* centres_new, double* weight_sums, void* stream) {
+    if (weights) return launch_minibatch<true>(Xb, dtype, bs, d, k, labels, weights, centres_old, centres_new, weight_sums, stream);
+    return launch_minibatch<false>(Xb, dtype, bs, d, k, labels, nullptr, centres_old, centres_new, weight_sums, stream);
 }
 
 static int rowdist_grid(int64_t n, int batch) {

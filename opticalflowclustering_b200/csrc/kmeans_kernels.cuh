@@ -70,8 +70,9 @@ int launch_kmeans_update(int batch, int d, int k, const double* sums, const doub
                          const unsigned long long* n_changed, const double* tol, int it, unsigned char* active,
                          unsigned char* just_done, int* n_iter, int* n_active, int64_t n, const int32_t* labels_cur,
                          int32_t* labels_other, int* it_counter, void* stream);
-int launch_minibatch_update(const void* Xb, int dtype, int bs, int d, int k, const int32_t* labels, const double* centres_old,
-                            double* centres_new, double* weight_sums, void* stream);
+// weights NULL: unit weights (the unweighted kernel)
+int launch_minibatch_update(const void* Xb, int dtype, int bs, int d, int k, const int32_t* labels, const double* weights,
+                            const double* centres_old, double* centres_new, double* weight_sums, void* stream);
 int launch_kmeans_relocate(const void* X, int64_t x_stride, int dtype, int batch, int64_t n, int d, int k, const double* mean,
                            const int32_t* labels, const double* centres_old, double* sums, long long* counts,
                            int raw_sums, const unsigned char* active, double* scratch, void* stream);

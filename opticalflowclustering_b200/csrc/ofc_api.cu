@@ -892,7 +892,16 @@ int ofc_minibatch_update(const void* Xb, int dtype, int batch_rows, int d, int k
     OFC_REQUIRE(dtype == OFC_U8 || dtype == OFC_F32 || dtype == OFC_F64, "bad dtype %d", dtype);
     OFC_REQUIRE(batch_rows >= 1 && d >= 1 && k >= 1, "bad shape");
     OFC_REQUIRE(Xb && labels && centres_old && centres_new && weight_sums, "null buffer");
-    return launch_minibatch_update(Xb, dtype, batch_rows, d, k, labels, centres_old, centres_new, weight_sums, stream);
+    return launch_minibatch_update(Xb, dtype, batch_rows, d, k, labels, nullptr, centres_old, centres_new, weight_sums, stream);
+}
+
+int ofc_minibatch_update_weighted(const void* Xb, int dtype, int batch_rows, int d, int k, const int32_t* labels,
+                                  const double* weights, const double* centres_old, double* centres_new, double* weight_sums,
+                                  void* stream) {
+    OFC_REQUIRE(dtype == OFC_U8 || dtype == OFC_F32 || dtype == OFC_F64, "bad dtype %d", dtype);
+    OFC_REQUIRE(batch_rows >= 1 && d >= 1 && k >= 1, "bad shape");
+    OFC_REQUIRE(Xb && labels && weights && centres_old && centres_new && weight_sums, "null buffer");
+    return launch_minibatch_update(Xb, dtype, batch_rows, d, k, labels, weights, centres_old, centres_new, weight_sums, stream);
 }
 
 int ofc_kmeans_relocate(const void* X, int dtype, int batch, int64_t n, int d, int k, const double* mean,

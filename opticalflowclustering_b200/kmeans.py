@@ -891,13 +891,14 @@ def best_start(labels, inertia, k: int) -> int:
     return best
 
 
-def _resolve_n_init(n_init, init) -> int:
-    """sklearn's ``_check_params_vs_input`` (_kmeans.py:884-907): "auto" is 1 for k-means++ and an array, 10 for
-    "random"; an array with n_init != 1 warns and runs one start."""
+def _resolve_n_init(n_init, init, default_n_init: int = 10) -> int:
+    """sklearn's ``_check_params_vs_input`` (_kmeans.py:884-907): "auto" is 1 for k-means++ and an array,
+    ``default_n_init`` for "random" (10 for KMeans, 3 for MiniBatchKMeans); an array with n_init != 1 warns and runs
+    one start."""
     if isinstance(n_init, str):
         if n_init != "auto":
             raise ValueError(f"n_init must be 'auto' or an int >= 1, got {n_init!r}")
-        r = 10 if isinstance(init, str) and init == "random" else 1
+        r = default_n_init if isinstance(init, str) and init == "random" else 1
     else:
         if isinstance(n_init, bool) or not isinstance(n_init, (int, np.integer)) or n_init < 1:
             raise ValueError(f"n_init must be 'auto' or an int >= 1, got {n_init!r}")
@@ -992,16 +993,22 @@ class KMeans:
     def score(self, X, y=None, sample_weight=None):
         """sklearn's ``KMeans.score`` (_kmeans.py:1159-1187): minus the (weighted) inertia of X against the fitted centres,
         on the un-centred rows as :meth:`predict` assigns them."""
-        Xb, single = _as_batch(X, _target_device(X))
-        if not single:
-            raise ValueError("Expected 2D array")
-        n = int(Xb.shape[1])
-        w = _check_sample_weight(sample_weight, n, Xb.dtype)
-        w = None if w is None else torch.from_numpy(w.astype(np.float64)).to(Xb.device)
-        c = self._centres_t.to(device=Xb.device, dtype=torch.float64).unsqueeze(0).contiguous()
-        st = LloydState(_Ctx(Xb.device), Xb, int(c.shape[1]), weights=w)
-        st.assign(None, c, st.labels[0], inertia=st.inertia)
-        return -float(st.inertia[0].item())
+        return score(X, self._centres_t, sample_weight)
+
+
+def score(X, centres, sample_weight=None) -> float:
+    """sklearn's ``score`` of KMeans and MiniBatchKMeans (_kmeans.py:1159-1187): minus the (weighted) inertia of X
+    ``[n, d]`` against ``centres`` ``[k, d]``, on the un-centred rows as :func:`predict` assigns them."""
+    Xb, single = _as_batch(X, _target_device(X))
+    if not single:
+        raise ValueError("Expected 2D array")
+    n = int(Xb.shape[1])
+    w = _check_sample_weight(sample_weight, n, Xb.dtype)
+    w = None if w is None else torch.from_numpy(w.astype(np.float64)).to(Xb.device)
+    c = centres.to(device=Xb.device, dtype=torch.float64).unsqueeze(0).contiguous()
+    st = LloydState(_Ctx(Xb.device), Xb, int(c.shape[1]), weights=w)
+    st.assign(None, c, st.labels[0], inertia=st.inertia)
+    return -float(st.inertia[0].item())
 
 
 def kmeans_fit(X, init, max_iter: int = 300, tol: float = 1e-4, sample_weight=None):
