@@ -422,6 +422,19 @@ int ofc_kmeans_tc_sums_u8_weighted(const uint8_t* X, int64_t n, int d, int k, co
                                    double* sums, int64_t* counts, double* weight_sums, void* workspace, size_t workspace_bytes,
                                    void* stream);
 
+/* ---- k-means transform: row-to-centre distances ----------------------------
+ * Replaces KMeans.transform(X) / MiniBatchKMeans.transform(X) (and the transform half of fit_transform), which
+ * scikit-learn 1.9.0 computes as euclidean_distances(X, cluster_centers_) (sklearn/cluster/_kmeans.py _transform,
+ * sklearn/metrics/pairwise.py _euclidean_distances; float32 inputs are upcast chunk by chunk to float64 by
+ * _euclidean_distances_upcast because the norm form cancels).  out[i][j] = sqrt(d2) with d2 one sequential float64 fma
+ * chain over t = 0 .. d-1 of (double(X[i][t]) - centres[j][t])^2 -- the direct difference, on the un-centred rows,
+ * correctly rounded square roots.  With out_f32 the output is float32: sqrtf(float(d2)), sklearn's float32 path after its
+ * float64 chunk.  An element depends only on its row and centre (not on n, k or the kernel form).
+ * dtype OFC_U8 / OFC_F32 / OFC_F64; centres f64 [k][d] (float32 values for a float32 fit); out f64 [n][k], or f32 [n][k]
+ * when out_f32, which is valid with OFC_F32 rows only (OFC_ERR_INVALID otherwise).  n may exceed 2^31 / k. */
+int ofc_kmeans_distances(const void* X, int dtype, int64_t n, int d, int k,
+                         const double* centres /* [k][d] */, void* out /* [n][k] */, int out_f32, void* stream);
+
 /* image_dict ROIs (KmeanGrids.py:85,113) + preprocess_image (:269-286) for every cell:
  * out u8 [n_frames][rows*cols][ (H/rows)*(W/cols) ][4] = (c0, c1, c2, alpha).  draw_lines:
  * white row 0 / column 0 as at the reference's k-means stage (SURVEY.md Q3); swap_rb:

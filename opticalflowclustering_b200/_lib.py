@@ -84,6 +84,7 @@ SIGNATURES = {
     "ofc_kmeans_tc_assign_weighted": (_i, [_vp, _vp, _vp, _i64, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
     "ofc_kmeans_tc_sums_weighted": (_i, [_vp, _vp, _i64, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
     "ofc_kmeans_tc_sums_u8_weighted": (_i, [_vp, _i64, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "ofc_kmeans_distances": (_i, [_vp, _i, _i64, _i, _i, _vp, _vp, _i, _vp]),
     "ofc_grid_extract_cells": (_i, [_vp, _i, _i, _i, _i, _i, _i, _i, _i, _vp, _vp]),
     "ofc_sliding_cosine": (_i, [_vp, _i, _vp, _i64, _vp, _vp, _vp, _vp]),
     "ofc_row_cosine": (_i, [_vp, _i, _i64, _i, _vp, _vp, _vp]),

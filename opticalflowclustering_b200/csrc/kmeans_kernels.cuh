@@ -122,6 +122,9 @@ int launch_kmeans_cells_fast(KmCellsFastParams p, int batch, void* stream);
 bool kmeans_step_u8d4_usable(const KmAssignParams& p, int batch);
 int launch_kmeans_step_u8d4(const KmAssignParams& p, int batch, int grid, double* partial, long long* cnt_partial, void* stream);
 int kmeans_assign_grid(int64_t n);
+// row-to-centre distances (kmeans_distances.cu); out_f32 only with float32 rows (the caller checks)
+int launch_kmeans_distances(const void* X, int dtype, int64_t n, int d, int k, const double* centres, void* out, int out_f32,
+                            void* stream);
 int kmeans_sums_splits(int64_t n, int batch);
 
 int launch_sliding_cosine(const double* a, int n, const double* b, int64_t m, double* sims, double* best,

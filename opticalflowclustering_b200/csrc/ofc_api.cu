@@ -1041,6 +1041,16 @@ int ofc_grid_extract_cells(const uint8_t* bgr, int n_frames, int height, int wid
     return launch_extract_cells(bgr, n_frames, height, width, rows, cols, draw_lines, threshold, swap_rb, out, stream);
 }
 
+int ofc_kmeans_distances(const void* X, int dtype, int64_t n, int d, int k, const double* centres, void* out, int out_f32,
+                         void* stream) {
+    OFC_REQUIRE(dtype == OFC_U8 || dtype == OFC_F32 || dtype == OFC_F64, "bad dtype %d", dtype);
+    OFC_REQUIRE(!out_f32 || dtype == OFC_F32, "float32 output needs float32 rows (dtype %d)", dtype);
+    OFC_REQUIRE(n >= 0 && d >= 1 && k >= 1, "bad shape n=%lld d=%d k=%d", (long long)n, d, k);
+    if (n == 0) return OFC_OK;
+    OFC_REQUIRE(X && centres && out, "null buffer");
+    return launch_kmeans_distances(X, dtype, n, d, k, centres, out, out_f32 ? 1 : 0, stream);
+}
+
 // ---- cosine ----------------------------------------------------------------
 int ofc_sliding_cosine(const double* a, int n, const double* b, int64_t m, double* sims, double* best,
                        int64_t* best_idx, void* stream) {

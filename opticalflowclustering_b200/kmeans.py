@@ -761,6 +761,42 @@ def predict(X, centres):
     return st.labels[0][0] if single else st.labels[0]
 
 
+def transform(X, centres):
+    """``KMeans.transform``: every row's Euclidean distance to every centre, ``euclidean_distances(X, centres)``
+    (_kmeans.py ``_transform``), as ``[n, k]`` on X's compute device.  The distances are the direct difference in float64
+    on the un-centred rows (``ofc_kmeans_distances``), not sklearn's norm form, so they do not cancel.  The output is
+    float32 exactly when X and ``centres`` are both float32 (sklearn's ``check_pairwise_arrays``), float64 otherwise;
+    X of another dtype is worked as float64, as sklearn's ``validate_data(dtype=[float64, float32])``."""
+    Xb, single = _as_batch(X, _target_device(X))
+    if not single:
+        raise ValueError("Expected 2D array")
+    n, d = int(Xb.shape[1]), int(Xb.shape[2])
+    if n == 0:
+        raise ValueError(f"Found array with 0 sample(s) (shape=(0, {d})) while a minimum of 1 is required.")
+    c = centres if isinstance(centres, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(centres))
+    out_f32 = Xb.dtype == torch.float32 and c.dtype == torch.float32
+    c = c.to(device=Xb.device, dtype=torch.float64).contiguous()
+    if c.dim() != 2 or int(c.shape[1]) != d:
+        raise ValueError(f"centres shape {tuple(c.shape)} does not match X with {d} features")
+    k = int(c.shape[0])
+    out = torch.empty((n, k), dtype=torch.float32 if out_f32 else torch.float64, device=Xb.device)
+    ctx = _Ctx(Xb.device)
+    ctx.check(ctx.lib.ofc_kmeans_distances(_ptr(Xb), _DT[Xb.dtype], C.c_int64(n), d, k, _ptr(c), _ptr(out), int(out_f32),
+                                           ctx.stream()))
+    return out
+
+
+def _estimator_transform(est, X):
+    """``transform`` of KMeans and MiniBatchKMeans: the feature-count check, the centres sklearn's ``cluster_centers_``
+    holds (float32 after a float32 fit), and numpy out for anything but a torch tensor in"""
+    d = int(X.shape[1]) if np.ndim(X) == 2 else None
+    if d is not None and d != est.n_features_in_:
+        raise ValueError(f"X has {d} features, but {type(est).__name__} is expecting {est.n_features_in_} features as input.")
+    centres = est._centres_t.to(torch.float32) if est._f32 else est._centres_t
+    out = transform(X, centres)
+    return out if isinstance(X, torch.Tensor) else out.cpu().numpy()
+
+
 def kmeans_plusplus(X, n_clusters: int, random_state=None, sample_weight=None):
     """k-means++ seeding with sklearn's procedure and RNG call sequence
     (sklearn/cluster/_kmeans.py:181-268): first centre by ``random_state.choice``, then
@@ -976,6 +1012,9 @@ class KMeans:
                 init = self.init
             labels, centres, inertia, n_iter = lloyd(Xa, init, self.max_iter, self.tol, sample_weight=sw)
         self._centres_t = centres
+        # a float32 fit: sklearn's cluster_centers_ are float32, and transform measures against those
+        self._f32 = Xa.dtype == (torch.float32 if isinstance(Xa, torch.Tensor) else np.float32)
+        self.n_features_in_ = int(Xa.shape[1])
         self.cluster_centers_ = centres.cpu().numpy()
         if not isinstance(X, torch.Tensor) and np.asarray(X).dtype == np.float32:
             self.cluster_centers_ = self.cluster_centers_.astype(np.float32)
@@ -994,6 +1033,14 @@ class KMeans:
         """sklearn's ``KMeans.score`` (_kmeans.py:1159-1187): minus the (weighted) inertia of X against the fitted centres,
         on the un-centred rows as :meth:`predict` assigns them."""
         return score(X, self._centres_t, sample_weight)
+
+    def transform(self, X):
+        """sklearn's ``KMeans.transform``: the ``[n, k]`` distances of X's rows to ``cluster_centers_`` (see
+        :func:`transform`).  numpy in gives numpy out; a torch tensor in gives a tensor on the compute device."""
+        return _estimator_transform(self, X)
+
+    def fit_transform(self, X, y=None, sample_weight=None):
+        return self.fit(X, sample_weight=sample_weight).transform(X)
 
 
 def score(X, centres, sample_weight=None) -> float:

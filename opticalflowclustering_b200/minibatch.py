@@ -293,6 +293,13 @@ class MiniBatchKMeans:
         """minus the (weighted) inertia of X against the centres (sklearn's ``score``, shared with KMeans)"""
         return _km.score(X, self._centres_t, sample_weight)
 
+    def transform(self, X):
+        """sklearn's ``transform``: the ``[n, k]`` distances of X's rows to ``cluster_centers_`` (:func:`kmeans.transform`)"""
+        return _km._estimator_transform(self, X)
+
+    def fit_transform(self, X, y=None, sample_weight=None):
+        return self.fit(X, sample_weight=sample_weight).transform(X)
+
 
 def quantize(image_lab, n_clusters, random_state=None):
     """quant.py:15-20 on an image that is already in LAB (uint8 [H, W, 3], numpy or CUDA tensor): returns
