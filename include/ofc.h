@@ -435,6 +435,57 @@ int ofc_kmeans_tc_sums_u8_weighted(const uint8_t* X, int64_t n, int d, int k, co
 int ofc_kmeans_distances(const void* X, int dtype, int64_t n, int d, int k,
                          const double* centres /* [k][d] */, void* out /* [n][k] */, int out_f32, void* stream);
 
+/* ---- k-means (Elkan) --------------------------------------------------------
+ * KMeans(algorithm="elkan").fit as scikit-learn 1.9.0 runs it (sklearn/cluster/_kmeans.py:462-624,
+ * _kmeans_single_elkan; dense kernels in _k_means_elkan.pyx).  The M-step, relocation and centre update are
+ * the Lloyd calls above (ofc_kmeans_sums[_weighted], ofc_kmeans_relocate[_weighted], ofc_kmeans_update[_weighted]);
+ * these calls keep the triangle-inequality bounds.  The working type W is float for OFC_F32 rows and double for
+ * OFC_U8 and OFC_F64 rows: upper [batch][n], lower [batch][n][k] (a row's k bounds contiguous), chd [batch][k][k] and
+ * dnc [batch][k] are W arrays the caller owns.  Every distance is _euclidean_dense_dense (_k_means_common.pyx:16-43)
+ * in W on the centred rows: groups of four features summed ((d0^2 + d1^2) + d2^2) + d3^2, then added to the total,
+ * the remainder one feature at a time, every operation rounded on its own, the square root in W.  `mean`, `batch`,
+ * `active` and OFC_KMEANS_SHARED_ROWS (in dtype) as in ofc_kmeans_assign.  k >= 2 (np.partition(kth=1) of the
+ * centre geometry needs two centres); OFC_ERR_INVALID otherwise. */
+
+/* chd = euclidean_distances(centres) / 2 and dnc = np.partition(chd, kth=1, axis=0)[1] (_kmeans.py:531-534, 575-578),
+ * on the device (no host read-back): chd from ofc_kmeans_distances (centres against centres, direct difference;
+ * float32 output for OFC_F32), halved in W.  This differs from sklearn's norm form in the last bits; only the pruning
+ * reads it.  Every problem is recomputed.  workspace: batch * k * d * 4 bytes for OFC_F32, unused otherwise. */
+int ofc_kmeans_elkan_centres(int dtype, int batch, int d, int k, const double* centres /* [batch][k][d] */,
+                             void* chd, void* dnc, void* workspace, size_t workspace_bytes, void* stream);
+/* init_bounds_dense (_k_means_elkan.pyx:24-97): labels, upper = the distance to the chosen centre, lower[i][j] = the
+ * distances computed (to centre 0, then to centre j only while min_dist > chd[best][j]), 0 elsewhere.  A label changes
+ * on a strictly smaller distance only. */
+int ofc_kmeans_elkan_init(const void* X, int dtype, int batch, int64_t n, int d, int k, const double* mean,
+                          const double* centres, const void* chd, int32_t* labels, void* upper, void* lower,
+                          const uint8_t* active, void* stream);
+/* the label half of _update_chunk_dense (_k_means_elkan.pyx:352-427) over all rows: a row is skipped when
+ * dnc[label] >= upper; otherwise every centre j other than the current label with upper > lower[j] and
+ * upper > chd[label][j] makes the upper bound tight once (stored in lower[label]) and, if upper > lower[j] or
+ * upper > chd[label][j] still holds, has its distance stored in lower[j] and taken when strictly smaller.
+ * Reads labels_in (may equal labels), writes labels, upper and lower.  n_changed (nullable) = #{i: labels[i] !=
+ * prev_labels[i]} for the active problems, every row when prev_labels is NULL (sklearn's -1 start); n_dist
+ * (nullable) += the distances evaluated. */
+int ofc_kmeans_elkan_step(const void* X, int dtype, int batch, int64_t n, int d, int k, const double* mean,
+                          const double* centres, const void* chd, const void* dnc, const int32_t* labels_in,
+                          int32_t* labels, const int32_t* prev_labels, void* upper, void* lower, uint64_t* n_changed,
+                          uint64_t* n_dist, const uint8_t* active, void* stream);
+/* the end of elkan_iter_chunked_dense (_k_means_elkan.pyx:331-343): shift[j] = _center_shift of centres_old and
+ * centres (:298-311 of _k_means_common.pyx, in W), then upper[i] += shift[labels[i]] and lower[i][j] -= shift[j]
+ * clamped at 0.  A problem is updated when active[b] or just_done[b] is set (both nullable; active NULL = all): the
+ * iteration that stops a fit still updates its bounds, as sklearn does before its stopping test.  workspace:
+ * batch * k * 8 bytes. */
+int ofc_kmeans_elkan_bounds(int dtype, int batch, int64_t n, int d, int k, const double* centres_old,
+                            const double* centres, const int32_t* labels, void* upper, void* lower,
+                            const uint8_t* active, const uint8_t* just_done, void* workspace, size_t workspace_bytes,
+                            void* stream);
+/* _inertia_dense (_k_means_common.pyx) of the given labels: inertia[b] = sum over rows of the squared distance (in W)
+ * to the centre of its label, times its weight (weights [batch][n], [n] with OFC_KMEANS_SHARED_ROWS, or NULL).
+ * workspace: ofc_kmeans_assign_workspace_bytes. */
+int ofc_kmeans_elkan_inertia(const void* X, int dtype, int batch, int64_t n, int d, int k, const double* mean,
+                             const double* centres, const int32_t* labels, const double* weights, double* inertia,
+                             const uint8_t* active, void* workspace, size_t workspace_bytes, void* stream);
+
 /* image_dict ROIs (KmeanGrids.py:85,113) + preprocess_image (:269-286) for every cell:
  * out u8 [n_frames][rows*cols][ (H/rows)*(W/cols) ][4] = (c0, c1, c2, alpha).  draw_lines:
  * white row 0 / column 0 as at the reference's k-means stage (SURVEY.md Q3); swap_rb:

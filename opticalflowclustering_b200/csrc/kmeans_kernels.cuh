@@ -126,6 +126,36 @@ int kmeans_assign_grid(int64_t n);
 int launch_kmeans_distances(const void* X, int dtype, int64_t n, int d, int k, const double* centres, void* out, int out_f32,
                             void* stream);
 int kmeans_sums_splits(int64_t n, int batch);
+// Elkan step kernels (kmeans_elkan.cu).  Bounds, chd and dnc are in the working type: float for DT_F32, else double.
+struct ElkanArgs {
+    const void* X;
+    int64_t x_stride;            // n * d, or 0 (OFC_KMEANS_SHARED_ROWS)
+    int dtype, batch;
+    int64_t n;
+    int d, k;
+    const double* mean;          // [batch][d] or null
+    const double* centres;       // [batch][k][d]
+    const void* chd;             // [batch][k][k] centre half-distances
+    const void* dnc;             // [batch][k] (step only)
+    const int32_t* labels_in;    // [batch][n] (step only; may equal labels)
+    int32_t* labels;             // [batch][n] out
+    const int32_t* prev_labels;  // [batch][n] or null (step only: every row counts as changed)
+    void* upper;                 // [batch][n]
+    void* lower;                 // [batch][n][k]
+    unsigned long long* n_changed;   // [batch] or null (step only)
+    unsigned long long* n_dist;      // [batch] or null (step only: += distances evaluated)
+    const unsigned char* active;
+    bool init;                   // init_bounds_dense instead of the step
+};
+int launch_kmeans_elkan(const ElkanArgs& a, void* stream);
+int launch_kmeans_elkan_bounds(int dtype, int batch, int64_t n, int d, int k, const double* centres_old, const double* centres,
+                               const int32_t* labels, void* upper, void* lower, const unsigned char* active,
+                               const unsigned char* just_done, void* shift_ws, void* stream);
+int launch_kmeans_elkan_centres(int dtype, int batch, int d, int k, const double* centres, void* chd, void* dnc, float* f32_ws,
+                                void* stream);
+int launch_kmeans_elkan_inertia(const void* X, int64_t x_stride, int dtype, int batch, int64_t n, int d, int k, const double* mean,
+                                const double* centres, const int32_t* labels, const double* weights, int64_t w_stride, double* partial,
+                                int parts, double* inertia, const unsigned char* active, void* stream);
 
 int launch_sliding_cosine(const double* a, int n, const double* b, int64_t m, double* sims, double* best,
                           long long* best_idx, void* stream);

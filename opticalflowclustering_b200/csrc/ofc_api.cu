@@ -1051,6 +1051,95 @@ int ofc_kmeans_distances(const void* X, int dtype, int64_t n, int d, int k, cons
     return launch_kmeans_distances(X, dtype, n, d, k, centres, out, out_f32 ? 1 : 0, stream);
 }
 
+// ---- k-means (Elkan) -------------------------------------------------------
+static int elkan_check(const void* X, int& dtype, bool& shared, int batch, int64_t n, int d, int k) {
+    int rc = km_check(X, dtype, shared, batch, n, d, k);
+    if (rc != OFC_OK) return rc;
+    OFC_REQUIRE(k >= 2, "Elkan needs k >= 2 (k=%d)", k);
+    OFC_REQUIRE(batch <= 65535, "Elkan batch too large (%d)", batch);
+    return OFC_OK;
+}
+
+int ofc_kmeans_elkan_centres(int dtype, int batch, int d, int k, const double* centres, void* chd, void* dnc, void* workspace,
+                             size_t workspace_bytes, void* stream) {
+    bool shared;
+    int rc = elkan_check(centres, dtype, shared, batch, 1, d, k);
+    if (rc != OFC_OK) return rc;
+    if (batch == 0) return OFC_OK;
+    OFC_REQUIRE(chd && dnc, "null chd / dnc");
+    const size_t need = dtype == OFC_F32 ? (size_t)batch * k * d * sizeof(float) : 0;
+    if (need && (!workspace || workspace_bytes < need)) { set_error("Elkan centre workspace too small: %zu < %zu", workspace_bytes, need); return OFC_ERR_WORKSPACE; }
+    return launch_kmeans_elkan_centres(dtype, batch, d, k, centres, chd, dnc, (float*)workspace, stream);
+}
+
+static ElkanArgs elkan_args(const void* X, int dtype, bool shared, int batch, int64_t n, int d, int k, const double* mean,
+                            const double* centres, const void* chd, int32_t* labels, void* upper, void* lower, const uint8_t* active) {
+    ElkanArgs a{};
+    a.X = X; a.x_stride = shared ? 0 : n * d; a.dtype = dtype; a.batch = batch; a.n = n; a.d = d; a.k = k; a.mean = mean;
+    a.centres = centres; a.chd = chd; a.labels = labels; a.upper = upper; a.lower = lower; a.active = active;
+    return a;
+}
+
+int ofc_kmeans_elkan_init(const void* X, int dtype, int batch, int64_t n, int d, int k, const double* mean, const double* centres,
+                          const void* chd, int32_t* labels, void* upper, void* lower, const uint8_t* active, void* stream) {
+    bool shared;
+    int rc = elkan_check(X, dtype, shared, batch, n, d, k);
+    if (rc != OFC_OK) return rc;
+    if (batch == 0 || n == 0) return OFC_OK;
+    OFC_REQUIRE(centres && chd && labels && upper && lower, "null buffer");
+    ElkanArgs a = elkan_args(X, dtype, shared, batch, n, d, k, mean, centres, chd, labels, upper, lower, active);
+    a.init = true;
+    return launch_kmeans_elkan(a, stream);
+}
+
+int ofc_kmeans_elkan_step(const void* X, int dtype, int batch, int64_t n, int d, int k, const double* mean, const double* centres,
+                          const void* chd, const void* dnc, const int32_t* labels_in, int32_t* labels, const int32_t* prev_labels,
+                          void* upper, void* lower, uint64_t* n_changed, uint64_t* n_dist, const uint8_t* active, void* stream) {
+    bool shared;
+    int rc = elkan_check(X, dtype, shared, batch, n, d, k);
+    if (rc != OFC_OK) return rc;
+    if (batch == 0 || n == 0) {
+        if (batch > 0 && n_changed) OFC_CUDA(cudaMemsetAsync(n_changed, 0, sizeof(uint64_t) * batch, (cudaStream_t)stream));
+        return OFC_OK;
+    }
+    OFC_REQUIRE(centres && chd && dnc && labels_in && labels && upper && lower, "null buffer");
+    ElkanArgs a = elkan_args(X, dtype, shared, batch, n, d, k, mean, centres, chd, labels, upper, lower, active);
+    a.dnc = dnc; a.labels_in = labels_in; a.prev_labels = prev_labels;
+    a.n_changed = (unsigned long long*)n_changed; a.n_dist = (unsigned long long*)n_dist;
+    return launch_kmeans_elkan(a, stream);
+}
+
+int ofc_kmeans_elkan_bounds(int dtype, int batch, int64_t n, int d, int k, const double* centres_old, const double* centres,
+                            const int32_t* labels, void* upper, void* lower, const uint8_t* active, const uint8_t* just_done,
+                            void* workspace, size_t workspace_bytes, void* stream) {
+    bool shared;
+    int rc = elkan_check(upper, dtype, shared, batch, n, d, k);
+    if (rc != OFC_OK) return rc;
+    if (batch == 0 || n == 0) return OFC_OK;
+    OFC_REQUIRE(centres_old && centres && labels && upper && lower, "null buffer");
+    OFC_REQUIRE((size_t)k * 8 <= 200 * 1024, "Elkan bound update: k=%d shifts do not fit shared memory", k);
+    const size_t need = (size_t)batch * k * 8;
+    if (!workspace || workspace_bytes < need) { set_error("Elkan bound workspace too small: %zu < %zu", workspace_bytes, need); return OFC_ERR_WORKSPACE; }
+    return launch_kmeans_elkan_bounds(dtype, batch, n, d, k, centres_old, centres, labels, upper, lower, active, just_done, workspace,
+                                      stream);
+}
+
+int ofc_kmeans_elkan_inertia(const void* X, int dtype, int batch, int64_t n, int d, int k, const double* mean, const double* centres,
+                             const int32_t* labels, const double* weights, double* inertia, const uint8_t* active, void* workspace,
+                             size_t workspace_bytes, void* stream) {
+    bool shared;
+    int rc = km_check(X, dtype, shared, batch, n, d, k);
+    if (rc != OFC_OK) return rc;
+    if (batch == 0) return OFC_OK;
+    OFC_REQUIRE(batch <= 65535, "batch too large (%d)", batch);
+    OFC_REQUIRE(centres && labels && inertia, "null buffer");
+    if (n == 0) { OFC_CUDA(cudaMemsetAsync(inertia, 0, sizeof(double) * batch, (cudaStream_t)stream)); return OFC_OK; }
+    KmWorkspace w = km_layout(batch, n, d, k, shared);
+    if (!workspace || workspace_bytes < w.assign_total) { set_error("k-means workspace too small: %zu < %zu", workspace_bytes, w.assign_total); return OFC_ERR_WORKSPACE; }
+    return launch_kmeans_elkan_inertia(X, shared ? 0 : n * d, dtype, batch, n, d, k, mean, centres, labels, weights, shared ? 0 : n,
+                                       (double*)((char*)workspace + w.off_inertia), w.parts, inertia, active, stream);
+}
+
 // ---- cosine ----------------------------------------------------------------
 int ofc_sliding_cosine(const double* a, int n, const double* b, int64_t m, double* sims, double* best,
                        int64_t* best_idx, void* stream) {

@@ -320,6 +320,58 @@ class TensorCoreSteps:
                                          _ptr(counts), _ptr(self.ws), C.c_size_t(self.ws_bytes), c.stream()))
 
 
+class ElkanSteps:
+    """Elkan's E-step for the problems of a :class:`LloydState` (sklearn's ``_kmeans_single_elkan``, libofc's
+    ofc_kmeans_elkan_*): the triangle-inequality bounds (``upper [B, n]``, ``lower [B, n, k]``), the centre geometry
+    (``chd [B, k, k]``, ``dnc [B, k]``) and the centres before the last update, all in the working dtype (float32 for
+    float32 rows, float64 otherwise).  The M-step, relocation and centre update stay the Lloyd kernels."""
+
+    def __init__(self, st: "LloydState", mean: torch.Tensor):
+        self.st, self.mean = st, mean
+        B, n, k, d, dev = st.B, st.n, st.k, st.d, st.X.device
+        wdt = torch.float32 if st.dtype == 1 else torch.float64
+        self.upper = torch.empty((B, n), dtype=wdt, device=dev)
+        self.lower = torch.empty((B, n, k), dtype=wdt, device=dev)
+        self.chd = torch.empty((B, k, k), dtype=wdt, device=dev)
+        self.dnc = torch.empty((B, k), dtype=wdt, device=dev)
+        self.old = torch.empty((B, k, d), dtype=torch.float64, device=dev)
+        self.geo_ws = torch.empty(max(B * k * d * 4 if st.dtype == 1 else 0, 256), dtype=torch.uint8, device=dev)
+        #: [B] int64 distances evaluated by the steps (None: not counted)
+        self.n_dist = None
+
+    def centres_(self, centres):
+        """chd and dnc of ``centres`` (every problem)"""
+        st, c = self.st, self.st.ctx
+        c.check(c.lib.ofc_kmeans_elkan_centres(st.dtype, st.B, st.d, st.k, _ptr(centres), _ptr(self.chd), _ptr(self.dnc),
+                                               _ptr(self.geo_ws), C.c_size_t(self.geo_ws.numel()), c.stream()))
+
+    def init(self, centres, labels):
+        st, c = self.st, self.st.ctx
+        c.check(c.lib.ofc_kmeans_elkan_init(_ptr(st.X), st.dtype | st.flags, st.B, C.c_int64(st.n), st.d, st.k, _ptr(self.mean),
+                                            _ptr(centres), _ptr(self.chd), _ptr(labels), _ptr(self.upper), _ptr(self.lower),
+                                            _ptr(None), c.stream()))
+
+    def step(self, centres, labels_in, labels, prev=None, n_changed=None, active=None):
+        st, c = self.st, self.st.ctx
+        c.check(c.lib.ofc_kmeans_elkan_step(_ptr(st.X), st.dtype | st.flags, st.B, C.c_int64(st.n), st.d, st.k, _ptr(self.mean),
+                                            _ptr(centres), _ptr(self.chd), _ptr(self.dnc), _ptr(labels_in), _ptr(labels), _ptr(prev),
+                                            _ptr(self.upper), _ptr(self.lower), _ptr(n_changed), _ptr(self.n_dist), _ptr(active),
+                                            c.stream()))
+
+    def bounds(self, centres, labels):
+        """the bound update from ``self.old`` to ``centres`` for the running problems and those that just stopped"""
+        st, c = self.st, self.st.ctx
+        c.check(c.lib.ofc_kmeans_elkan_bounds(st.dtype, st.B, C.c_int64(st.n), st.d, st.k, _ptr(self.old), _ptr(centres), _ptr(labels),
+                                              _ptr(self.upper), _ptr(self.lower), _ptr(st.active), _ptr(st.just_done), _ptr(st.ws),
+                                              C.c_size_t(st.ws.numel()), c.stream()))
+
+    def inertia(self, centres, labels, inertia):
+        st, c = self.st, self.st.ctx
+        c.check(c.lib.ofc_kmeans_elkan_inertia(_ptr(st.X), st.dtype | st.flags, st.B, C.c_int64(st.n), st.d, st.k, _ptr(self.mean),
+                                               _ptr(centres), _ptr(labels), _ptr(st.w), _ptr(inertia), _ptr(None), _ptr(st.ws),
+                                               C.c_size_t(st.ws.numel()), c.stream()))
+
+
 def _tc_worth_it(dtype: int, d: int, k: int) -> bool:
     """float32 rows: always past d = 32.  uint8 rows pay 8 bytes per element for the split copy, so the tensor cores
     are only used where the float64 CUDA-core E-step is the bottleneck (k * d large)."""
@@ -431,7 +483,8 @@ _POLL_LAG = 4
 _EAGER_ITERATIONS = 8
 
 
-def lloyd(X, init, max_iter: int = 300, tol: float = 1e-4, group=None, sample_weight=None, _host_relocation: bool = False):
+def lloyd(X, init, max_iter: int = 300, tol: float = 1e-4, group=None, sample_weight=None, algorithm: str = "lloyd",
+          _host_relocation: bool = False, _n_dist=None):
     """Batched ``KMeans(n_clusters=k, init=init, n_init=1, max_iter=max_iter, tol=tol).fit(X, sample_weight=sample_weight)``.
 
     X ``[n,d]`` or ``[B,n,d]`` (uint8 / float32 / float64; torch on the compute device, or numpy);
@@ -459,11 +512,23 @@ def lloyd(X, init, max_iter: int = 300, tol: float = 1e-4, group=None, sample_we
     relocation and inertia.  The column mean, the tolerance and the stopping rule stay unweighted, as in sklearn.  The
     weighted fit never takes the fused uint8 step.  ``None`` runs the unweighted kernels.  Not with ``group``.
 
+    ``algorithm="elkan"``: sklearn's ``_kmeans_single_elkan`` (_kmeans.py:462-624).  The E-step of every iteration is
+    Elkan's bound-pruned step (:class:`ElkanSteps`), which keeps a row's label when a distance ties where Lloyd takes
+    the first minimum; the M-step, relocation, centre update, stopping rule and loop are Lloyd's.  After a non-strict
+    stop one more Elkan step runs on the current bounds, and the inertia is that of the resulting labels.  Never on
+    the tensor cores or the fused uint8 step; with ``sample_weight`` and shared-row batches as above; not with
+    ``group``.  With k = 1 the fit is Lloyd's.  ``_n_dist`` (benchmark hook): a ``[B]`` uint64-sized int64 device tensor the
+    Elkan steps add the number of distances they evaluate to.
+
     Returns ``(labels int32, centres float64, inertia float64, n_iter int64)`` as torch
     tensors on X's device, squeezed when X was ``[n,d]``.
     """
+    if algorithm not in ("lloyd", "elkan"):
+        raise ValueError(f"algorithm must be 'lloyd' or 'elkan', got {algorithm!r}")
     if sample_weight is not None and group is not None:
         raise NotImplementedError("sample_weight with a row-sharded fit (group)")
+    if algorithm == "elkan" and group is not None:
+        raise NotImplementedError("algorithm='elkan' with a row-sharded fit (group)")
     Xb, single = _as_batch(X, _target_device(X))
     ctx = _Ctx(Xb.device)
     w_host = _check_sample_weight(sample_weight, int(Xb.shape[1]), Xb.dtype, rows=int(Xb.shape[0]))
@@ -474,7 +539,7 @@ def lloyd(X, init, max_iter: int = 300, tol: float = 1e-4, group=None, sample_we
     if shared:
         if group is not None:
             raise NotImplementedError("several starts (init [R, k, d]) of a row-sharded fit")
-        if _tc_wanted(Xb, int(init.shape[1])):
+        if algorithm == "lloyd" and _tc_wanted(Xb, int(init.shape[1])):
             runs = [lloyd(Xb[0], init[r], max_iter, tol, sample_weight=w_host) for r in range(int(init.shape[0]))]
             return tuple(torch.stack(t) for t in zip(*runs))
     elif init.dim() == 2:
@@ -486,7 +551,8 @@ def lloyd(X, init, max_iter: int = 300, tol: float = 1e-4, group=None, sample_we
     k = int(init.shape[1])
     if init.dim() != 3 or init.shape[0] != B or init.shape[2] != d:
         raise ValueError(f"init shape {tuple(init.shape)} does not match X {tuple(Xb.shape)}")
-    use_tc = not shared and _tc_wanted(Xb, k)
+    elkan = algorithm == "elkan" and k >= 2
+    use_tc = not shared and not elkan and _tc_wanted(Xb, k)
     weighted = w_host is not None
     w_dev = None
     if weighted:                     # float64 on the device: [n] read by every start of a shared batch, else [B, n]
@@ -520,7 +586,12 @@ def lloyd(X, init, max_iter: int = 300, tol: float = 1e-4, group=None, sample_we
     # dense float32 corner (d > 32): E/M steps on the tensor-core path, same labels as the float32 kernels
     tc = TensorCoreSteps(st, mean[0].contiguous()) if use_tc else None
     # the fused step's exact integer accumulators do not hold real-valued x w: a weighted uint8 fit takes two kernels
-    fused = tc is None and is_u8 and not weighted and st.step_supported()
+    fused = tc is None and not elkan and is_u8 and not weighted and st.step_supported()
+    el = ElkanSteps(st, mean) if elkan else None
+    if el is not None:
+        el.n_dist = _n_dist                   # init_bounds_dense; its labels are the ones iteration 0 starts from
+        el.centres_(centres)
+        el.init(centres, st.labels[1])
     counts_or_w = st.wsum if weighted else st.counts            # what the relocation and the centre update run on
 
     active = st.active
@@ -560,9 +631,10 @@ def lloyd(X, init, max_iter: int = 300, tol: float = 1e-4, group=None, sample_we
         payload = px.region(px.gather_offset(), payload.numel() * 8).view(torch.float64).view(B, n_far, 3 + d)
     it_counter = torch.zeros(1, dtype=torch.int32, device=dev)       # iteration number, kept on the device
 
-    def iteration(cur):
+    def iteration(cur, first=False):
         """one Lloyd iteration, enqueued on the current stream; nothing in it depends on host-side values, so on one GPU it
-        can be captured in a CUDA graph (the iteration number is `it_counter`)"""
+        can be captured in a CUDA graph (the iteration number is `it_counter`).  ``first``: iteration 0, whose Elkan step
+        compares its labels with sklearn's -1 start"""
         lab, lab_old = st.labels[cur], st.labels[cur ^ 1]
         sums_w, counts_w, changed_w = local[cur]                 # where this rank's partial results go
         if tc is not None:
@@ -571,7 +643,10 @@ def lloyd(X, init, max_iter: int = 300, tol: float = 1e-4, group=None, sample_we
         elif fused:
             st.step(mean, centres, lab, lab_old, changed_w, sums_w, counts_w, active=active)
         else:
-            st.assign(mean, centres, lab, prev=lab_old, n_changed=changed_w, active=active)
+            if el is not None:
+                el.step(centres, lab_old, lab, prev=None if first else lab_old, n_changed=changed_w, active=active)
+            else:
+                st.assign(mean, centres, lab, prev=lab_old, n_changed=changed_w, active=active)
             # uint8: raw (exact integer) sums; floats: sums of the centred rows like sklearn
             if weighted:
                 st.sums_weighted(None if is_u8 else mean, lab, sums_w, st.wsum, active=active)
@@ -611,8 +686,13 @@ def lloyd(X, init, max_iter: int = 300, tol: float = 1e-4, group=None, sample_we
                                                             _ptr(overflow), _ptr(active), ctx.stream()))
         else:
             st.relocate(mean, lab, centres, st.sums, counts_or_w, is_u8, active=active)
+        if el is not None:
+            el.old.copy_(centres)
         st.update_(st.sums, counts_or_w, mean if is_u8 else None, 0 if is_u8 else 1, 1 if is_f32 else 0, centres, st.n_changed,
                    tol_, 0, n_active, lab, lab_old, it_counter=it_counter)
+        if el is not None:           # elkan_iter_chunked_dense's bound update, then the new centres' geometry
+            el.bounds(centres, lab)
+            el.centres_(centres)
 
     def stopped(upto):
         """have all problems stopped by iteration `upto` (as far as the host has seen)?  None = keep going"""
@@ -638,7 +718,7 @@ def lloyd(X, init, max_iter: int = 300, tol: float = 1e-4, group=None, sample_we
     # and short fits never pay for a capture: measured (r02i) a 5-iteration fit of 8 M x 4 rows takes 1.4 ms eagerly
     # and 2.4 ms when a graph is captured after two iterations
     while it < n_eager and not done:
-        iteration(it & 1)
+        iteration(it & 1, first=it == 0)
         seen[it:it + 1].copy_(n_active[it:it + 1], non_blocking=True)
         if overflow is not None:
             overflow_seen[it:it + 1].copy_(overflow, non_blocking=True)
@@ -690,12 +770,19 @@ def lloyd(X, init, max_iter: int = 300, tol: float = 1e-4, group=None, sample_we
         if int(overflow.item()):
             # more clusters empty at once than the device-side candidate list holds: redo the fit with the host-merged
             # relocation (every rank takes this branch: the all-reduced counts are the same everywhere)
-            return lloyd(X, init_arg, max_iter, tol, group, sample_weight, _host_relocation=True)
+            return lloyd(X, init_arg, max_iter, tol, group, sample_weight, algorithm, _host_relocation=True)
     final = st.labels[0]
     # strict stops already hold the labels of the final centres; the rest get one more E-step
     # (_kmeans.py:745-755).  Re-running it for everyone is idempotent for the strict ones and
     # yields the inertia of the final (centres, labels) in the same pass.
-    if tc is not None:
+    if el is not None:
+        # a problem's labels are in the buffer of its last iteration; n_changed is that iteration's count (the Elkan step
+        # leaves stopped problems' counts alone), so n_changed != 0 is a non-strict stop, which gets sklearn's closing
+        # Elkan step on the current bounds (_kmeans.py:601-617); the inertia is that of these labels
+        final = torch.where(((st.n_iter - 1) & 1).to(torch.bool).view(B, 1), st.labels[1], st.labels[0]).contiguous()
+        el.step(centres, final, final, active=(st.n_changed != 0).to(torch.uint8))
+        el.inertia(centres, final, st.inertia)
+    elif tc is not None:
         tc.assign(centres, final, inertia=st.inertia)
     else:
         st.assign(mean, centres, final, inertia=st.inertia)
@@ -974,11 +1061,18 @@ class KMeans:
     clustering.
 
     ``fit(X, sample_weight=w)`` is sklearn's weighted fit (seeding, M-step, relocation and inertia weighted; see
-    :func:`_check_sample_weight` for the accepted weights); :meth:`score` is its negative weighted inertia."""
+    :func:`_check_sample_weight` for the accepted weights); :meth:`score` is its negative weighted inertia.
 
-    def __init__(self, n_clusters=8, *, init="k-means++", n_init="auto", max_iter=300, tol=1e-4, random_state=None):
+    ``algorithm`` is ``"lloyd"`` (default) or ``"elkan"`` (see :func:`lloyd`); any other value raises ValueError at
+    ``fit``, and ``"elkan"`` with one cluster warns and runs Lloyd, as sklearn does.  ``copy_x`` and ``verbose`` are
+    accepted for compatibility: X is never modified (the rows are centred on the fly), and the per-iteration printout
+    of ``verbose`` is not reproduced."""
+
+    def __init__(self, n_clusters=8, *, init="k-means++", n_init="auto", max_iter=300, tol=1e-4, verbose=0, random_state=None,
+                 copy_x=True, algorithm="lloyd"):
         self.n_clusters, self.init, self.n_init = int(n_clusters), init, n_init
         self.max_iter, self.tol, self.random_state = int(max_iter), float(tol), random_state
+        self.verbose, self.copy_x, self.algorithm = verbose, copy_x, algorithm
 
     def fit(self, X, y=None, sample_weight=None):
         Xa = X if isinstance(X, torch.Tensor) else np.asarray(X)
@@ -990,6 +1084,15 @@ class KMeans:
         if isinstance(self.init, str) and self.init not in ("k-means++", "random"):
             raise ValueError(f"init={self.init!r}: 'k-means++', 'random' or an array")
         n_init = _resolve_n_init(self.n_init, self.init)
+        if not isinstance(self.algorithm, str) or self.algorithm not in ("lloyd", "elkan"):
+            raise ValueError("The 'algorithm' parameter of KMeans must be a str among {'lloyd', 'elkan'}. "
+                             f"Got {self.algorithm!r} instead.")
+        algorithm = self.algorithm
+        if algorithm == "elkan" and self.n_clusters == 1:
+            import warnings
+            warnings.warn("algorithm='elkan' doesn't make sense for a single cluster. Using 'lloyd' instead.", RuntimeWarning,
+                          stacklevel=2)
+            algorithm = "lloyd"
         if isinstance(self.init, str) and self.n_clusters > 1 and (n_init > 1 or self.init == "random"):
             rs = (self.random_state if isinstance(self.random_state, np.random.RandomState)
                   else np.random.RandomState(self.random_state))
@@ -999,7 +1102,7 @@ class KMeans:
                 init, _ = random_starts(Xd, self.n_clusters, n_init, rs, sw)
             else:
                 init, _ = kmeans_plusplus_starts(Xd, self.n_clusters, n_init, rs, sw)
-            labels, centres, inertia, n_iter = lloyd(Xd, init, self.max_iter, self.tol, sample_weight=sw)
+            labels, centres, inertia, n_iter = lloyd(Xd, init, self.max_iter, self.tol, sample_weight=sw, algorithm=algorithm)
             b = best_start(labels, inertia, self.n_clusters)
             labels, centres, inertia, n_iter = labels[b], centres[b], inertia[b], n_iter[b]
         else:
@@ -1010,7 +1113,7 @@ class KMeans:
                     init, _ = kmeans_plusplus(Xa, self.n_clusters, self.random_state, sw)
             else:
                 init = self.init
-            labels, centres, inertia, n_iter = lloyd(Xa, init, self.max_iter, self.tol, sample_weight=sw)
+            labels, centres, inertia, n_iter = lloyd(Xa, init, self.max_iter, self.tol, sample_weight=sw, algorithm=algorithm)
         self._centres_t = centres
         # a float32 fit: sklearn's cluster_centers_ are float32, and transform measures against those
         self._f32 = Xa.dtype == (torch.float32 if isinstance(Xa, torch.Tensor) else np.float32)
